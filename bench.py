@@ -23,6 +23,10 @@ oracle timed on this box's host cores on a bounded sample (rank 0, N=1 only).
 --scaling strong shards a FIXED global batch (--global-batch, default 2048 frames per step) over the GPUs instead of 256
 frames per GPU (SURVEY.md 8d config 4).  At N = 1 the line also carries `other_configs`: the same step at the C path's
 native geometry (240x320 RGB444), from fp32 NCHW input, and under contract P (the contract pinned on the reference module).
+
+--dump-outputs DIR writes the detection lists of the last timed step (at N > 1, every rank's lists as collected on rank 0)
+to DIR as .npy files (see dump_outputs).  Frames and weights are seeded, so two builds of the project run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -214,6 +218,29 @@ def yolo_v2_maps(qnet, h, w):
     return dims
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, counts, records, max_det):
+    """Writes the detection lists of one step (counts [frames], records int32 [sum(counts), 8] in frame order, as the
+    C-ABI's yolo_b200_det) to out_dir as float32 .npy files: frames (index of each dumped frame), counts, and per
+    detection boxes (x1, y1, x2, y2), scores, classes, anchor_index.  The integer fields (frames, counts, classes,
+    anchor_index) are float32 too, like every dumped array, and exact: they stay far below 2**24.  When max_det records per frame could exceed
+    DUMP_BYTES, a fixed seeded sample of frames is written; it does not depend on the results, so two builds of the
+    project dump the same frames and can be compared output for output."""
+    n = len(counts)
+    k = min(n, DUMP_BYTES // (max_det * 7 * 4 + 2 * 4))
+    frames = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    start = np.concatenate([[0], np.cumsum(counts, dtype=np.int64)])
+    assert start[-1] == len(records)
+    rec = np.ascontiguousarray(records[np.concatenate([np.arange(start[f], start[f + 1]) for f in frames]).astype(np.int64)])
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"frames": frames, "counts": np.asarray(counts)[frames], "boxes": rec.view(np.float32)[:, :4],
+           "scores": rec.view(np.float32)[:, 4], "classes": rec[:, 5], "anchor_index": rec[:, 6]}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def time_steps(stream, fn, warm, steps):
     import torch
     for i in range(warm):
@@ -239,7 +266,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip other_configs / sparse head / image front end")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the detections of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what --impl b200 computed")
+    sys.dont_write_bytecode = True     # the tree may be read-only: nothing is cached next to the sources
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -323,6 +356,15 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs and rank == 0:    # before the per-kernel timing passes below overwrite d_dets / d_counts
+        if coll is None:
+            filled = torch.arange(MAXDET, device="cuda")[None, :] < d_counts[:, None]
+            counts, records = d_counts.cpu().numpy(), d_dets[filled].cpu().numpy()
+        else:                              # every rank's lists as they arrived on rank 0
+            parts = coll.collected(args.warmup + args.steps - 1)
+            counts = np.concatenate([np.diff(off.cpu().numpy()) for off, _ in parts])
+            records = np.concatenate([rec.cpu().numpy() for _, rec in parts])
+        dump_outputs(args.dump_outputs, counts, records, MAXDET)
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

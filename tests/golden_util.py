@@ -60,6 +60,64 @@ def load(name):
     return _cache[name]
 
 
+def tier_golden():
+    """tests/golden/tier_ref.npz (oracle/gen_golden_tier.py): what the reference's compiled C functions return on the
+    seeded inputs below, for the tier-A / tier-B tests to compare with when oracle/_ref/libtierA.so / libtierB.so are absent."""
+    if "tier" not in _cache:
+        _cache["tier"] = dict(np.load(os.path.join(GOLDEN, "tier_ref.npz"), allow_pickle=False))
+    return _cache["tier"]
+
+
+def tier_shift_cases():
+    """(sa_in, sw, sb, retune, sa_out) of set_quantize_scale: the ten shipped layers, then 200 seeded random ones."""
+    rng = np.random.default_rng(0)
+    cases = [(ex.SHIPPED_SCALE_A[l], ex.SHIPPED_SCALE_W[l], ex.SHIPPED_SCALE_B[l], ex.SHIPPED_RETUNE[l],
+              ex.SHIPPED_SCALE_A[l + 1]) for l in range(10)]
+    return cases + [tuple(int(v) for v in rng.integers(0, 17, 5)) for _ in range(200)]
+
+
+def tier_head_trials():
+    """(sa, one-cell int8 prediction map [1][1][48]) for the C head primitives, 200 seeded trials."""
+    rng = np.random.default_rng(1)
+    out = []
+    for _ in range(200):
+        sa = int(rng.integers(2, 6))
+        pred = np.zeros((1, 1, 48), np.int8)
+        pred[0, 0, :35] = rng.integers(-40, 40, 35)
+        out.append((sa, pred))
+    return out
+
+
+def tier_tie_trials():
+    """(trial, boxes int32 [n][x_max, x_min, y_max, y_min], scores float32 [n]) with scores drawn from a handful of values
+    (full of ties) and unique boxes, for conf_sort + NMS."""
+    rng = np.random.default_rng(7)
+    out = []
+    for trial in range(60):
+        n = int(rng.integers(2, 200))
+        levels = int(rng.integers(1, 8))
+        x1 = rng.integers(0, 200, n); y1 = rng.integers(0, 150, n)
+        x2 = x1 + rng.integers(1, 120, n); y2 = y1 + rng.integers(1, 120, n)
+        boxes = np.stack([x2, x1, y2, y1], 1).astype(np.int32)
+        if len({tuple(b) for b in boxes}) != n:           # the shim maps sorted entries back by (score, box): keep boxes unique
+            continue
+        conf = (rng.integers(0, levels, n).astype(np.float32) + 1) / np.float32(levels + 1)
+        out.append((trial, boxes, conf))
+    return out
+
+
+def tier_b_inputs():
+    """One 240x320 RGB444 frame (with the slack rows the literal driver reads past its end), 16x3x3x3 int8 weights and
+    the 32-entry bias buffer of the first layer."""
+    rng = np.random.default_rng(0)
+    frame = np.zeros(240 * 320 + 64 * 320, np.int16)
+    frame[:240 * 320] = rng.integers(0, 4096, 240 * 320)
+    w = rng.integers(-6, 6, (16, 3, 3, 3), dtype=np.int8)
+    b = np.zeros(32, np.int8)
+    b[:16] = rng.integers(-40, 40, 16)
+    return frame, w, b
+
+
 def reference_kept_indices(g, i):
     """Anchor indices of the detections the reference returned for frame i.  postprocess() returns them in ascending
     anchor order (np.where(keep > 0), slim_yolo_v2.py:205), so they are matched in one ascending pass against the
