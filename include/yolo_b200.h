@@ -196,6 +196,17 @@ int yolo_b200_forward_u8bgr(yolo_b200_ctx *ctx, const uint8_t *bgr, int n, int h
 int yolo_b200_forward_u8bgr_resize(yolo_b200_ctx *ctx, const uint8_t *bgr, int n, int sh, int sw, int h, int w,
                                    yolo_b200_det *dets, int32_t *counts);
 
+/* The same for a batch of images of DIFFERENT sizes (a folder of image files, the VOC evaluator): one call, the chunked
+ * copies, one batch-wide decode + NMS, as for one size.  src_hw: HOST int32 [n][2] = (sh, sw) of each image; the images are
+ * packed back to back, image i at byte offset 3 * sum_{j<i} sh_j * sw_j, no padding, no alignment requirement.  Each image is
+ * resized to h x w (bit-exact as above); boxes are normalised, so image i scales them by its own [sw, sh, sw, sh].
+ * Errors: n < 0, sh or sw < 1, src_hw NULL with n > 0, null buffers: E_ARG (-1); an image over 2 GiB: E_UNSUPPORTED (-3).
+ * n == 0 writes nothing.  The submit form is the asynchronous pair of yolo_b200_submit_u8bgr (needs n >= 1; + yolo_b200_wait). */
+int yolo_b200_forward_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
+                                   yolo_b200_det *dets, int32_t *counts);
+int yolo_b200_submit_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
+                                  yolo_b200_det *dets, int32_t *counts);
+
 /* Replaces SlimYOLOv2_quantize_bnfuse.forward(x, quantization=True) inference branch,
  * slim_yolo_v2.py:212-358, for a float NCHW batch (input quantised by a_tracker_in, :218). */
 int yolo_b200_forward_f32(yolo_b200_ctx *ctx, const float *nchw, int n, int h, int w,
@@ -213,6 +224,11 @@ int yolo_b200_forward_u8bgr_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n,
                                 yolo_b200_det *d_dets, int32_t *d_counts);
 /* Block until everything queued on the context stream is done. */
 int yolo_b200_forward_u8bgr_resize_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n, int sh, int sw, int h, int w,
+                                       yolo_b200_det *d_dets, int32_t *d_counts);
+/* Images of different sizes packed back to back in device memory (layout and errors as yolo_b200_forward_u8bgr_ragged;
+ * src_hw stays a HOST array).  Calls may be queued back to back without a synchronise: each call's resize tables are
+ * written in stream order on the context stream. */
+int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n, const int32_t *src_hw, int h, int w,
                                        yolo_b200_det *d_dets, int32_t *d_counts);
 
 int yolo_b200_sync(yolo_b200_ctx *ctx);
@@ -236,6 +252,11 @@ int yolo_b200_u8bgr_lut(yolo_b200_ctx *ctx, int8_t *lut_host);
  * d_dst 4-byte aligned and dw a multiple of 4 take the vectorised kernel (same results otherwise). */
 int yolo_b200_resize_u8bgr(yolo_b200_ctx *ctx, const uint8_t *d_src, int n, int sh, int sw,
                            uint8_t *d_dst, int dh, int dw);
+/* The same for images of different sizes packed back to back in d_src (src_hw: HOST int32 [n][2] = (sh, sw) of each image,
+ * image i at byte offset 3 * sum_{j<i} sh_j * sw_j) -> uint8 [n][dh][dw][3]; one kernel launch whatever the number of sizes.
+ * Errors as yolo_b200_forward_u8bgr_ragged; n == 0 writes nothing. */
+int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *d_src, int n, const int32_t *src_hw,
+                                  uint8_t *d_dst, int dh, int dw);
 /* Host only (no GPU needed), for tests: the per-index programme of that resize along one axis, taps[4*d + {0,1,2,3}] =
  * (source index 0, source index 1, weight 0, weight 1), weights in units of 1/2048; horizontal != 0 re-anchors the tap
  * at the image border as OpenCV's horizontal pass does. */

@@ -106,38 +106,56 @@ def main():
         run_video(ctx, args, size)
         ctx.close()
         return
+    md = 1024
     if args.images.startswith("synthetic:"):
         rng = np.random.default_rng(0)
-        imgs = [rng.integers(0, 256, (480, 640, 3), dtype=np.uint8) for _ in range(int(args.images.split(":")[1]))]
-        names = ["synthetic_%d" % i for i in range(len(imgs))]
+        count = int(args.images.split(":")[1])
+        sources = [("synthetic_%d" % i, lambda: rng.integers(0, 256, (480, 640, 3), dtype=np.uint8)) for i in range(count)]
     else:
         files = sorted(glob.glob(os.path.join(args.images, "*")) if os.path.isdir(args.images) else glob.glob(args.images))
-        imgs = [cv2.imread(f, cv2.IMREAD_COLOR) for f in files]
-        names = [os.path.splitext(os.path.basename(f))[0] for f in files]
-        imgs, names = zip(*[(i, n) for i, n in zip(imgs, names) if i is not None]) if files else ((), ())
-    os.makedirs(args.out, exist_ok=True)
-    t_dev = 0.0
-    for b0 in range(0, len(imgs), args.batch):
-        chunk = imgs[b0:b0 + args.batch]
-        # data/__init__.py:36 (cv2.resize, bilinear) runs on the GPU too: images of one size go in one call
-        t0 = time.time()
-        dets = np.zeros((len(chunk), 1024), dtype=lib.DET_DTYPE)
-        counts = np.zeros(len(chunk), dtype=np.int32)
-        shapes = sorted({im.shape[:2] for im in chunk})
-        for shp in shapes:
-            idx = [k for k, im in enumerate(chunk) if im.shape[:2] == shp]
-            d, c_ = ctx.forward_u8bgr_resize(np.stack([chunk[k] for k in idx]), size)
-            dets[idx] = d
-            counts[idx] = c_
-        t_dev += time.time() - t0
-        for k, im in enumerate(chunk):
-            boxes, scores, cls, _ = lib.dets_to_arrays(dets[k], int(min(counts[k], 1024)))
+        sources = [(os.path.splitext(os.path.basename(f))[0], lambda f=f: cv2.imread(f, cv2.IMREAD_COLOR)) for f in files]
+
+    def batches():
+        """Batches of --batch readable images, read only when the batch is formed (unreadable files are skipped)."""
+        names, imgs = [], []
+        for name, read in sources:
+            im = read()
+            if im is None:
+                continue
+            names.append(name); imgs.append(im)
+            if len(imgs) == args.batch:
+                yield names, imgs
+                names, imgs = [], []
+        if imgs:
+            yield names, imgs
+
+    def finish(job):
+        ticket, names, imgs, dets, counts, _ = job
+        ctx.wait(ticket)
+        for k, im in enumerate(imgs):
+            boxes, scores, cls, _ = lib.dets_to_arrays(dets[k], int(min(counts[k], md)))
             h, w = im.shape[:2]
             boxes = boxes * np.array([[w, h, w, h]], dtype=np.float32)          # test.py:88-90
             out = vis(im.copy(), boxes, scores, cls, args.visual_threshold)
-            cv2.imwrite(os.path.join(args.out, names[b0 + k] + ".jpg"), out)
-            print("%s: %d detections (%d above %.2f)" % (names[b0 + k], len(scores), int((scores > args.visual_threshold).sum()), args.visual_threshold))
-    print("%d images, %.1f ms in yolo_b200_forward_u8bgr_resize" % (len(imgs), 1e3 * t_dev))
+            cv2.imwrite(os.path.join(args.out, names[k] + ".jpg"), out)
+            print("%s: %d detections (%d above %.2f)" % (names[k], len(scores), int((scores > args.visual_threshold).sum()), args.visual_threshold))
+
+    # data/__init__.py:36 (cv2.resize, bilinear) runs on the GPU too: each batch, whatever its mix of sizes, is one call.  Two
+    # batches are in flight: reading batch k+1 and writing the annotated images of batch k-1 overlap the GPU work of batch k.
+    os.makedirs(args.out, exist_ok=True)
+    t0, total, inflight = time.time(), 0, []
+    for names, imgs in batches():
+        packed, shapes = lib.pack_images(imgs)
+        packed = torch.from_numpy(packed).pin_memory()                     # asynchronous host-to-device copies
+        dets = np.zeros((len(imgs), md), dtype=lib.DET_DTYPE)
+        counts = np.zeros(len(imgs), dtype=np.int32)
+        if len(inflight) == 2:
+            finish(inflight.pop(0))
+        inflight.append((ctx.submit_u8bgr_images(packed, shapes, size, dets, counts), names, imgs, dets, counts, packed))
+        total += len(imgs)
+    while inflight:
+        finish(inflight.pop(0))
+    print("%d images, %.1f ms reading, detecting and writing (yolo_b200_submit_u8bgr_ragged / yolo_b200_wait)" % (total, 1e3 * (time.time() - t0)))
     ctx.close()
 
 

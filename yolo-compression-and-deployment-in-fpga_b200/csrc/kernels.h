@@ -90,6 +90,13 @@ void resize_axis_table(int src, int dst, bool clamp_weights, int index_scale, in
 // xtab: per column (byte offset of tap 0 in its row, weight0 | weight1 << 16), tap 1 = the next pixel; ytab: per row (row 0, row 1, weight0 << 16, weight1 << 16)
 cudaError_t resize_u8bgr(const uint8_t *src, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                          const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
+// taps and weights of one geometry (sh, sw) -> (dh, dw) in the layout above: ytab [dh], xtab [dw] (host)
+void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab);
+// Images of different sizes packed back to back in one buffer of src_bytes bytes: frame f starts at byte off of src, its
+// rows are pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
+struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
+cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames_dev, int n, uint8_t *dst, int dh, int dw,
+                                const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
 
 // head.cu
 struct HeadArgs {

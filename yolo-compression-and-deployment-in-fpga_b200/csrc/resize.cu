@@ -122,60 +122,104 @@ __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__
 // 32-pixel chunk (with one CTA per row every warp repeated them for its single chunk: 150 instead of 85 instructions per
 // chunk).  Everything that depends on the row only (taps, weights, row pointers, their misalignment) is warp-uniform.
 // WORD_STORE needs dst 4-byte aligned and dw % 4 == 0, so that every row and every 32-pixel chunk starts on a word.
-template <bool WORD_STORE>
-__global__ void __launch_bounds__(256, 6) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+// RAGGED: the frames have different source sizes (every frame still becomes dh x dw).  Frame f is described by
+// frames[f] = {byte offset in src, row pitch, geometry g}; its row / column tables are ytab + g * dh / xtab + g * dw.  The
+// descriptor is loaded when dy wraps, so its cost is warp-uniform and paid once per frame.  Otherwise frames are
+// sh x sw and packed at a uniform stride.
+template <bool WORD_STORE, bool RAGGED>
+__global__ void __launch_bounds__(256, RAGGED ? 5 : 6) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                           const int2 *__restrict__ xtab, const int4 *__restrict__ ytab,
+                                                          const ResizeFrame *__restrict__ frames,
                                                           unsigned rows, unsigned rows_per_warp, int sh, int sw, int dh, int dw, size_t src_bytes)
 {
     const int lane = threadIdx.x & 31;
     unsigned row = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * rows_per_warp;
     if (row >= rows) return;
     const unsigned row_end = min(rows, row + rows_per_warp);
-    const size_t src_frame = (size_t)sh * sw * 3, src_row = (size_t)sw * 3;
     const size_t delta = reinterpret_cast<uintptr_t>(src) & 3;                             // word-aligned view of the source
     const unsigned char *base = src - delta;
     const size_t end = delta + src_bytes;                                                  // one past the last source byte
     const int p = (4 * lane) / 3;
     const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
     unsigned dy = row % (unsigned)dh;
-    size_t frame_off = delta + (size_t)(row / (unsigned)dh) * src_frame;
+    size_t src_frame = 0, src_row, frame_off;
+    unsigned f = row / (unsigned)dh, geom = 0;
+    auto load_frame = [&](unsigned fi) {
+        const int4 d = __ldg(reinterpret_cast<const int4 *>(frames) + fi);
+        frame_off = delta + ((size_t)(unsigned)d.x | ((size_t)(unsigned)d.y << 32));
+        src_row = (unsigned)d.z;
+        geom = (unsigned)d.w;
+    };
+    if constexpr (RAGGED) {
+        load_frame(f);
+    } else {
+        src_frame = (size_t)sh * sw * 3; src_row = (size_t)sw * 3;
+        frame_off = delta + (size_t)f * src_frame;
+    }
     uint8_t *drow = dst + (size_t)row * dw * 3;
     for (; row < row_end; ++row) {
-        const int4 yt = __ldg(ytab + dy);
+        const int4 yt = __ldg(ytab + (RAGGED ? geom * (unsigned)dh + dy : dy));
         const size_t o0 = frame_off + (size_t)yt.x * src_row, o1 = frame_off + (size_t)yt.y * src_row;
         const unsigned char *r0 = base + (o0 & ~(size_t)3), *r1 = base + (o1 & ~(size_t)3);
         const unsigned d0 = (unsigned)o0 & 3u, d1 = (unsigned)o1 & 3u;
-        // a window reaches at most 11 bytes past the start of its pixel; rows for which that stays inside the buffer need no clamp
+        // a window reaches at most 11 bytes past the start of its pixel; rows for which that stays inside the buffer need no
+        // clamp (in a ragged batch, bytes past a frame's last pixel belong to the next frame and carry zero weight)
         const size_t omax = o0 > o1 ? o0 : o1;
         if (omax + src_row + 12 <= end) {
-            resize_one_row<WORD_STORE, false>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, xtab, drow, dw, lane, 0, 1, p, rsh);
+            resize_one_row<WORD_STORE, false>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
         } else {
             const size_t room0 = end - 1 - (o0 & ~(size_t)3), room1 = end - 1 - (o1 & ~(size_t)3);
-            resize_one_row<WORD_STORE, true>(r0, r1, d0, d1, (unsigned)room0, (unsigned)room1, (unsigned)yt.z, (unsigned)yt.w, xtab, drow, dw, lane, 0, 1, p, rsh);
+            resize_one_row<WORD_STORE, true>(r0, r1, d0, d1, (unsigned)room0, (unsigned)room1, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
         }
         drow += (size_t)dw * 3;
-        if (++dy == (unsigned)dh) { dy = 0; frame_off += src_frame; }
+        if (++dy == (unsigned)dh) {
+            dy = 0;
+            if constexpr (RAGGED) { if (row + 1 < row_end) load_frame(++f); }
+            else frame_off += src_frame;
+        }
     }
+}
+
+// one wave of resident CTAs (8 warps each), equal runs of rows per warp
+template <bool RAGGED>
+static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames, int n, int sh, int sw, uint8_t *dst,
+                                 int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+{
+    if (n <= 0) return cudaSuccess;
+    const size_t rows = (size_t)n * dh;
+    if (rows > 0x7fffffffull) return cudaErrorInvalidValue;
+    const int threads = 256;
+    // 6 resident CTAs per SM at 40 registers; the ragged variant's descriptor bookkeeping needs 48 (5 CTAs) to run without spills
+    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * (RAGGED ? 5 : 6) * (threads / 32);
+    const unsigned rows_per_warp = (unsigned)((rows + max_warps - 1) / max_warps);
+    const size_t warps = (rows + rows_per_warp - 1) / rows_per_warp;
+    const size_t blocks = (warps + threads / 32 - 1) / (threads / 32);
+    if ((reinterpret_cast<uintptr_t>(dst) & 3) == 0 && dw % 4 == 0)
+        resize_u8c3_kernel<true, RAGGED><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+    else
+        resize_u8c3_kernel<false, RAGGED><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+    return cudaGetLastError();
 }
 
 cudaError_t resize_u8bgr(const uint8_t *src, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                          const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
 {
-    if (n <= 0) return cudaSuccess;
-    const size_t rows = (size_t)n * dh;
-    if (rows > 0x7fffffffull) return cudaErrorInvalidValue;
-    // one wave of resident CTAs (8 warps each), equal runs of rows per warp
-    const int threads = 256;
-    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * 6 * (threads / 32);     // 6 resident CTAs per SM at 40 registers
-    const unsigned rows_per_warp = (unsigned)((rows + max_warps - 1) / max_warps);
-    const size_t warps = (rows + rows_per_warp - 1) / rows_per_warp;
-    const size_t blocks = (warps + threads / 32 - 1) / (threads / 32);
-    const size_t src_bytes = (size_t)n * sh * sw * 3;
-    if ((reinterpret_cast<uintptr_t>(dst) & 3) == 0 && dw % 4 == 0)
-        resize_u8c3_kernel<true><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
-    else
-        resize_u8c3_kernel<false><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
-    return cudaGetLastError();
+    return resize_launch<false>(src, (size_t)n * sh * sw * 3, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+}
+
+cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames_dev, int n, uint8_t *dst, int dh, int dw,
+                                const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+{
+    return resize_launch<true>(src, src_bytes, frames_dev, n, 0, 0, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+}
+
+void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab)
+{
+    resize_axis_table(sh, dh, false, 1, ytab);               // row taps; weights pre-shifted for the kernel's high multiply
+    for (int d = 0; d < dh; ++d) { ytab[d].z <<= 16; ytab[d].w <<= 16; }
+    std::vector<int4> t((size_t)dw);
+    resize_axis_table(sw, dw, true, 3, t.data());            // column taps as byte offsets inside a row; tap 1 = the next pixel
+    for (int d = 0; d < dw; ++d) xtab[d] = make_int2(t[d].x, t[d].z | (t[d].w << 16));
 }
 
 }  // namespace yb

@@ -9,6 +9,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <map>
 #include <mutex>
 #include <vector>
 #include <string>
@@ -78,6 +79,8 @@ constexpr int YB_HOST_SLOTS = 2;
 struct HostSlot {
     void *stage_in = nullptr; size_t stage_in_cap = 0;      // device staging of the host frames (network-size frames)
     void *rs_src = nullptr; size_t rs_src_cap = 0;          // resize front end: staged source images
+    void *rg_tab = nullptr; size_t rg_tab_cap = 0;          // images of different sizes: descriptors + tables of the call (device)
+    char *rg_host = nullptr; size_t rg_host_cap = 0;        // ... and their pinned staging copy
     int8_t *pred_all = nullptr; size_t pred_all_cap = 0;    // batch-wide prediction map
     yolo_b200_det *d_dets = nullptr; size_t dets_cap = 0;
     int32_t *d_counts = nullptr; size_t counts_cap = 0;
@@ -111,6 +114,12 @@ struct yolo_b200_ctx {
     void *rs_tab = nullptr; size_t rs_tab_cap = 0;      // [dh] int4 row taps/weights, then [dw] int2 column offsets/weights
     const int4 *rs_ytab = nullptr; const int2 *rs_xtab = nullptr;
     int rs_key[4] = {0, 0, 0, 0};                       // (sh, sw, dh, dw) the tables were built for
+    // images of different sizes, device entry points: descriptors + tables of the most recent call, rewritten in stream
+    // order on the context stream; two pinned staging buffers alternate (one is refilled once the copy out of it has run)
+    void *rg_tab = nullptr; size_t rg_tab_cap = 0;
+    char *rg_host[2] = {nullptr, nullptr}; size_t rg_host_cap[2] = {0, 0};
+    cudaEvent_t rg_ev[2] = {nullptr, nullptr};
+    int rg_next = 0;
     float *h_scores = nullptr; int *h_cls = nullptr; float4 *h_boxes = nullptr; size_t head_cap = 0;
     int last_n = 0;
     int64_t launches = 0;
@@ -205,12 +214,17 @@ void yolo_b200_destroy(yolo_b200_ctx *c)
     cudaStreamSynchronize(c->stream);
     free_layers(c);
     cudaFree(c->lut_dev); cudaFree(c->lut8_dev); cudaFree(c->ovf_dev); cudaFree(c->stats_dev); cudaFree(c->in_q);
-    cudaFree(c->rs_out); cudaFree(c->rs_tab);
+    cudaFree(c->rs_out); cudaFree(c->rs_tab); cudaFree(c->rg_tab);
+    for (int k = 0; k < 2; ++k) {
+        if (c->rg_host[k]) cudaFreeHost(c->rg_host[k]);
+        if (c->rg_ev[k]) cudaEventDestroy(c->rg_ev[k]);
+    }
     cudaFree(c->h_scores); cudaFree(c->h_cls); cudaFree(c->h_boxes);
     for (auto e : c->ev) cudaEventDestroy(e);
     for (auto &S : c->slots) {
-        cudaFree(S.stage_in); cudaFree(S.rs_src); cudaFree(S.pred_all); cudaFree(S.d_dets); cudaFree(S.d_counts);
+        cudaFree(S.stage_in); cudaFree(S.rs_src); cudaFree(S.rg_tab); cudaFree(S.pred_all); cudaFree(S.d_dets); cudaFree(S.d_counts);
         if (S.counts_pinned) cudaFreeHost(S.counts_pinned);
+        if (S.rg_host) cudaFreeHost(S.rg_host);
         for (auto e : S.ev_in) cudaEventDestroy(e);
         for (auto e : S.ev_done) cudaEventDestroy(e);
         for (auto e : S.ev_cnt) cudaEventDestroy(e);
@@ -605,17 +619,11 @@ static int ensure_resize_tables(yolo_b200_ctx *c, int sh, int sw, int dh, int dw
     if (c->rs_tab && c->rs_key[0] == sh && c->rs_key[1] == sw && c->rs_key[2] == dh && c->rs_key[3] == dw) return 0;
     const size_t ybytes = (size_t)dh * sizeof(int4), xbytes = (size_t)dw * sizeof(int2);
     int rc = ensure(&c->rs_tab, &c->rs_tab_cap, ybytes + xbytes); if (rc) return rc;
-    std::vector<int4> t((size_t)(dw > dh ? dw : dh));
-    std::vector<char> img(ybytes + xbytes);
-    resize_axis_table(sh, dh, false, 1, t.data());           // row taps; weights pre-shifted for the kernel's high multiply
-    for (int d = 0; d < dh; ++d) { t[d].z <<= 16; t[d].w <<= 16; }
-    memcpy(img.data(), t.data(), ybytes);
-    resize_axis_table(sw, dw, true, 3, t.data());            // column taps as byte offsets inside a row; tap 1 = the next pixel
-    int2 *xt = reinterpret_cast<int2 *>(img.data() + ybytes);
-    for (int d = 0; d < dw; ++d) xt[d] = make_int2(t[d].x, t[d].z | (t[d].w << 16));
+    std::vector<int4> img((ybytes + xbytes + sizeof(int4) - 1) / sizeof(int4));
+    resize_geometry_tables(sh, sw, dh, dw, img.data(), reinterpret_cast<int2 *>(reinterpret_cast<char *>(img.data()) + ybytes));
     c->rs_key[0] = 0;
     // an earlier resize queued on the context stream may still read the tables: stream-ordered copy from pageable memory
-    CU(cudaMemcpyAsync(c->rs_tab, img.data(), img.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->rs_tab, img.data(), ybytes + xbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     c->rs_ytab = reinterpret_cast<const int4 *>(c->rs_tab);
     c->rs_xtab = reinterpret_cast<const int2 *>(reinterpret_cast<const char *>(c->rs_tab) + ybytes);
@@ -644,6 +652,95 @@ int yolo_b200_resize_u8bgr(yolo_b200_ctx *c, const uint8_t *d_src, int n, int sh
     CU(resize_u8bgr(d_src, n, sh, sw, d_dst, dh, dw, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream));
     c->launches++;
     return 0;
+}
+
+// A batch of images of different sizes, packed back to back without padding.  (sh, sw) of image i = src_hw[2 * i * stride]
+// and the entry after it: stride 1 reads one size per image, stride 0 gives every image the size src_hw[0..1] (a uniform batch).
+struct RaggedPlan {
+    std::vector<size_t> off;                        // [n + 1]: byte offset of image i in the packed buffer; off[n] = total
+    std::vector<ResizeFrame> frames;                // [n]: what the kernel reads per frame
+    std::vector<std::pair<int, int>> geoms;         // distinct source sizes in order of first appearance
+    std::vector<int4> img;                          // descriptors, then int4 [G][dh] row tables, then int2 [G][dw] column tables
+    size_t ytab_off = 0, xtab_off = 0, img_bytes = 0;
+};
+
+static int ragged_plan(int n, const int32_t *src_hw, int stride, RaggedPlan &p)
+{
+    p.off.assign((size_t)n + 1, 0);
+    p.frames.resize((size_t)n);
+    p.geoms.clear();
+    std::map<std::pair<int, int>, int> index;
+    for (int i = 0; i < n; ++i) {
+        const int sh = src_hw[2 * (size_t)i * stride], sw = src_hw[2 * (size_t)i * stride + 1];
+        if (sh < 1 || sw < 1) return fail(E_ARG, "image %d: bad source shape %dx%d", i, sh, sw);
+        const size_t bytes = (size_t)sh * sw * 3;
+        if (bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "image %d: source image larger than 2 GiB", i);
+        auto it = index.emplace(std::make_pair(sh, sw), (int)p.geoms.size()).first;
+        if (it->second == (int)p.geoms.size()) p.geoms.push_back(it->first);
+        p.frames[i].off = p.off[i]; p.frames[i].pitch = sw * 3; p.frames[i].geom = it->second;
+        p.off[i + 1] = p.off[i] + bytes;
+    }
+    return 0;
+}
+
+// the plan's table image: per distinct size exactly the tables ensure_resize_tables builds
+static void ragged_tables(RaggedPlan &p, int dh, int dw)
+{
+    const size_t G = p.geoms.size();
+    p.ytab_off = p.frames.size() * sizeof(ResizeFrame);
+    p.xtab_off = p.ytab_off + G * dh * sizeof(int4);
+    p.img_bytes = p.xtab_off + G * dw * sizeof(int2);
+    p.img.resize((p.img_bytes + sizeof(int4) - 1) / sizeof(int4));
+    char *b = reinterpret_cast<char *>(p.img.data());
+    memcpy(b, p.frames.data(), p.ytab_off);
+    for (size_t g = 0; g < G; ++g)
+        resize_geometry_tables(p.geoms[g].first, p.geoms[g].second, dh, dw, reinterpret_cast<int4 *>(b + p.ytab_off) + g * dh,
+                               reinterpret_cast<int2 *>(b + p.xtab_off) + g * dw);
+}
+
+static int ensure_pinned(char **p, size_t *cap, size_t need)
+{
+    if (*cap >= need) return 0;
+    if (*p) cudaFreeHost(*p);
+    *p = nullptr; *cap = 0;
+    cudaError_t e = cudaHostAlloc((void **)p, need, cudaHostAllocDefault);
+    if (e != cudaSuccess) return fail(E_NOMEM, "cudaHostAlloc(%zu): %s", need, cudaGetErrorString(e));
+    *cap = need;
+    return 0;
+}
+
+// Ragged resize of the device entry points on the context stream: the plan's tables go to the context-owned buffer in
+// stream order (after every resize queued earlier on the stream has read the previous ones), then one launch.
+static int resize_ragged_dev(yolo_b200_ctx *c, const uint8_t *d_src, int n, RaggedPlan &p, uint8_t *d_dst, int dh, int dw)
+{
+    ragged_tables(p, dh, dw);
+    const int k = c->rg_next;
+    if (!c->rg_ev[k]) CU(cudaEventCreateWithFlags(&c->rg_ev[k], cudaEventDisableTiming));
+    CU(cudaEventSynchronize(c->rg_ev[k]));                    // the copy out of this staging buffer two calls ago has run
+    int rc = ensure_pinned(&c->rg_host[k], &c->rg_host_cap[k], p.img_bytes); if (rc) return rc;
+    rc = ensure(&c->rg_tab, &c->rg_tab_cap, p.img_bytes); if (rc) return rc;      // (a cudaFree waits for queued work)
+    memcpy(c->rg_host[k], p.img.data(), p.img_bytes);
+    CU(cudaMemcpyAsync(c->rg_tab, c->rg_host[k], p.img_bytes, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaEventRecord(c->rg_ev[k], c->stream));
+    c->rg_next ^= 1;
+    const char *t = (const char *)c->rg_tab;
+    CU(resize_u8bgr_ragged(d_src, p.off[n], (const ResizeFrame *)t, n, d_dst, dh, dw, (const int2 *)(t + p.xtab_off),
+                           (const int4 *)(t + p.ytab_off), c->sm_count, c->stream));
+    c->launches++;
+    return 0;
+}
+
+int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *d_src, int n, const int32_t *src_hw, uint8_t *d_dst, int dh, int dw)
+{
+    if (!c) return fail(E_ARG, "null ctx");
+    if (n < 0 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d -> %dx%d", n, dh, dw);
+    CU(cudaSetDevice(c->device));
+    if (n == 0) return 0;
+    if (!src_hw) return fail(E_ARG, "null src_hw");
+    RaggedPlan p;
+    int rc = ragged_plan(n, src_hw, 1, p); if (rc) return rc;
+    if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
+    return resize_ragged_dev(c, d_src, n, p, d_dst, dh, dw);
 }
 
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
@@ -1175,6 +1272,20 @@ int yolo_b200_forward_u8bgr_resize_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, i
     return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
 }
 
+int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, int n, const int32_t *src_hw, int h, int w,
+                                       yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    int rc = check_ready(c, n, h, w); if (rc) return rc;
+    if (n == 0) return 0;
+    if (!src_hw) return fail(E_ARG, "null src_hw");
+    RaggedPlan p;
+    rc = ragged_plan(n, src_hw, 1, p); if (rc) return rc;
+    if (!d_bgr || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
+    rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)n * h * w * 3); if (rc) return rc;
+    rc = resize_ragged_dev(c, d_bgr, n, p, c->rs_out, h, w); if (rc) return rc;
+    return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
+}
+
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 { return forward_dev(c, 2, d_nchw, n, h, w, d_dets, d_counts); }
 
@@ -1191,22 +1302,38 @@ int yolo_b200_sync(yolo_b200_ctx *c)
 // chunking changes no result); every chunk's prediction map lands in one batch-wide buffer and decode + NMS then run once
 // over the whole batch (a per-chunk NMS launch cannot fill the GPU: it is one CTA per frame).  Only the filled part of the
 // detection lists is copied back.
-// sh, sw > 0 (kind 3 only): the host images are sh x sw and are resized to h x w on the GPU chunk by chunk, between the
-// copy and the first layer (in_bytes = bytes of the source images).
+// src_hw != nullptr (kind 3 only): the host images have the source sizes src_hw (ragged_plan: stride 0 = one size for all),
+// are packed back to back and are resized to h x w on the GPU chunk by chunk, between the copy and the first layer; chunk
+// k's copy is the byte range [off[f0], off[f0 + nk]) of the packed images.  One source size takes the uniform kernel and the
+// context's cached tables (no resize at all when it is h x w); several take the ragged kernel with the descriptors and
+// tables of this call in the slot's own buffers, uploaded on the copy stream (the slot's previous call has completed, so
+// nothing queued still reads them).
 // host_enqueue queues the whole call (copies in, layers, decode + NMS, copy of the counts) on the context's streams and
 // returns; host_complete waits for the counts, copies the filled part of the lists back and waits for that copy.
 static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, int sh = 0, int sw = 0)
+                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1)
 {
     HostSlot &S = c->slots[si];
     S.ngroups = 0; S.dets = dets; S.counts = counts;
-    const bool resize = sh > 0 && sw > 0 && !(sh == h && sw == w);
-    const size_t net_frame_bytes = resize ? (size_t)h * w * 3 : in_bytes / (size_t)n;
-    int rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
+    RaggedPlan rp;
+    int rc;
+    if (src_hw) { rc = ragged_plan(n, src_hw, hw_stride, rp); if (rc) return rc; }
+    const bool resize = src_hw && !(rp.geoms.size() == 1 && rp.geoms[0] == std::make_pair(h, w));
+    const bool ragged = resize && rp.geoms.size() > 1;
+    const size_t frame_bytes = src_hw ? 0 : in_bytes / (size_t)n;
+    auto src_off = [&](int f) { return src_hw ? rp.off[f] : (size_t)f * frame_bytes; };     // byte offset of frame f in host_in
+    const size_t net_frame_bytes = src_hw ? (size_t)h * w * 3 : frame_bytes;
+    rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
     if (resize) {
-        if ((size_t)sh * sw * 3 > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "source image larger than 2 GiB");
-        rc = ensure(&S.rs_src, &S.rs_src_cap, in_bytes); if (rc) return rc;
-        rc = ensure_resize_tables(c, sh, sw, h, w); if (rc) return rc;
+        rc = ensure(&S.rs_src, &S.rs_src_cap, rp.off[n]); if (rc) return rc;
+        if (ragged) {
+            ragged_tables(rp, h, w);
+            rc = ensure(&S.rg_tab, &S.rg_tab_cap, rp.img_bytes); if (rc) return rc;
+            rc = ensure_pinned(&S.rg_host, &S.rg_host_cap, rp.img_bytes); if (rc) return rc;
+            memcpy(S.rg_host, rp.img.data(), rp.img_bytes);
+        } else {
+            rc = ensure_resize_tables(c, rp.geoms[0].first, rp.geoms[0].second, h, w); if (rc) return rc;
+        }
     }
     const size_t md = (size_t)c->prm.max_det;
     rc = ensure((void **)&S.d_dets, &S.dets_cap, (size_t)n * md * sizeof(yolo_b200_det)); if (rc) return rc;
@@ -1233,7 +1360,6 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
         for (int f = 0; f < n; f += chunk) { cf0.push_back(f); cnk.push_back((n - f) < chunk ? (n - f) : chunk); }
     }
     const int nchunks = (int)cf0.size();
-    const size_t frame_bytes = in_bytes / (size_t)n;
     const size_t N = (size_t)gh * gw * c->prm.num_anchors;
     if (N > (size_t)HEAD_MAX_CAND) return fail(E_UNSUPPORTED, "grid %dx%d x %d anchors exceeds %d candidates per frame", gh, gw, c->prm.num_anchors, HEAD_MAX_CAND);
     rc = ensure_head(c, (size_t)n, N); if (rc) return rc;
@@ -1264,6 +1390,8 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
     tr.ev.clear();
     tr.on = getenv("YOLO_B200_TRACE_HOST") != nullptr;
     if (tr.on) { cudaEventCreate(&tr.t0); cudaEventRecord(tr.t0, c->s_in); }
+    if (ragged) CU(cudaMemcpyAsync(S.rg_tab, S.rg_host, rp.img_bytes, cudaMemcpyHostToDevice, c->s_in));
+    const char *rg = (const char *)S.rg_tab;
     // The slot's buffers are its own: nothing queued earlier reads or writes them once the slot's previous call has been
     // completed, so the copies of this call do NOT wait for the context stream (the layers of the previous call may still
     // be running there: that overlap is the point of the second slot).
@@ -1276,13 +1404,16 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
     for (int k = 0; k < nchunks; ++k) {
         const int f0 = cf0[k], nk = cnk[k];
         char *stage = (char *)S.stage_in + (size_t)f0 * net_frame_bytes;
-        char *land = resize ? (char *)S.rs_src + (size_t)f0 * frame_bytes : stage;
-        CU(cudaMemcpyAsync(land, (const char *)host_in + (size_t)f0 * frame_bytes, (size_t)nk * frame_bytes, cudaMemcpyHostToDevice, c->s_in));
+        char *land = resize ? (char *)S.rs_src + src_off(f0) : stage;
+        CU(cudaMemcpyAsync(land, (const char *)host_in + src_off(f0), src_off(f0 + nk) - src_off(f0), cudaMemcpyHostToDevice, c->s_in));
         CU(cudaEventRecord(S.ev_in[k], c->s_in));
         tr.mark("h2d done", k, c->s_in);
         CU(cudaStreamWaitEvent(c->stream, S.ev_in[k], 0));
         if (resize) {
-            cudaError_t e = resize_u8bgr((const uint8_t *)land, nk, sh, sw, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream);
+            // the ragged kernel reads the call's buffer up to the end of this chunk's landed bytes, never into a later chunk
+            cudaError_t e = ragged ? resize_u8bgr_ragged((const uint8_t *)S.rs_src, rp.off[f0 + nk], (const ResizeFrame *)rg + f0, nk, (uint8_t *)stage, h, w,
+                                                         (const int2 *)(rg + rp.xtab_off), (const int4 *)(rg + rp.ytab_off), c->sm_count, c->stream)
+                                   : resize_u8bgr((const uint8_t *)land, nk, rp.geoms[0].first, rp.geoms[0].second, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream);
             if (e != cudaSuccess) { drain(); return fail(E_CUDA, "resize: %s", cudaGetErrorString(e)); }
             c->launches++;
         }
@@ -1343,28 +1474,28 @@ static int host_free_slot(yolo_b200_ctx *c)
 
 // blocking call = submit + wait on any free slot
 static int forward_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, int sh = 0, int sw = 0)
+                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     if (n == 0) return 0;
     if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
     const int si = host_free_slot(c);
     if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, sh, sw); if (rc) return rc;
+    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride); if (rc) return rc;
     return host_complete(c, si);
 }
 
 // asynchronous pair: returns a ticket (>= 0) once the call is queued; the caller's buffers belong to the library until
 // yolo_b200_wait(ticket) returns
 static int submit_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                       yolo_b200_det *dets, int32_t *counts)
+                       yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     if (n < 1) return fail(E_ARG, "submit needs n >= 1");
     if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
     const int si = host_free_slot(c);
     if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts); if (rc) return rc;
+    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw); if (rc) return rc;
     return si;
 }
 
@@ -1372,6 +1503,12 @@ int yolo_b200_submit_rgb444(yolo_b200_ctx *c, const uint16_t *frames, int n, int
 { return submit_host(c, frames, (size_t)n * h * w * 2, 0, n, h, w, dets, counts); }
 int yolo_b200_submit_u8bgr(yolo_b200_ctx *c, const uint8_t *bgr, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
 { return submit_host(c, bgr, (size_t)n * h * w * 3, 3, n, h, w, dets, counts); }
+int yolo_b200_submit_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
+                                  yolo_b200_det *dets, int32_t *counts)
+{
+    if (!src_hw && n > 0) return fail(E_ARG, "null src_hw");
+    return submit_host(c, bgr, 0, 3, n, h, w, dets, counts, src_hw);
+}
 int yolo_b200_wait(yolo_b200_ctx *c, int ticket)
 {
     if (!c) return fail(E_ARG, "null ctx");
@@ -1391,7 +1528,14 @@ int yolo_b200_forward_f32(yolo_b200_ctx *c, const float *nchw, int n, int h, int
 int yolo_b200_forward_u8bgr_resize(yolo_b200_ctx *c, const uint8_t *bgr, int n, int sh, int sw, int h, int w, yolo_b200_det *dets, int32_t *counts)
 {
     if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
-    return forward_host(c, bgr, (size_t)n * sh * sw * 3, 3, n, h, w, dets, counts, sh, sw);
+    const int32_t hw[2] = { sh, sw };
+    return forward_host(c, bgr, (size_t)n * sh * sw * 3, 3, n, h, w, dets, counts, hw, 0);
+}
+int yolo_b200_forward_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
+                                   yolo_b200_det *dets, int32_t *counts)
+{
+    if (!src_hw && n > 0) return fail(E_ARG, "null src_hw");
+    return forward_host(c, bgr, 0, 3, n, h, w, dets, counts, src_hw);
 }
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------

@@ -35,6 +35,8 @@ EXPORTS = [
     "yolo_b200_pack_detections", "yolo_b200_ipc_alloc", "yolo_b200_ipc_open", "yolo_b200_ipc_close", "yolo_b200_copy_async",
     "yolo_b200_submit_rgb444", "yolo_b200_submit_u8bgr", "yolo_b200_wait",
     "yolo_b200_resize_taps", "yolo_b200_resize_u8bgr", "yolo_b200_forward_u8bgr_resize", "yolo_b200_forward_u8bgr_resize_dev",
+    "yolo_b200_resize_u8bgr_ragged", "yolo_b200_forward_u8bgr_ragged", "yolo_b200_submit_u8bgr_ragged",
+    "yolo_b200_forward_u8bgr_ragged_dev",
 ]
 
 
@@ -103,6 +105,9 @@ def load_library(path: Optional[str] = None):
     L.yolo_b200_resize_taps.argtypes = [i32, i32, i32, vp]
     L.yolo_b200_forward_u8bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp]
     L.yolo_b200_forward_u8bgr_resize_dev.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp]
+    L.yolo_b200_resize_u8bgr_ragged.argtypes = [vp, vp, i32, vp, vp, i32, i32]
+    for name in ("yolo_b200_forward_u8bgr_ragged", "yolo_b200_submit_u8bgr_ragged", "yolo_b200_forward_u8bgr_ragged_dev"):
+        getattr(L, name).argtypes = [vp, vp, i32, vp, i32, i32, vp, vp]
     L.yolo_b200_quantize_rgb444.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_quantize_f32.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_rgb444_lut.argtypes = [vp, vp]
@@ -166,6 +171,20 @@ def _ptr(x):
     if isinstance(x, np.ndarray):
         return x.ctypes.data
     return x.data_ptr()        # torch.Tensor
+
+
+def pack_images(images) -> "tuple[np.ndarray, np.ndarray]":
+    """A list of uint8 BGR images [h][w][3] of any sizes (what cv2.imread returns) -> (flat uint8 buffer with the images
+    back to back, int32 [n][2] of their (h, w)): the input of the *_ragged entry points."""
+    shapes = np.zeros((len(images), 2), dtype=np.int32)
+    for i, im in enumerate(images):
+        if not isinstance(im, np.ndarray) or im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3:
+            raise ValueError("image %d: need a uint8 array [h][w][3], got %s %s" % (i, getattr(im, "dtype", type(im)), getattr(im, "shape", "")))
+        if not im.flags.c_contiguous:
+            raise ValueError("image %d is not C-contiguous" % i)
+        shapes[i] = im.shape[:2]
+    flat = np.concatenate([im.reshape(-1) for im in images]) if len(images) else np.zeros(0, dtype=np.uint8)
+    return flat, shapes
 
 
 class Context:
@@ -283,6 +302,29 @@ class Context:
         self._check(self.L.yolo_b200_forward_u8bgr_resize(self._h, f.ctypes.data, n, sh, sw, h, w, dets.ctypes.data, counts.ctypes.data))
         return dets, counts
 
+    def forward_u8bgr_images(self, images, size):
+        """A list of uint8 BGR images of any sizes (cv2.imread arrays) -> (dets [n][max_det], counts [n]) in one call: the
+        whole BaseTransform (resize to size = (h, w) included) + forward pass on the GPU.  Boxes are normalised: image i
+        scales them by its own [w, h, w, h]."""
+        flat, shapes = pack_images(images)
+        n, md = len(shapes), self.params.max_det
+        dets = np.zeros((n, md), dtype=DET_DTYPE)
+        counts = np.zeros(n, dtype=np.int32)
+        self._check(self.L.yolo_b200_forward_u8bgr_ragged(self._h, flat.ctypes.data, n, shapes.ctypes.data, int(size[0]), int(size[1]),
+                                                          dets.ctypes.data, counts.ctypes.data))
+        return dets, counts
+
+    def submit_u8bgr_images(self, packed, shapes: np.ndarray, size, dets: np.ndarray, counts: np.ndarray) -> int:
+        """Queue one batch of packed images (pack_images; `packed` a numpy array or a pinned torch tensor) for size = (h, w);
+        packed, dets [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until wait(ticket)."""
+        shapes = np.ascontiguousarray(shapes, dtype=np.int32)
+        assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= len(shapes) and len(counts) >= len(shapes)
+        t = self.L.yolo_b200_submit_u8bgr_ragged(self._h, _ptr(packed), len(shapes), shapes.ctypes.data, int(size[0]), int(size[1]),
+                                                 dets.ctypes.data, counts.ctypes.data)
+        if t < 0:
+            self._check(t)
+        return t
+
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
@@ -310,6 +352,17 @@ class Context:
 
     def forward_u8bgr_resize_dev(self, d_in, n, sh, sw, h, w, d_dets, d_counts):
         self._check(self.L.yolo_b200_forward_u8bgr_resize_dev(self._h, _ptr(d_in), n, sh, sw, h, w, _ptr(d_dets), _ptr(d_counts)))
+
+    def forward_u8bgr_ragged_dev(self, d_in, shapes, h, w, d_dets, d_counts):
+        """Packed images of different sizes in device memory; shapes: host int32 [n][2] (pack_images)."""
+        shapes = np.ascontiguousarray(shapes, dtype=np.int32).reshape(-1, 2)
+        self._check(self.L.yolo_b200_forward_u8bgr_ragged_dev(self._h, _ptr(d_in), len(shapes), shapes.ctypes.data, h, w,
+                                                              _ptr(d_dets), _ptr(d_counts)))
+
+    def resize_u8bgr_ragged(self, d_src, shapes, d_dst, dh, dw):
+        """cv2.resize (bilinear) of packed device images of different sizes (shapes: host int32 [n][2]) into d_dst [n][dh][dw][3]."""
+        shapes = np.ascontiguousarray(shapes, dtype=np.int32).reshape(-1, 2)
+        self._check(self.L.yolo_b200_resize_u8bgr_ragged(self._h, _ptr(d_src), len(shapes), shapes.ctypes.data, _ptr(d_dst), dh, dw))
 
     def resize_u8bgr(self, d_src, n, sh, sw, d_dst, dh, dw):
         """cv2.resize (bilinear) of n uint8 [sh][sw][3] device images into d_dst [n][dh][dw][3]."""
