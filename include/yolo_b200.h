@@ -207,6 +207,28 @@ int yolo_b200_forward_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *bgr, int n
 int yolo_b200_submit_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
                                   yolo_b200_det *dets, int32_t *counts);
 
+/* Camera and video frames in YUV, as decoders and webcams deliver them: each frame is converted to BGR exactly as
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420 / _YUYV) does (BT.601 limited range) and resized exactly as
+ * yolo_b200_forward_u8bgr_resize does, on the GPU, in one pass, chunk by chunk between the copy and the first layer; the
+ * rest is yolo_b200_forward_u8bgr_resize, so the results equal it run on the cvtColor'd frames.  4:2:0 frames cross the
+ * host-to-device link at 1.5 bytes per pixel and YUYV at 2, against 3 for BGR.  Frames use cv2's Mat layout and are packed
+ * at yolo_b200_yuv_frame_bytes() with no padding (frame i at byte i * frame_bytes):
+ *   NV12: Y plane sh x sw, then sh/2 rows of sw bytes U,V interleaved           sh, sw even
+ *   I420: Y plane, then the U plane (sh/2) x (sw/2), then the V plane            sh, sw even
+ *   YUYV: sh rows of 2*sw bytes, macropixel Y0 U Y1 V                            sw even
+ * sh == h && sw == w converts without resizing.  Errors: unknown format, odd sizes where the format needs even ones,
+ * n < 0, sh / sw / h / w < 1, null buffers: E_ARG (-1); a frame over 2 GiB: E_UNSUPPORTED (-3).  n == 0 writes nothing.
+ * The submit form is the asynchronous pair of yolo_b200_submit_u8bgr (needs n >= 1; + yolo_b200_wait). */
+#define YOLO_B200_YUV_NV12  0
+#define YOLO_B200_YUV_I420  1
+#define YOLO_B200_YUV_YUYV  2
+/* Bytes of one frame of this format and size (host only, no GPU needed), or a negative error as above. */
+int yolo_b200_yuv_frame_bytes(int format, int sh, int sw);
+int yolo_b200_forward_yuv(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                          yolo_b200_det *dets, int32_t *counts);
+int yolo_b200_submit_yuv(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                         yolo_b200_det *dets, int32_t *counts);
+
 /* Replaces SlimYOLOv2_quantize_bnfuse.forward(x, quantization=True) inference branch,
  * slim_yolo_v2.py:212-358, for a float NCHW batch (input quantised by a_tracker_in, :218). */
 int yolo_b200_forward_f32(yolo_b200_ctx *ctx, const float *nchw, int n, int h, int w,
@@ -230,6 +252,9 @@ int yolo_b200_forward_u8bgr_resize_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr,
  * written in stream order on the context stream. */
 int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n, const int32_t *src_hw, int h, int w,
                                        yolo_b200_det *d_dets, int32_t *d_counts);
+/* YUV frames in device memory (layout and errors as yolo_b200_forward_yuv). */
+int yolo_b200_forward_yuv_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
+                              yolo_b200_det *d_dets, int32_t *d_counts);
 
 int yolo_b200_sync(yolo_b200_ctx *ctx);
 
@@ -257,6 +282,11 @@ int yolo_b200_resize_u8bgr(yolo_b200_ctx *ctx, const uint8_t *d_src, int n, int 
  * Errors as yolo_b200_forward_u8bgr_ragged; n == 0 writes nothing. */
 int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *d_src, int n, const int32_t *src_hw,
                                   uint8_t *d_dst, int dh, int dw);
+/* The front end of yolo_b200_forward_yuv as a stage: n YUV frames (layout as there) -> uint8 BGR [n][dh][dw][3], equal to
+ * cv2.resize(cv2.cvtColor(frame, code), (dw, dh)); one kernel launch, nothing written at source resolution.  Needs no
+ * loaded network; no alignment requirement (d_dst 4-byte aligned and dw a multiple of 4 take word stores). */
+int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int format, int n, int sh, int sw,
+                                uint8_t *d_dst, int dh, int dw);
 /* Host only (no GPU needed), for tests: the per-index programme of that resize along one axis, taps[4*d + {0,1,2,3}] =
  * (source index 0, source index 1, weight 0, weight 1), weights in units of 1/2048; horizontal != 0 re-anchors the tap
  * at the image border as OpenCV's horizontal pass does. */

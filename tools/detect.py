@@ -7,6 +7,7 @@ BaseTransform does, data/__init__.py:36) is normalised, quantised, convolved, de
     python tools/detect.py --trained_model slim_yolo_v2_retune_quantize1.pth --images dir/ -size 416 --out output/
     python tools/detect.py --trained_model random --images synthetic:4          (no checkpoint / no images at hand)
     python tools/detect.py --trained_model ckpt.pth --video clip.avi --batch 32  (demo.py's video / camera modes, batched)
+    python tools/detect.py --yuv clip.nv12 --yuv_format nv12 --yuv_size 1920x1080   (raw decoder / webcam frames)
 """
 import argparse
 import glob
@@ -76,6 +77,61 @@ def run_video(ctx, args, size):
     print("%d frames, %.1f ms in yolo_b200_forward_u8bgr_resize (%.0f frames/s incl. copies)" % (frames, 1e3 * t_dev, frames / max(t_dev, 1e-9)))
 
 
+YUV_FORMATS = {"nv12": lib.YUV_NV12, "i420": lib.YUV_I420, "yuyv": lib.YUV_YUYV}
+YUV_CV2 = {"nv12": cv2.COLOR_YUV2BGR_NV12, "i420": cv2.COLOR_YUV2BGR_I420, "yuyv": cv2.COLOR_YUV2BGR_YUYV}
+
+
+def run_yuv(ctx, args, size):
+    """Raw video as `ffmpeg -f rawvideo -pix_fmt {nv12,yuv420p,yuyv422}` writes it (frames back to back, no header): each
+    batch of --batch frames goes to the GPU as it is (1.5 or 2 bytes per pixel, pinned), is converted to BGR, resized,
+    normalised, quantised, convolved, decoded and NMS-ed there (yolo_b200_submit_yuv), with two batches in flight.  The
+    host converts with cvtColor only to draw <out>/detections.avi (MJPG, the source size, --yuv_fps)."""
+    fmt = YUV_FORMATS[args.yuv_format]
+    try:
+        sw, sh = (int(v) for v in args.yuv_size.lower().split("x"))
+        shape = lib.yuv_frame_shape(fmt, sh, sw)
+    except ValueError as e:
+        raise SystemExit("--yuv_size %s: %s" % (args.yuv_size, e))
+    fbytes = int(np.prod(shape))
+    md = 1024
+    os.makedirs(args.out, exist_ok=True)
+    writer = cv2.VideoWriter(os.path.join(args.out, "detections.avi"), cv2.VideoWriter_fourcc(*"MJPG"), args.yuv_fps, (sw, sh))
+    state = {"frames": 0}
+
+    def finish(job):
+        ticket, frames, dets, counts = job
+        ctx.wait(ticket)
+        for k in range(len(frames)):
+            boxes, scores, cls, _ = lib.dets_to_arrays(dets[k], int(min(counts[k], md)))
+            bgr = cv2.cvtColor(frames[k].numpy(), YUV_CV2[args.yuv_format])                 # for drawing only
+            writer.write(vis(bgr, boxes * np.array([[sw, sh, sw, sh]], dtype=np.float32), scores, cls, args.visual_threshold))
+            print("frame %d: %d detections" % (state["frames"], len(scores)))
+            state["frames"] += 1
+
+    t0, inflight = time.time(), []
+    with open(args.yuv, "rb") as f:
+        while True:
+            want = args.batch if not args.max_frames else min(args.batch, args.max_frames - state["frames"] - sum(len(j[1]) for j in inflight))
+            if want <= 0:
+                break
+            raw = f.read(want * fbytes)
+            n = len(raw) // fbytes
+            if n == 0:
+                break
+            frames = torch.from_numpy(np.frombuffer(raw[:n * fbytes], dtype=np.uint8).reshape((n,) + shape).copy()).pin_memory()
+            dets = np.zeros((n, md), dtype=lib.DET_DTYPE)
+            counts = np.zeros(n, dtype=np.int32)
+            if len(inflight) == 2:
+                finish(inflight.pop(0))
+            inflight.append((ctx.submit_yuv(frames, fmt, size, dets, counts), frames, dets, counts))
+            if n < want:
+                break
+    while inflight:
+        finish(inflight.pop(0))
+    writer.release()
+    print("%d frames, %.1f ms reading, detecting and writing (yolo_b200_submit_yuv / yolo_b200_wait)" % (state["frames"], 1e3 * (time.time() - t0)))
+
+
 def main():
     ap = argparse.ArgumentParser(description="slim_yolo_v2 fixed-point detection on B200")
     ap.add_argument("-v", "--version", default="slim_yolo_v2_q_bf", help="only slim_yolo_v2_q_bf runs on this path")
@@ -87,7 +143,11 @@ def main():
     ap.add_argument("--cuda", action="store_true", default=True, help="kept for compatibility: this path always runs on CUDA")
     ap.add_argument("--images", default="synthetic:2", help="directory / glob of images, or synthetic:N")
     ap.add_argument("--video", default=None, help="video file (demo.py --mode video, :123-158) or camera index (--mode camera, :60-96): frames are batched, detected on the GPU and written, annotated, to <out>/detections.avi")
-    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video run after this many frames (0 = to the end)")
+    ap.add_argument("--yuv", default=None, help="raw YUV video file (ffmpeg -f rawvideo): frames are detected on the GPU straight from YUV and written, annotated, to <out>/detections.avi")
+    ap.add_argument("--yuv_format", default="nv12", choices=sorted(YUV_FORMATS), help="pixel format of --yuv: nv12, i420 (ffmpeg yuv420p) or yuyv (yuyv422)")
+    ap.add_argument("--yuv_size", default=None, help="frame size of --yuv as WxH, e.g. 640x480")
+    ap.add_argument("--yuv_fps", default=25.0, type=float, help="frame rate written to detections.avi in --yuv mode")
+    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video / --yuv run after this many frames (0 = to the end)")
     ap.add_argument("--out", default="output")
     ap.add_argument("--batch", default=64, type=int)
     args = ap.parse_args()
@@ -102,6 +162,12 @@ def main():
     ctx = lib.Context(0)
     ctx.load_quantnet(qnet, contract=lib.CONTRACT_P, head_mode=lib.HEAD_PYTHON, conf_thresh=args.conf_thresh,
                       nms_thresh=args.nms_thresh, max_det=1024)
+    if args.yuv is not None:
+        if not args.yuv_size:
+            raise SystemExit("--yuv needs --yuv_size WxH")
+        run_yuv(ctx, args, size)
+        ctx.close()
+        return
     if args.video is not None:
         run_video(ctx, args, size)
         ctx.close()

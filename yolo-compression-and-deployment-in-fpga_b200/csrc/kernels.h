@@ -97,6 +97,12 @@ void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xt
 struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
 cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames_dev, int n, uint8_t *dst, int dh, int dw,
                                 const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
+// YUV frames (format = YOLO_B200_YUV_*: NV12, I420, YUYV in cv2's Mat layout, packed at yuv_frame_bytes) -> BGR as
+// cv2.cvtColor does, resized as resize_u8bgr does, in one pass with the same tables: uint8 [n][dh][dw][3]
+enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YUV_YUYV = YOLO_B200_YUV_YUYV, RS_BGR = 3 };
+size_t yuv_frame_bytes(int format, int sh, int sw);        // 0 for an unknown format
+cudaError_t resize_yuv_u8bgr(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
+                             const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
 
 // head.cu
 struct HeadArgs {

@@ -85,10 +85,23 @@ __device__ __forceinline__ unsigned resize_combine(unsigned lo0, unsigned hi0, u
     return o[0] | (o[1] << 8) | (o[2] << 16);
 }
 
+// The store of one 32-pixel chunk (v = B | G << 8 | R << 16 of this lane's pixel).  WORD_STORE: the 32 three-byte pixels
+// of a full warp are regrouped by two shuffles into 24 aligned 32-bit stores (output word j = bytes 4j .. 4j+3 of the
+// chunk = pixels p = 4j/3 and p + 1 from byte rsh/8 of p); partial chunks and other geometries store bytes.
+template <bool WORD_STORE>
+__device__ __forceinline__ void resize_store(unsigned v, bool live, int dx0, int dx, int dw, uint8_t *__restrict__ drow, int lane, int p, unsigned rsh)
+{
+    if (WORD_STORE && dx0 + 32 <= dw) {
+        const unsigned va = __shfl_sync(0xffffffffu, v, p & 31), vb = __shfl_sync(0xffffffffu, v, (p + 1) & 31);
+        const unsigned word = __funnelshift_r(va | (vb << 24), vb >> 8, rsh);
+        if (lane < 24) reinterpret_cast<unsigned *>(drow)[(dx0 >> 5) * 24 + lane] = word;
+    } else if (live) {
+        uint8_t *o = drow + (size_t)dx * 3;
+        o[0] = (uint8_t)v; o[1] = (uint8_t)(v >> 8); o[2] = (uint8_t)(v >> 16);
+    }
+}
+
 // One output row of the batch: one thread = one output pixel, a warp = 32 consecutive pixels = 96 contiguous output bytes.
-// WORD_STORE: the 32 three-byte pixels of a full warp are regrouped by two shuffles into 24 aligned 32-bit stores
-// (output word j = bytes 4j .. 4j+3 of the chunk = pixels p = 4j/3 and p + 1 from byte rsh/8 of p); partial chunks and other
-// geometries store bytes.
 template <bool WORD_STORE, bool CLAMP>
 __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__ r0, const unsigned char *__restrict__ r1,
                                                unsigned d0, unsigned d1, unsigned lim0, unsigned lim1, unsigned B0, unsigned B1,
@@ -106,16 +119,104 @@ __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__
             resize_row_taps<CLAMP>(r1, (unsigned)xt.x + d1, lim1, lo1, hi1);
             v = resize_combine(lo0, hi0, lo1, hi1, (unsigned)xt.y, B0, B1);
         }
-        if (WORD_STORE && dx0 + 32 <= dw) {
-            const unsigned va = __shfl_sync(0xffffffffu, v, p & 31), vb = __shfl_sync(0xffffffffu, v, (p + 1) & 31);
-            const unsigned word = __funnelshift_r(va | (vb << 24), vb >> 8, rsh);
-            if (lane < 24) reinterpret_cast<unsigned *>(drow)[(dx0 >> 5) * 24 + lane] = word;
-        } else if (live) {
-            uint8_t *o = drow + (size_t)dx * 3;
-            o[0] = (uint8_t)v; o[1] = (uint8_t)(v >> 8); o[2] = (uint8_t)(v >> 16);
-        }
+        resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
     }
 }
+
+// ---- YUV sources: cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420 / _YUYV) fused in front of the resize -------------------------
+// OpenCV's 8-bit YUV -> RGB (BT.601 limited range, 20-bit fixed point, modules/imgproc/src/color_yuv.simd.hpp):
+//   y = max(Y - 16, 0) * 1220542;  u = U - 128;  v = V - 128
+//   R = sat8((y + 2^19 + 1673527 v) >> 20);  G = sat8((y + 2^19 - 852492 v - 409993 u) >> 20);  B = sat8((y + 2^19 + 2116026 u) >> 20)
+// with an arithmetic (floor) shift; every sum stays below 6e8 in magnitude, so int32 is exact.  Chroma is nearest:
+// one U,V pair per 2x2 block (4:2:0) or per horizontal pixel pair (4:2:2).  Returns B | G << 8 | R << 16.
+__device__ __forceinline__ unsigned yuv_to_bgr(unsigned Y, unsigned U, unsigned V)
+{
+    const int y = max((int)Y - 16, 0) * 1220542 + (1 << 19);
+    const int u = (int)U - 128, v = (int)V - 128;
+    const int r = (y + 1673527 * v) >> 20, g = (y - 852492 * v - 409993 * u) >> 20, b = (y + 2116026 * u) >> 20;
+    return (unsigned)min(max(b, 0), 255) | ((unsigned)min(max(g, 0), 255) << 8) | ((unsigned)min(max(r, 0), 255) << 16);
+}
+
+// One source row r of a YUV frame: where its luma and the chroma it uses start (cv2 Mat layouts, no padding).
+//   NV12: Y plane sh x sw, then sh/2 rows of sw bytes U,V,U,V...  -> y = row r, u = interleaved chroma row r/2 (v unused)
+//   I420: Y plane, U plane (sh/2) x (sw/2), V plane              -> y, u, v = row r, r/2, r/2 of their planes
+//   YUYV: sh rows of 2*sw bytes, macropixel Y0 U Y1 V             -> y = row r (u, v unused)
+struct YuvRow { const uint8_t *y, *u, *v; };
+
+template <int FMT>
+__device__ __forceinline__ YuvRow yuv_row(const uint8_t *frame, unsigned r, int sh, int sw)
+{
+    const size_t plane = (size_t)sh * sw, c = r >> 1;         // the chroma row is warp-uniform: r is the row's tap
+    if (FMT == RS_YUV_NV12) return { frame + (size_t)r * sw, frame + plane + c * sw, nullptr };
+    if (FMT == RS_YUV_I420) return { frame + (size_t)r * sw, frame + plane + c * (sw >> 1), frame + plane + plane / 4 + c * (sw >> 1) };
+    return { frame + (size_t)r * 2 * sw, nullptr, nullptr };
+}
+
+// B | G << 8 | R << 16 of source pixel x of the row
+template <int FMT>
+__device__ __forceinline__ unsigned yuv_pixel(const YuvRow &row, unsigned x)
+{
+    if (FMT == RS_YUV_NV12) return yuv_to_bgr(__ldg(row.y + x), __ldg(row.u + (x & ~1u)), __ldg(row.u + (x | 1u)));
+    if (FMT == RS_YUV_I420) return yuv_to_bgr(__ldg(row.y + x), __ldg(row.u + (x >> 1)), __ldg(row.v + (x >> 1)));
+    const uint8_t *m = row.y + 2 * (x & ~1u);                 // the macropixel of x
+    return yuv_to_bgr(__ldg(row.y + 2 * x), __ldg(m + 1), __ldg(m + 3));
+}
+
+// A row's 6-byte window in the BGR kernel's form (tap 0 = bytes 0..2, tap 1 = bytes 3..5), converted from YUV.  Tap 1 is
+// pixel x0 + 1 except at the right border, where the horizontal table gives tap 1 weight 0 (resize_axis_table re-anchors
+// it); there the window takes pixel sw - 1 instead, so no byte left of column 0 or right of column sw - 1 is ever read.
+template <int FMT>
+__device__ __forceinline__ void yuv_row_taps(const YuvRow &row, unsigned x0, unsigned x1, unsigned &lo, unsigned &hi)
+{
+    const unsigned p0 = yuv_pixel<FMT>(row, x0), p1 = yuv_pixel<FMT>(row, x1);
+    lo = p0 | (p1 << 24);
+    hi = p1 >> 8;
+}
+
+// The YUV form of resize_u8c3_kernel's row loop: frames of frame_bytes bytes at a uniform stride, the uniform row / column
+// tables (xtab's byte offsets are 3 * source column), resize_combine and the same stores.
+// Bounds: a source row index comes from ytab (clamped to [0, sh - 1]), a column from xtab (in [0, sw - 1]) or its clamped
+// successor, so with sh, sw even where the format subsamples every byte read (luma, chroma row r/2 <= sh/2 - 1, chroma
+// column x/2 <= sw/2 - 1) lies inside its own frame, and frames are those of this launch: nothing is read past
+// src + n * frame_bytes.  In the chunked host path that is the end of the chunk's landed bytes.  Loads are bytes (a warp's
+// lanes are ~1.5 luma bytes apart for 640 -> 416, so each byte load touches one or two 128-byte lines), so there is no
+// aligned word that could straddle the end and no clamped-row variant.
+template <bool WORD_STORE, int FMT>
+__device__ __forceinline__ void resize_yuv_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
+                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+{
+    const int p = (4 * lane) / 3;
+    const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
+    const size_t plane = (size_t)sh * sw, frame_bytes = FMT == RS_YUV_YUYV ? 2 * plane : plane + plane / 2;
+    unsigned dy = row % (unsigned)dh;
+    const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
+    uint8_t *drow = dst + (size_t)row * dw * 3;
+    for (; row < row_end; ++row) {
+        const int4 yt = __ldg(ytab + dy);
+        const YuvRow r0 = yuv_row<FMT>(frame, (unsigned)yt.x, sh, sw), r1 = yuv_row<FMT>(frame, (unsigned)yt.y, sh, sw);
+        for (int dx0 = 0; dx0 < dw; dx0 += 32) {
+            const int dx = dx0 + lane;
+            const bool live = dx < dw;
+            unsigned v = 0;
+            if (live) {
+                const int2 xt = __ldg(xtab + dx);
+                const unsigned x0 = (unsigned)xt.x / 3u, x1 = min(x0 + 1u, (unsigned)sw - 1u);
+                unsigned lo0, hi0, lo1, hi1;
+                yuv_row_taps<FMT>(r0, x0, x1, lo0, hi0);
+                yuv_row_taps<FMT>(r1, x0, x1, lo1, hi1);
+                v = resize_combine(lo0, hi0, lo1, hi1, (unsigned)xt.y, (unsigned)yt.z, (unsigned)yt.w);
+            }
+            resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
+        }
+        drow += (size_t)dw * 3;
+        if (++dy == (unsigned)dh) { dy = 0; frame += frame_bytes; }
+    }
+}
+
+// resident CTAs of 256 threads per SM the launch plans for (= the kernel's __launch_bounds__): 6 at 40 registers; the
+// ragged descriptor bookkeeping needs 48 (5 CTAs) and the 4:2:0 instantiations, which keep luma and chroma row pointers of
+// both source rows, up to 64 (4 CTAs) to run without spills; YUYV fits 40
+constexpr int resize_ctas_per_sm(bool ragged, int fmt) { return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 ? 4 : 6; }
 
 // One WARP = a contiguous run of output rows of the batch (so the row bookkeeping is incremental: no divisions), one
 // whole row at a time, chunk after chunk: the ~70 instructions of row bookkeeping are paid once per row, not once per
@@ -126,8 +227,9 @@ __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__
 // frames[f] = {byte offset in src, row pitch, geometry g}; its row / column tables are ytab + g * dh / xtab + g * dw.  The
 // descriptor is loaded when dy wraps, so its cost is warp-uniform and paid once per frame.  Otherwise frames are
 // sh x sw and packed at a uniform stride.
-template <bool WORD_STORE, bool RAGGED>
-__global__ void __launch_bounds__(256, RAGGED ? 5 : 6) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+// FMT: the source format, RS_BGR (uint8 [sh][sw][3]) or one of the YUV layouts (uniform stride only; resize_yuv_rows).
+template <bool WORD_STORE, bool RAGGED, int FMT = RS_BGR>
+__global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                           const int2 *__restrict__ xtab, const int4 *__restrict__ ytab,
                                                           const ResizeFrame *__restrict__ frames,
                                                           unsigned rows, unsigned rows_per_warp, int sh, int sw, int dh, int dw, size_t src_bytes)
@@ -136,6 +238,11 @@ __global__ void __launch_bounds__(256, RAGGED ? 5 : 6) resize_u8c3_kernel(const 
     unsigned row = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * rows_per_warp;
     if (row >= rows) return;
     const unsigned row_end = min(rows, row + rows_per_warp);
+    if constexpr (FMT != RS_BGR) {
+        static_assert(!RAGGED, "YUV sources are one size per launch");
+        resize_yuv_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        return;
+    }
     const size_t delta = reinterpret_cast<uintptr_t>(src) & 3;                             // word-aligned view of the source
     const unsigned char *base = src - delta;
     const size_t end = delta + src_bytes;                                                  // one past the last source byte
@@ -181,7 +288,7 @@ __global__ void __launch_bounds__(256, RAGGED ? 5 : 6) resize_u8c3_kernel(const 
 }
 
 // one wave of resident CTAs (8 warps each), equal runs of rows per warp
-template <bool RAGGED>
+template <bool RAGGED, int FMT = RS_BGR>
 static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames, int n, int sh, int sw, uint8_t *dst,
                                  int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
 {
@@ -189,15 +296,14 @@ static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const Res
     const size_t rows = (size_t)n * dh;
     if (rows > 0x7fffffffull) return cudaErrorInvalidValue;
     const int threads = 256;
-    // 6 resident CTAs per SM at 40 registers; the ragged variant's descriptor bookkeeping needs 48 (5 CTAs) to run without spills
-    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * (RAGGED ? 5 : 6) * (threads / 32);
+    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * resize_ctas_per_sm(RAGGED, FMT) * (threads / 32);
     const unsigned rows_per_warp = (unsigned)((rows + max_warps - 1) / max_warps);
     const size_t warps = (rows + rows_per_warp - 1) / rows_per_warp;
     const size_t blocks = (warps + threads / 32 - 1) / (threads / 32);
     if ((reinterpret_cast<uintptr_t>(dst) & 3) == 0 && dw % 4 == 0)
-        resize_u8c3_kernel<true, RAGGED><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+        resize_u8c3_kernel<true, RAGGED, FMT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
     else
-        resize_u8c3_kernel<false, RAGGED><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+        resize_u8c3_kernel<false, RAGGED, FMT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
     return cudaGetLastError();
 }
 
@@ -211,6 +317,23 @@ cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const Resi
                                 const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
 {
     return resize_launch<true>(src, src_bytes, frames_dev, n, 0, 0, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+}
+
+size_t yuv_frame_bytes(int format, int sh, int sw)
+{
+    const size_t px = (size_t)sh * sw;
+    return format == RS_YUV_NV12 || format == RS_YUV_I420 ? px + px / 2 : format == RS_YUV_YUYV ? 2 * px : 0;
+}
+
+cudaError_t resize_yuv_u8bgr(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
+                             const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+{
+    switch (format) {
+    case RS_YUV_NV12: return resize_launch<false, RS_YUV_NV12>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_YUV_I420: return resize_launch<false, RS_YUV_I420>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_YUV_YUYV: return resize_launch<false, RS_YUV_YUYV>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    default: return cudaErrorInvalidValue;
+    }
 }
 
 void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab)

@@ -743,6 +743,42 @@ int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *d_src, int n,
     return resize_ragged_dev(c, d_src, n, p, d_dst, dh, dw);
 }
 
+// One YUV frame of (format, sh, sw): its byte count, or E_ARG / E_UNSUPPORTED (include/yolo_b200.h)
+static int yuv_check(int format, int sh, int sw, size_t *bytes)
+{
+    if (format != YOLO_B200_YUV_NV12 && format != YOLO_B200_YUV_I420 && format != YOLO_B200_YUV_YUYV)
+        return fail(E_ARG, "unknown YUV format %d", format);
+    if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
+    if (sw % 2 || (format != YOLO_B200_YUV_YUYV && sh % 2))
+        return fail(E_ARG, "YUV format %d needs an even %s (%dx%d)", format, format == YOLO_B200_YUV_YUYV ? "width" : "height and width", sh, sw);
+    *bytes = yuv_frame_bytes(format, sh, sw);
+    if (*bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "YUV frame larger than 2 GiB");
+    return 0;
+}
+
+int yolo_b200_yuv_frame_bytes(int format, int sh, int sw)
+{
+    size_t b = 0;
+    int rc = yuv_check(format, sh, sw, &b); if (rc) return rc;
+    return (int)b;
+}
+
+// YUV -> BGR + resize on the context stream with the context's cached tables (ensure_resize_tables uploads in stream order)
+int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int format, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+{
+    if (!c) return fail(E_ARG, "null ctx");
+    if (n < 0 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d -> %dx%d", n, dh, dw);
+    size_t fb;
+    int rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    if (n == 0) return 0;
+    if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
+    rc = ensure_resize_tables(c, sh, sw, dh, dw); if (rc) return rc;
+    CU(resize_yuv_u8bgr(d_src, format, n, sh, sw, d_dst, dh, dw, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream));
+    c->launches++;
+    return 0;
+}
+
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
 {
     if (!c || !lut_host) return fail(E_ARG, "null argument");
@@ -1286,6 +1322,19 @@ int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, i
     return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
 }
 
+int yolo_b200_forward_yuv_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
+                              yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    int rc = check_ready(c, n, h, w); if (rc) return rc;
+    size_t fb;
+    rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
+    if (n == 0) return 0;
+    if (!d_frames || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
+    rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)n * h * w * 3); if (rc) return rc;
+    rc = yolo_b200_yuv_to_bgr_resize(c, d_frames, format, n, sh, sw, c->rs_out, h, w); if (rc) return rc;
+    return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
+}
+
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 { return forward_dev(c, 2, d_nchw, n, h, w, d_dets, d_counts); }
 
@@ -1308,31 +1357,36 @@ int yolo_b200_sync(yolo_b200_ctx *c)
 // context's cached tables (no resize at all when it is h x w); several take the ragged kernel with the descriptors and
 // tables of this call in the slot's own buffers, uploaded on the copy stream (the slot's previous call has completed, so
 // nothing queued still reads them).
+// yuv >= 0 (kind 3 only, with src_hw = the one source size, stride 0): the host frames are YUV of that format, packed at
+// in_bytes / n bytes; each chunk's landed frames take one fused YUV -> BGR + resize launch with the context's cached
+// tables (also when the size is h x w: the conversion is needed anyway).
 // host_enqueue queues the whole call (copies in, layers, decode + NMS, copy of the counts) on the context's streams and
 // returns; host_complete waits for the counts, copies the filled part of the lists back and waits for that copy.
 static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1)
+                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
 {
     HostSlot &S = c->slots[si];
     S.ngroups = 0; S.dets = dets; S.counts = counts;
     RaggedPlan rp;
     int rc;
-    if (src_hw) { rc = ragged_plan(n, src_hw, hw_stride, rp); if (rc) return rc; }
-    const bool resize = src_hw && !(rp.geoms.size() == 1 && rp.geoms[0] == std::make_pair(h, w));
-    const bool ragged = resize && rp.geoms.size() > 1;
-    const size_t frame_bytes = src_hw ? 0 : in_bytes / (size_t)n;
-    auto src_off = [&](int f) { return src_hw ? rp.off[f] : (size_t)f * frame_bytes; };     // byte offset of frame f in host_in
+    const bool packed = src_hw && yuv < 0;                       // BGR images at ragged_plan's offsets
+    if (packed) { rc = ragged_plan(n, src_hw, hw_stride, rp); if (rc) return rc; }
+    const bool resize = yuv >= 0 || (packed && !(rp.geoms.size() == 1 && rp.geoms[0] == std::make_pair(h, w)));
+    const bool ragged = packed && resize && rp.geoms.size() > 1;
+    const int sh = yuv >= 0 ? src_hw[0] : packed ? rp.geoms[0].first : 0, sw = yuv >= 0 ? src_hw[1] : packed ? rp.geoms[0].second : 0;
+    const size_t frame_bytes = packed ? 0 : in_bytes / (size_t)n;
+    auto src_off = [&](int f) { return packed ? rp.off[f] : (size_t)f * frame_bytes; };      // byte offset of frame f in host_in
     const size_t net_frame_bytes = src_hw ? (size_t)h * w * 3 : frame_bytes;
     rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
     if (resize) {
-        rc = ensure(&S.rs_src, &S.rs_src_cap, rp.off[n]); if (rc) return rc;
+        rc = ensure(&S.rs_src, &S.rs_src_cap, src_off(n)); if (rc) return rc;
         if (ragged) {
             ragged_tables(rp, h, w);
             rc = ensure(&S.rg_tab, &S.rg_tab_cap, rp.img_bytes); if (rc) return rc;
             rc = ensure_pinned(&S.rg_host, &S.rg_host_cap, rp.img_bytes); if (rc) return rc;
             memcpy(S.rg_host, rp.img.data(), rp.img_bytes);
         } else {
-            rc = ensure_resize_tables(c, rp.geoms[0].first, rp.geoms[0].second, h, w); if (rc) return rc;
+            rc = ensure_resize_tables(c, sh, sw, h, w); if (rc) return rc;
         }
     }
     const size_t md = (size_t)c->prm.max_det;
@@ -1410,10 +1464,12 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
         tr.mark("h2d done", k, c->s_in);
         CU(cudaStreamWaitEvent(c->stream, S.ev_in[k], 0));
         if (resize) {
-            // the ragged kernel reads the call's buffer up to the end of this chunk's landed bytes, never into a later chunk
+            // the ragged kernel reads the call's buffer up to the end of this chunk's landed bytes, never into a later chunk;
+            // the uniform and YUV kernels read only the nk frames at `land`
             cudaError_t e = ragged ? resize_u8bgr_ragged((const uint8_t *)S.rs_src, rp.off[f0 + nk], (const ResizeFrame *)rg + f0, nk, (uint8_t *)stage, h, w,
                                                          (const int2 *)(rg + rp.xtab_off), (const int4 *)(rg + rp.ytab_off), c->sm_count, c->stream)
-                                   : resize_u8bgr((const uint8_t *)land, nk, rp.geoms[0].first, rp.geoms[0].second, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream);
+                          : yuv >= 0 ? resize_yuv_u8bgr((const uint8_t *)land, yuv, nk, sh, sw, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream)
+                                   : resize_u8bgr((const uint8_t *)land, nk, sh, sw, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream);
             if (e != cudaSuccess) { drain(); return fail(E_CUDA, "resize: %s", cudaGetErrorString(e)); }
             c->launches++;
         }
@@ -1474,28 +1530,28 @@ static int host_free_slot(yolo_b200_ctx *c)
 
 // blocking call = submit + wait on any free slot
 static int forward_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1)
+                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     if (n == 0) return 0;
     if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
     const int si = host_free_slot(c);
     if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride); if (rc) return rc;
+    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride, yuv); if (rc) return rc;
     return host_complete(c, si);
 }
 
 // asynchronous pair: returns a ticket (>= 0) once the call is queued; the caller's buffers belong to the library until
 // yolo_b200_wait(ticket) returns
 static int submit_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                       yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr)
+                       yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     if (n < 1) return fail(E_ARG, "submit needs n >= 1");
     if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
     const int si = host_free_slot(c);
     if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw); if (rc) return rc;
+    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride, yuv); if (rc) return rc;
     return si;
 }
 
@@ -1537,6 +1593,23 @@ int yolo_b200_forward_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *bgr, int n, 
     if (!src_hw && n > 0) return fail(E_ARG, "null src_hw");
     return forward_host(c, bgr, 0, 3, n, h, w, dets, counts, src_hw);
 }
+// YUV host frames: the uniform resize pipeline with the fused conversion (host_enqueue, yuv >= 0)
+static int yuv_host(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                    yolo_b200_det *dets, int32_t *counts, bool submit)
+{
+    size_t fb;
+    int rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
+    const int32_t hw[2] = { sh, sw };
+    const size_t bytes = n > 0 ? (size_t)n * fb : 0;
+    return submit ? submit_host(c, frames, bytes, 3, n, h, w, dets, counts, hw, 0, format)
+                  : forward_host(c, frames, bytes, 3, n, h, w, dets, counts, hw, 0, format);
+}
+int yolo_b200_forward_yuv(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                          yolo_b200_det *dets, int32_t *counts)
+{ return yuv_host(c, frames, format, n, sh, sw, h, w, dets, counts, false); }
+int yolo_b200_submit_yuv(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                         yolo_b200_det *dets, int32_t *counts)
+{ return yuv_host(c, frames, format, n, sh, sw, h, w, dets, counts, true); }
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------
 int yolo_b200_pack_detections(yolo_b200_ctx *c, const yolo_b200_det *d_dets, const int32_t *d_counts, int n,

@@ -20,6 +20,7 @@ CONTRACT_F, CONTRACT_P = 0, 1
 ROUND_RNE, ROUND_FLOOR, ROUND_HALF_UP = 0, 1, 2
 WLAYOUT_OIHW, WLAYOUT_OHWI, WLAYOUT_WEIGHT_H = 0, 1, 2
 HEAD_PYTHON, HEAD_C = 0, 1
+YUV_NV12, YUV_I420, YUV_YUYV = 0, 1, 2      # cv2.COLOR_YUV2BGR_NV12 / _I420 / _YUYV frames (yolo_b200_forward_yuv)
 
 EXPORTS = [
     "yolo_b200_abi_version", "yolo_b200_last_error", "yolo_b200_cstride", "yolo_b200_default_params",
@@ -37,6 +38,8 @@ EXPORTS = [
     "yolo_b200_resize_taps", "yolo_b200_resize_u8bgr", "yolo_b200_forward_u8bgr_resize", "yolo_b200_forward_u8bgr_resize_dev",
     "yolo_b200_resize_u8bgr_ragged", "yolo_b200_forward_u8bgr_ragged", "yolo_b200_submit_u8bgr_ragged",
     "yolo_b200_forward_u8bgr_ragged_dev",
+    "yolo_b200_yuv_frame_bytes", "yolo_b200_yuv_to_bgr_resize", "yolo_b200_forward_yuv", "yolo_b200_submit_yuv",
+    "yolo_b200_forward_yuv_dev",
 ]
 
 
@@ -108,6 +111,10 @@ def load_library(path: Optional[str] = None):
     L.yolo_b200_resize_u8bgr_ragged.argtypes = [vp, vp, i32, vp, vp, i32, i32]
     for name in ("yolo_b200_forward_u8bgr_ragged", "yolo_b200_submit_u8bgr_ragged", "yolo_b200_forward_u8bgr_ragged_dev"):
         getattr(L, name).argtypes = [vp, vp, i32, vp, i32, i32, vp, vp]
+    L.yolo_b200_yuv_frame_bytes.argtypes = [i32, i32, i32]
+    L.yolo_b200_yuv_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
+    for name in ("yolo_b200_forward_yuv", "yolo_b200_submit_yuv", "yolo_b200_forward_yuv_dev"):
+        getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.yolo_b200_quantize_rgb444.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_quantize_f32.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_rgb444_lut.argtypes = [vp, vp]
@@ -185,6 +192,27 @@ def pack_images(images) -> "tuple[np.ndarray, np.ndarray]":
         shapes[i] = im.shape[:2]
     flat = np.concatenate([im.reshape(-1) for im in images]) if len(images) else np.zeros(0, dtype=np.uint8)
     return flat, shapes
+
+
+def yuv_frame_shape(fmt: int, sh: int, sw: int) -> "tuple[int, ...]":
+    """The cv2 Mat shape of one YUV frame of source size sh x sw: (sh*3//2, sw) for YUV_NV12 / YUV_I420, (sh, sw, 2) for
+    YUV_YUYV.  Raises ValueError for an unknown format or sizes the format cannot hold (4:2:0 needs even sh and sw, YUYV an
+    even sw)."""
+    if fmt not in (YUV_NV12, YUV_I420, YUV_YUYV):
+        raise ValueError("unknown YUV format %r" % (fmt,))
+    sh, sw = int(sh), int(sw)
+    if sh < 1 or sw < 1 or sw % 2 or (fmt != YUV_YUYV and sh % 2):
+        raise ValueError("YUV format %d cannot hold a %dx%d frame" % (fmt, sh, sw))
+    return (sh * 3 // 2, sw) if fmt != YUV_YUYV else (sh, sw, 2)
+
+
+def yuv_source_size(fmt: int, frame_shape) -> "tuple[int, int]":
+    """(sh, sw) of a YUV frame from its cv2 Mat shape (the inverse of yuv_frame_shape)."""
+    fs = tuple(int(x) for x in frame_shape)
+    size = (fs[0] * 2 // 3, fs[1]) if fmt != YUV_YUYV and len(fs) == 2 else (fs[0], fs[1]) if len(fs) == 3 else None
+    if size is None or yuv_frame_shape(fmt, *size) != fs:
+        raise ValueError("%s is not the shape of a YUV format %r frame" % (fs, fmt))
+    return size
 
 
 class Context:
@@ -325,6 +353,37 @@ class Context:
             self._check(t)
         return t
 
+    def forward_yuv(self, frames: np.ndarray, fmt: int, size):
+        """uint8 YUV frames [n, *yuv_frame_shape(fmt, sh, sw)] (cv2 Mat layout: decoder NV12 / I420, webcam YUYV) ->
+        (dets [n][max_det], counts [n]): cv2.cvtColor to BGR, cv2.resize to size = (h, w) and the rest of
+        forward_u8bgr_resize, all on the GPU; the frames cross the link as they are (1.5 or 2 bytes per pixel)."""
+        f = np.ascontiguousarray(frames, dtype=np.uint8)
+        sh, sw = yuv_source_size(fmt, f.shape[1:])
+        n, md = f.shape[0], self.params.max_det
+        dets = np.zeros((n, md), dtype=DET_DTYPE)
+        counts = np.zeros(n, dtype=np.int32)
+        self._check(self.L.yolo_b200_forward_yuv(self._h, f.ctypes.data, fmt, n, sh, sw, int(size[0]), int(size[1]),
+                                                 dets.ctypes.data, counts.ctypes.data))
+        return dets, counts
+
+    def submit_yuv(self, frames, fmt: int, size, dets: np.ndarray, counts: np.ndarray) -> int:
+        """Queue one batch of YUV frames [n, *yuv_frame_shape] (a C-contiguous numpy array or a pinned torch tensor) for
+        size = (h, w); frames, dets [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until
+        wait(ticket).  Returns the ticket."""
+        shape = tuple(frames.shape)
+        sh, sw = yuv_source_size(fmt, shape[1:])
+        n = shape[0]
+        if isinstance(frames, np.ndarray):
+            assert frames.dtype == np.uint8 and frames.flags.c_contiguous
+        else:
+            assert str(frames.dtype) == "torch.uint8" and frames.is_contiguous()
+        assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= n and len(counts) >= n
+        t = self.L.yolo_b200_submit_yuv(self._h, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
+                                        dets.ctypes.data, counts.ctypes.data)
+        if t < 0:
+            self._check(t)
+        return t
+
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
@@ -363,6 +422,14 @@ class Context:
         """cv2.resize (bilinear) of packed device images of different sizes (shapes: host int32 [n][2]) into d_dst [n][dh][dw][3]."""
         shapes = np.ascontiguousarray(shapes, dtype=np.int32).reshape(-1, 2)
         self._check(self.L.yolo_b200_resize_u8bgr_ragged(self._h, _ptr(d_src), len(shapes), shapes.ctypes.data, _ptr(d_dst), dh, dw))
+
+    def forward_yuv_dev(self, d_in, fmt, n, sh, sw, h, w, d_dets, d_counts):
+        """n YUV frames of source size sh x sw packed in device memory (layout of forward_yuv)."""
+        self._check(self.L.yolo_b200_forward_yuv_dev(self._h, _ptr(d_in), fmt, n, sh, sw, h, w, _ptr(d_dets), _ptr(d_counts)))
+
+    def yuv_to_bgr_resize(self, d_src, fmt, n, sh, sw, d_dst, dh, dw):
+        """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device YUV frames into d_dst uint8 [n][dh][dw][3]."""
+        self._check(self.L.yolo_b200_yuv_to_bgr_resize(self._h, _ptr(d_src), fmt, n, sh, sw, _ptr(d_dst), dh, dw))
 
     def resize_u8bgr(self, d_src, n, sh, sw, d_dst, dh, dw):
         """cv2.resize (bilinear) of n uint8 [sh][sw][3] device images into d_dst [n][dh][dw][3]."""
