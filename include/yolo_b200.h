@@ -244,7 +244,6 @@ int yolo_b200_forward_f32_dev(yolo_b200_ctx *ctx, const float *d_nchw, int n, in
                               yolo_b200_det *d_dets, int32_t *d_counts);
 int yolo_b200_forward_u8bgr_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n, int h, int w,
                                 yolo_b200_det *d_dets, int32_t *d_counts);
-/* Block until everything queued on the context stream is done. */
 int yolo_b200_forward_u8bgr_resize_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr, int n, int sh, int sw, int h, int w,
                                        yolo_b200_det *d_dets, int32_t *d_counts);
 /* Images of different sizes packed back to back in device memory (layout and errors as yolo_b200_forward_u8bgr_ragged;
@@ -256,6 +255,7 @@ int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr,
 int yolo_b200_forward_yuv_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
                               yolo_b200_det *d_dets, int32_t *d_counts);
 
+/* Block until everything queued on the context stream is done. */
 int yolo_b200_sync(yolo_b200_ctx *ctx);
 
 /* ---- per-stage entry points (device buffers) -------------------------------------------- */

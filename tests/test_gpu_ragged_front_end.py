@@ -20,12 +20,16 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 E_ARG, E_STATE, E_UNSUPPORTED = -1, -2, -3
 
 
-def _resize_oracle():
+def _oracle(name):
     import importlib.util
-    spec = importlib.util.spec_from_file_location("oracle_resize_u8", os.path.join(ROOT, "oracle", "resize_u8.py"))
+    spec = importlib.util.spec_from_file_location("oracle_" + name, os.path.join(ROOT, "oracle", name + ".py"))
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
     return m
+
+
+def _resize_oracle():
+    return _oracle("resize_u8")
 
 
 def _images(rng, shapes):
@@ -132,7 +136,7 @@ def test_ragged_resize_matches_the_oracle_frame_by_frame(ctx):
         got = _gpu_resize_ragged(ctx, [im for _, im in group], dh, dw)
         for k, (seed, _) in enumerate(group):
             np.testing.assert_array_equal(got[k], g["out_%d" % seed], err_msg="golden seed %d -> %dx%d" % (seed, dh, dw))
-    # one source size: the ragged kernel equals the uniform one
+    # one source size: the ragged entry point equals the uniform one
     import torch
     same = _images(rng, [(48, 64)] * 5)
     got = _gpu_resize_ragged(ctx, same, 40, 44)
@@ -288,6 +292,51 @@ def test_ragged_calls_in_flight_keep_their_own_tables(ctx):
     for (_, _, d_dets, d_counts), wnt in zip(res, want + want[:1]):
         n = d_counts.numel()
         _same_dets((d_dets.cpu().numpy().view(lib.DET_DTYPE).reshape(n, 512), d_counts.cpu().numpy()), wnt, 512)
+
+
+@pytest.mark.gpu
+def test_stage_calls_of_changing_geometry_queued_back_to_back(ctx):
+    """Resize stages queued without a synchronise while the source geometry changes from call to call: the uniform tables
+    are rewritten in stream order behind the resizes that still read them, and each of the two staging buffers is refilled
+    while copies out of earlier ones are still queued.  Every output equals the oracle; every call is one launch."""
+    import torch
+    ro, yo = _resize_oracle(), _oracle("yuv_u8")
+    rng = np.random.default_rng(59)
+    dh, dw = 40, 44
+    calls = []                                                   # (issue the call, device output, expected output)
+
+    def uniform(sh, sw, n=3):
+        imgs = rng.integers(0, 256, (n, sh, sw, 3), dtype=np.uint8)
+        d, out = _dev(imgs), torch.zeros((n, dh, dw, 3), dtype=torch.uint8, device="cuda")
+        calls.append((lambda: ctx.resize_u8bgr(d, n, sh, sw, out, dh, dw), out, ro.resize_batch(imgs, dh, dw)))
+
+    def ragged(shapes):
+        imgs = _images(rng, shapes)
+        flat, hw = lib.pack_images(imgs)
+        d, out = _dev(flat), torch.zeros((len(imgs), dh, dw, 3), dtype=torch.uint8, device="cuda")
+        calls.append((lambda: ctx.resize_u8bgr_ragged(d, hw, out, dh, dw), out, np.stack([ro.resize_bilinear_u8(im, dh, dw) for im in imgs])))
+
+    def yuv(fmt, sh, sw, n=2):
+        frames = rng.integers(0, 256, (n,) + lib.yuv_frame_shape(fmt, sh, sw), dtype=np.uint8)
+        d, out = _dev(frames), torch.zeros((n, dh, dw, 3), dtype=torch.uint8, device="cuda")
+        calls.append((lambda: ctx.yuv_to_bgr_resize(d, fmt, n, sh, sw, out, dh, dw), out, ro.resize_batch(yo.to_bgr_batch(frames, fmt), dh, dw)))
+
+    uniform(48, 64); uniform(37, 53); uniform(90, 31)           # three geometry changes in a row
+    yuv(lib.YUV_NV12, 34, 66)
+    ragged([(60, 80), (17, 9), (48, 64), (1, 1)])
+    uniform(48, 64)
+    ragged([(60, 80)] * 4)                                       # one size: the uniform kernel with the cached tables
+    yuv(lib.YUV_YUYV, 7, 8)
+    ragged(MIX_SMALL)
+    uniform(200, 150); uniform(37, 53)
+    _torch_done()
+    before = ctx.launch_count()
+    for k, (issue, _, _) in enumerate(calls):
+        issue()
+        assert ctx.launch_count() == before + k + 1, "call %d: one launch" % k
+    ctx.sync()
+    for k, (_, out, want) in enumerate(calls):
+        np.testing.assert_array_equal(out.cpu().numpy(), want, err_msg="call %d" % k)
 
 
 @pytest.mark.gpu

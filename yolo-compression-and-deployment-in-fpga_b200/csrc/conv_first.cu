@@ -285,9 +285,9 @@ bool conv3x3_first_supported(const ConvArgs &a)
 }
 
 // alignment the quad loads need from the source pointer (frames are W*H pixels with W % 4 == 0, so every quad inherits it)
-bool conv3x3_first_src_ok(int src_kind, const void *src)
+bool conv3x3_first_src_ok(InKind src_kind, const void *src)
 {
-    return ((uintptr_t)src % (src_kind == 1 ? 8 : src_kind == 2 ? 4 : 16)) == 0;
+    return ((uintptr_t)src % (src_kind == IN_RGB444 ? 8 : src_kind == IN_BGR ? 4 : 16)) == 0;
 }
 
 template <bool POOL, int EPI, int SRC, bool WIDE = false>
@@ -316,14 +316,14 @@ static cudaError_t launch_first2(const FirstParams &p, cudaStream_t st)
         // wider first layers (darknet19's 3 -> 32): one pass per 16 output channels over the same input
         FirstParams q = p;
         for (q.co0 = 0; q.co0 < p.cs_out; q.co0 += 16) {
-            cudaError_t e = p.in16 ? launch_first3<POOL, EPI, 1, true>(q, st) : p.in8 ? launch_first3<POOL, EPI, 2, true>(q, st) : launch_first3<POOL, EPI, 0, true>(q, st);
+            cudaError_t e = p.in16 ? launch_first3<POOL, EPI, IN_RGB444, true>(q, st) : p.in8 ? launch_first3<POOL, EPI, IN_BGR, true>(q, st) : launch_first3<POOL, EPI, IN_INT8, true>(q, st);
             if (e != cudaSuccess) return e;
         }
         return cudaSuccess;
     }
-    if (p.in16) return launch_first3<POOL, EPI, 1>(p, st);
-    if (p.in8) return launch_first3<POOL, EPI, 2>(p, st);
-    return launch_first3<POOL, EPI, 0>(p, st);
+    if (p.in16) return launch_first3<POOL, EPI, IN_RGB444>(p, st);
+    if (p.in8) return launch_first3<POOL, EPI, IN_BGR>(p, st);
+    return launch_first3<POOL, EPI, IN_INT8>(p, st);
 }
 
 template <bool POOL>
@@ -337,21 +337,21 @@ static cudaError_t launch_first(const ConvArgs &a, FirstParams &p, cudaStream_t 
     }
 }
 
-// src_kind 1 / 2: fused RGB444 / uint8-BGR front end (a.in is ignored); lut = the context's table for that source
-cudaError_t conv3x3_first(const ConvArgs &a, cudaStream_t st, int src_kind, const void *src, const void *lut)
+// src_kind IN_RGB444 / IN_BGR: fused RGB444 / uint8-BGR front end (a.in is ignored); lut = the context's table for that source
+cudaError_t conv3x3_first(const ConvArgs &a, cudaStream_t st, InKind src_kind, const void *src, const void *lut)
 {
     if (a.n == 0) return cudaSuccess;
     if (!conv3x3_first_supported(a)) return cudaErrorInvalidValue;
     // the benchmark geometries (pooled, 16 channels, pooled width >= 128) run on the tcgen05 kernel of conv_fs.cu
-    if (conv3x3_fs_supported(a, src_kind, src_kind ? src : (const void *)a.in))
-        return conv3x3_fs(a, st, src_kind, src_kind ? src : (const void *)a.in, lut);
+    if (conv3x3_fs_supported(a, src_kind, src_kind != IN_INT8 ? src : (const void *)a.in))
+        return conv3x3_fs(a, st, src_kind, src_kind != IN_INT8 ? src : (const void *)a.in, lut);
     FirstParams p;
     memset(&p, 0, sizeof p);
     p.in = a.in; p.n_img = a.n; p.H = a.H; p.W = a.W;
-    if (src_kind == 1) { p.in16 = (const uint16_t *)src; p.lut = (const int *)lut; }
-    else if (src_kind == 2) { p.in8 = (const uint8_t *)src; p.lut8 = (const uint8_t *)lut; }
+    if (src_kind == IN_RGB444) { p.in16 = (const uint16_t *)src; p.lut = (const int *)lut; }
+    else if (src_kind == IN_BGR) { p.in8 = (const uint8_t *)src; p.lut8 = (const uint8_t *)lut; }
     // a pixel quad = 8 bytes of RGB444, 12 of BGR bytes (three word loads), 16 of NHWC4
-    if (!conv3x3_first_src_ok(src_kind, src_kind ? src : (const void *)a.in)) return cudaErrorInvalidValue;
+    if (!conv3x3_first_src_ok(src_kind, src_kind != IN_INT8 ? src : (const void *)a.in)) return cudaErrorInvalidValue;
     p.OH = a.q.pool ? a.H / 2 : a.H; p.OW = a.q.pool ? a.W / 2 : a.W;
     p.out_img_bytes = (size_t)p.OH * p.OW * a.cs_out;
     p.cs_out = a.cs_out; p.wgt = a.wgt; p.bias_sh = a.bias_sh; p.q = a.q; p.out = a.out; p.ovf = a.ovf;

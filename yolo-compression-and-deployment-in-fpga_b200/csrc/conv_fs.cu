@@ -469,11 +469,11 @@ static unsigned fs_magic(int d) { return (unsigned)(((1ull << 32) + (unsigned)d 
 constexpr uint32_t FS_SMEM_MAX = 227u * 1024u;
 
 // fills the geometry part of p; false = this kernel does not take the layer
-static bool fs_plan(const ConvArgs &a, int src_kind, const void *src, FsParams &p)
+static bool fs_plan(const ConvArgs &a, InKind src_kind, const void *src, FsParams &p)
 {
     memset(&p, 0, sizeof p);
-    if (!fs_enabled() || src_kind < 0 || src_kind > 2) return false;
-    if (src_kind == 2 && (a.W % 16)) return false;                 // rows of 3 W bytes are bulk-copied: multiples of 16 bytes
+    if (!fs_enabled() || src_kind == IN_F32) return false;
+    if (src_kind == IN_BGR && (a.W % 16)) return false;                 // rows of 3 W bytes are bulk-copied: multiples of 16 bytes
     if (a.cs_in != 4 || (a.cs_out != 16 && a.cs_out != 32) || a.w_rows < a.cs_out || !a.q.pool) return false;
     if (a.H < 2 || a.W < 256 || (a.W % 8)) return false;       // pooled width >= 128: a tile spans at most two pooled rows
     if (((uintptr_t)src & 15) || ((uintptr_t)a.out & 15)) return false;
@@ -488,9 +488,9 @@ static bool fs_plan(const ConvArgs &a, int src_kind, const void *src, FsParams &
     p.ow_magic = fs_magic(p.OW); p.upi_magic = fs_magic(p.upi);
     p.MR = (127 + p.OW - 1) / p.OW;                            // = 1
     p.segs = (p.OW + FS_SEGW - 1) / FS_SEGW;
-    p.row_bytes = (uint32_t)a.W * (src_kind == 1 ? 2u : src_kind == 2 ? 3u : 4u);
+    p.row_bytes = (uint32_t)a.W * (src_kind == IN_RGB444 ? 2u : src_kind == IN_BGR ? 3u : 4u);
     p.off_lut = 2u * 4u * (uint32_t)a.cs_out * 32u;             // the two weight images
-    p.off_raw = p.off_lut + (src_kind == 1 ? 4112u * 4u : src_kind == 2 ? 768u : 0u);       // 4097 table words / three byte tables
+    p.off_raw = p.off_lut + (src_kind == IN_RGB444 ? 4112u * 4u : src_kind == IN_BGR ? 768u : 0u);       // 4097 table words / three byte tables
     p.off_bias = p.off_raw + (uint32_t)FS_RAWR * 2u * p.row_bytes;
     p.off_bar = (p.off_bias + 128u + 15u) & ~15u;
     p.off_arr = (p.off_bar + 8u * (2 * FS_RAWR + 2 * FS_RMAX + 2 * FS_TBUF_MAX + 1) + 127u) & ~127u;
@@ -506,7 +506,7 @@ static bool fs_plan(const ConvArgs &a, int src_kind, const void *src, FsParams &
     return true;
 }
 
-bool conv3x3_fs_supported(const ConvArgs &a, int src_kind, const void *src)
+bool conv3x3_fs_supported(const ConvArgs &a, InKind src_kind, const void *src)
 {
     FsParams p;
     return fs_plan(a, src_kind, src, p);
@@ -576,18 +576,18 @@ static cudaError_t launch_fs2(const FsParams &p, cudaStream_t st, int sm_count)
 }
 
 template <int EPI>
-static cudaError_t launch_fs(const FsParams &p, int src_kind, cudaStream_t st, int sm_count)
+static cudaError_t launch_fs(const FsParams &p, InKind src_kind, cudaStream_t st, int sm_count)
 {
-    if (p.co == 32) return src_kind == 1 ? launch_fs2<EPI, 1, 32>(p, st, sm_count) : src_kind == 2 ? launch_fs2<EPI, 2, 32>(p, st, sm_count) : launch_fs2<EPI, 0, 32>(p, st, sm_count);
-    return src_kind == 1 ? launch_fs2<EPI, 1, 16>(p, st, sm_count) : src_kind == 2 ? launch_fs2<EPI, 2, 16>(p, st, sm_count) : launch_fs2<EPI, 0, 16>(p, st, sm_count);
+    if (p.co == 32) return src_kind == IN_RGB444 ? launch_fs2<EPI, IN_RGB444, 32>(p, st, sm_count) : src_kind == IN_BGR ? launch_fs2<EPI, IN_BGR, 32>(p, st, sm_count) : launch_fs2<EPI, IN_INT8, 32>(p, st, sm_count);
+    return src_kind == IN_RGB444 ? launch_fs2<EPI, IN_RGB444, 16>(p, st, sm_count) : src_kind == IN_BGR ? launch_fs2<EPI, IN_BGR, 16>(p, st, sm_count) : launch_fs2<EPI, IN_INT8, 16>(p, st, sm_count);
 }
 
-cudaError_t conv3x3_fs(const ConvArgs &a, cudaStream_t st, int src_kind, const void *src, const void *lut)
+cudaError_t conv3x3_fs(const ConvArgs &a, cudaStream_t st, InKind src_kind, const void *src, const void *lut)
 {
     if (a.n == 0) return cudaSuccess;
     FsParams p;
     if (!fs_plan(a, src_kind, src, p)) return cudaErrorInvalidValue;
-    if (src_kind >= 1 && !lut) return cudaErrorInvalidValue;
+    if (src_kind != IN_INT8 && !lut) return cudaErrorInvalidValue;
     p.src = src; p.lut = (const int *)lut;
     p.wgt = a.wgt; p.bias_sh = a.bias_sh; p.q = a.q; p.out = a.out; p.ovf = a.ovf;
     p.xsplit = a.out_xsplit ? 1 : 0;

@@ -38,15 +38,19 @@ struct ConvArgs {
 // conv_direct.cu
 cudaError_t conv3x3_direct(const ConvArgs &a, cudaStream_t st);
 
+// The input kinds of the network: int8 NHWC4, RGB444 uint16 frames (+ 4096-word table), uint8 BGR images (+ 3x256-byte
+// table), float NCHW.  The first three are also the first-layer kernels' source template argument; f32 is quantised first.
+enum InKind { IN_INT8 = 0, IN_RGB444 = 1, IN_BGR = 2, IN_F32 = 3 };
+
 // conv_first.cu (first layer: NHWC4 input, <= 16 output channels, warp-level integer MMAs)
 bool conv3x3_first_supported(const ConvArgs &a);
-bool conv3x3_first_src_ok(int src_kind, const void *src);      // pointer alignment the first-layer kernel needs (0 int8 NHWC4, 1 RGB444, 2 BGR bytes)
-// src_kind: 0 = a.in (int8 NHWC4), 1 = RGB444 uint16 frames + 4096-word table, 2 = uint8 BGR images + 3x256-byte table
-cudaError_t conv3x3_first(const ConvArgs &a, cudaStream_t st, int src_kind = 0, const void *src = nullptr, const void *lut = nullptr);
+bool conv3x3_first_src_ok(InKind src_kind, const void *src);    // pointer alignment the first-layer kernel needs
+// src_kind IN_INT8 reads a.in; IN_RGB444 / IN_BGR read src with the context's table lut for that source
+cudaError_t conv3x3_first(const ConvArgs &a, cudaStream_t st, InKind src_kind = IN_INT8, const void *src = nullptr, const void *lut = nullptr);
 
-// conv_fs.cu (first layer on tcgen05: 3 -> 16 channels + pool for pooled widths >= 128; src_kind 0 = int8 NHWC4, 1 = RGB444 + table)
-bool conv3x3_fs_supported(const ConvArgs &a, int src_kind, const void *src);
-cudaError_t conv3x3_fs(const ConvArgs &a, cudaStream_t st, int src_kind, const void *src, const void *lut);
+// conv_fs.cu (first layer on tcgen05: 3 -> 16 channels + pool for pooled widths >= 128; src_kind IN_INT8, IN_RGB444 or IN_BGR)
+bool conv3x3_fs_supported(const ConvArgs &a, InKind src_kind, const void *src);
+cudaError_t conv3x3_fs(const ConvArgs &a, cudaStream_t st, InKind src_kind, const void *src, const void *lut);
 
 // conv_umma.cu (tcgen05 / TMEM / TMA implicit GEMM)
 bool conv3x3_umma_supported(const ConvArgs &a);
@@ -88,21 +92,19 @@ cudaError_t quantize_f32(const float *nchw, int n, int h, int w, int sa, int8_t 
 // resize.cu (uint8 HxWx3 bilinear resize = cv2.resize of the reference's BaseTransform, data/__init__.py:36)
 void resize_axis_table(int src, int dst, bool clamp_weights, int index_scale, int4 *out);   // host: (tap0, tap1, weight0, weight1) per output index
 // xtab: per column (byte offset of tap 0 in its row, weight0 | weight1 << 16), tap 1 = the next pixel; ytab: per row (row 0, row 1, weight0 << 16, weight1 << 16)
-cudaError_t resize_u8bgr(const uint8_t *src, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
-                         const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
-// taps and weights of one geometry (sh, sw) -> (dh, dw) in the layout above: ytab [dh], xtab [dw] (host)
+// taps and weights of one geometry (sh, sw) -> (dh, dw) in that layout: ytab [dh], xtab [dw] (host)
 void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab);
-// Images of different sizes packed back to back in one buffer of src_bytes bytes: frame f starts at byte off of src, its
-// rows are pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
-struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
-cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames_dev, int n, uint8_t *dst, int dh, int dw,
-                                const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
-// YUV frames (format = YOLO_B200_YUV_*: NV12, I420, YUYV in cv2's Mat layout, packed at yuv_frame_bytes) -> BGR as
-// cv2.cvtColor does, resized as resize_u8bgr does, in one pass with the same tables: uint8 [n][dh][dw][3]
+// Source formats: the YUV layouts (NV12, I420, YUYV in cv2's Mat layout, frames packed at yuv_frame_bytes) and uint8 BGR
 enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YUV_YUYV = YOLO_B200_YUV_YUYV, RS_BGR = 3 };
 size_t yuv_frame_bytes(int format, int sh, int sw);        // 0 for an unknown format
-cudaError_t resize_yuv_u8bgr(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
-                             const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
+// Images of different sizes packed back to back in one buffer: frame f starts at byte off of src, its rows are
+// pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
+struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
+// One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for YUV).
+// frames_dev == nullptr: the frames are sh x sw at a uniform stride from src, with the tables ytab [dh], xtab [dw].
+// Otherwise (RS_BGR only) frames_dev[f] describes frame f as above.  A BGR launch reads no byte at or past src + src_bytes.
+cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
+                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
 
 // head.cu
 struct HeadArgs {

@@ -307,32 +307,23 @@ static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const Res
     return cudaGetLastError();
 }
 
-cudaError_t resize_u8bgr(const uint8_t *src, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
-                         const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
-{
-    return resize_launch<false>(src, (size_t)n * sh * sw * 3, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
-}
-
-cudaError_t resize_u8bgr_ragged(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames_dev, int n, uint8_t *dst, int dh, int dw,
-                                const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
-{
-    return resize_launch<true>(src, src_bytes, frames_dev, n, 0, 0, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
-}
-
 size_t yuv_frame_bytes(int format, int sh, int sw)
 {
     const size_t px = (size_t)sh * sw;
     return format == RS_YUV_NV12 || format == RS_YUV_I420 ? px + px / 2 : format == RS_YUV_YUYV ? 2 * px : 0;
 }
 
-cudaError_t resize_yuv_u8bgr(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
-                             const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
+                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
 {
-    switch (format) {
-    case RS_YUV_NV12: return resize_launch<false, RS_YUV_NV12>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
-    case RS_YUV_I420: return resize_launch<false, RS_YUV_I420>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
-    case RS_YUV_YUYV: return resize_launch<false, RS_YUV_YUYV>(src, 0, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
-    default: return cudaErrorInvalidValue;
+    if (frames_dev)
+        return fmt == RS_BGR ? resize_launch<true>(src, src_bytes, frames_dev, n, 0, 0, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st) : cudaErrorInvalidValue;
+    switch (fmt) {
+    case RS_BGR:      return resize_launch<false>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_YUV_NV12: return resize_launch<false, RS_YUV_NV12>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_YUV_I420: return resize_launch<false, RS_YUV_I420>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_YUV_YUYV: return resize_launch<false, RS_YUV_YUYV>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    default:          return cudaErrorInvalidValue;
     }
 }
 

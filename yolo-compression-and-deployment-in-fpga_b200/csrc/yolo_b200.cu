@@ -72,6 +72,17 @@ struct HostTrace {
     }
 };
 
+// Device tables of the resize front end (resize_tables): a table image uploaded in stream order through two alternating
+// pinned staging buffers, so an upload waits for no queued resize and overwrites nothing a queued resize still reads.
+struct ResizeTables {
+    void *dev = nullptr; size_t dev_cap = 0;
+    char *host[2] = {nullptr, nullptr}; size_t host_cap[2] = {0, 0};
+    cudaEvent_t ev[2] = {nullptr, nullptr};                 // recorded after the copy out of host[k]
+    int next = 0;
+    int key[4] = {0, 0, 0, 0};                              // the context's uniform cache: (sh, sw, dh, dw) of its tables
+    const ResizeFrame *frames = nullptr; const int4 *ytab = nullptr; const int2 *xtab = nullptr;     // inside dev
+};
+
 // One host-buffer call in flight: its device staging, batch-wide prediction map, detection lists, the pinned landing
 // area of the counts and its events.  Two slots let the tail of call i (last chunk's layers, decode + NMS, copy of the
 // detections) overlap the host-to-device copy of call i + 1 (yolo_b200_submit_* / yolo_b200_wait).
@@ -79,8 +90,7 @@ constexpr int YB_HOST_SLOTS = 2;
 struct HostSlot {
     void *stage_in = nullptr; size_t stage_in_cap = 0;      // device staging of the host frames (network-size frames)
     void *rs_src = nullptr; size_t rs_src_cap = 0;          // resize front end: staged source images
-    void *rg_tab = nullptr; size_t rg_tab_cap = 0;          // images of different sizes: descriptors + tables of the call (device)
-    char *rg_host = nullptr; size_t rg_host_cap = 0;        // ... and their pinned staging copy
+    ResizeTables tabs;                                      // images of different sizes: descriptors + tables of the call (s_in)
     int8_t *pred_all = nullptr; size_t pred_all_cap = 0;    // batch-wide prediction map
     yolo_b200_det *d_dets = nullptr; size_t dets_cap = 0;
     int32_t *d_counts = nullptr; size_t counts_cap = 0;
@@ -111,15 +121,8 @@ struct yolo_b200_ctx {
     int *stats_dev = nullptr;            // calibration: {max, min} of a layer's numerator / abs-max bits of the input
     int8_t *in_q = nullptr; size_t in_q_cap = 0;        // quantised NHWC4 input
     uint8_t *rs_out = nullptr; size_t rs_out_cap = 0;   // resize front end: resized images (device entry point)
-    void *rs_tab = nullptr; size_t rs_tab_cap = 0;      // [dh] int4 row taps/weights, then [dw] int2 column offsets/weights
-    const int4 *rs_ytab = nullptr; const int2 *rs_xtab = nullptr;
-    int rs_key[4] = {0, 0, 0, 0};                       // (sh, sw, dh, dw) the tables were built for
-    // images of different sizes, device entry points: descriptors + tables of the most recent call, rewritten in stream
-    // order on the context stream; two pinned staging buffers alternate (one is refilled once the copy out of it has run)
-    void *rg_tab = nullptr; size_t rg_tab_cap = 0;
-    char *rg_host[2] = {nullptr, nullptr}; size_t rg_host_cap[2] = {0, 0};
-    cudaEvent_t rg_ev[2] = {nullptr, nullptr};
-    int rg_next = 0;
+    ResizeTables rs_cache;                              // one source size: the tables of the most recent geometry
+    ResizeTables rs_call;                               // images of different sizes, device entry points: the most recent call's
     float *h_scores = nullptr; int *h_cls = nullptr; float4 *h_boxes = nullptr; size_t head_cap = 0;
     int last_n = 0;
     int64_t launches = 0;
@@ -197,6 +200,15 @@ int yolo_b200_create(yolo_b200_ctx **out, int device)
     return 0;
 }
 
+static void free_tables(ResizeTables &t)
+{
+    cudaFree(t.dev);
+    for (int k = 0; k < 2; ++k) {
+        if (t.host[k]) cudaFreeHost(t.host[k]);
+        if (t.ev[k]) cudaEventDestroy(t.ev[k]);
+    }
+}
+
 static void free_layers(yolo_b200_ctx *c)
 {
     for (auto &l : c->layers) { l.view = nullptr; cudaFree(l.w); cudaFree(l.w_k160); cudaFree(l.wimg); cudaFree(l.wimg_tap); cudaFree(l.wimg_tap2); cudaFree(l.wimg_tap3); cudaFree(l.wimg_rp); cudaFree(l.wimg_rps); cudaFree(l.w_swz); cudaFree(l.bias_sh); cudaFree(l.out); cudaFree(l.w1); cudaFree(l.raw); cudaFree(l.cat); }
@@ -214,17 +226,13 @@ void yolo_b200_destroy(yolo_b200_ctx *c)
     cudaStreamSynchronize(c->stream);
     free_layers(c);
     cudaFree(c->lut_dev); cudaFree(c->lut8_dev); cudaFree(c->ovf_dev); cudaFree(c->stats_dev); cudaFree(c->in_q);
-    cudaFree(c->rs_out); cudaFree(c->rs_tab); cudaFree(c->rg_tab);
-    for (int k = 0; k < 2; ++k) {
-        if (c->rg_host[k]) cudaFreeHost(c->rg_host[k]);
-        if (c->rg_ev[k]) cudaEventDestroy(c->rg_ev[k]);
-    }
+    cudaFree(c->rs_out); free_tables(c->rs_cache); free_tables(c->rs_call);
     cudaFree(c->h_scores); cudaFree(c->h_cls); cudaFree(c->h_boxes);
     for (auto e : c->ev) cudaEventDestroy(e);
     for (auto &S : c->slots) {
-        cudaFree(S.stage_in); cudaFree(S.rs_src); cudaFree(S.rg_tab); cudaFree(S.pred_all); cudaFree(S.d_dets); cudaFree(S.d_counts);
+        cudaFree(S.stage_in); cudaFree(S.rs_src); cudaFree(S.pred_all); cudaFree(S.d_dets); cudaFree(S.d_counts);
+        free_tables(S.tabs);
         if (S.counts_pinned) cudaFreeHost(S.counts_pinned);
-        if (S.rg_host) cudaFreeHost(S.rg_host);
         for (auto e : S.ev_in) cudaEventDestroy(e);
         for (auto e : S.ev_done) cudaEventDestroy(e);
         for (auto e : S.ev_cnt) cudaEventDestroy(e);
@@ -613,24 +621,6 @@ int yolo_b200_quantize_u8bgr(yolo_b200_ctx *c, const uint8_t *d_bgr, int n, int 
     return 0;
 }
 
-// taps and weights of the bilinear resize (sh, sw) -> (dh, dw), rebuilt when the geometry changes
-static int ensure_resize_tables(yolo_b200_ctx *c, int sh, int sw, int dh, int dw)
-{
-    if (c->rs_tab && c->rs_key[0] == sh && c->rs_key[1] == sw && c->rs_key[2] == dh && c->rs_key[3] == dw) return 0;
-    const size_t ybytes = (size_t)dh * sizeof(int4), xbytes = (size_t)dw * sizeof(int2);
-    int rc = ensure(&c->rs_tab, &c->rs_tab_cap, ybytes + xbytes); if (rc) return rc;
-    std::vector<int4> img((ybytes + xbytes + sizeof(int4) - 1) / sizeof(int4));
-    resize_geometry_tables(sh, sw, dh, dw, img.data(), reinterpret_cast<int2 *>(reinterpret_cast<char *>(img.data()) + ybytes));
-    c->rs_key[0] = 0;
-    // an earlier resize queued on the context stream may still read the tables: stream-ordered copy from pageable memory
-    CU(cudaMemcpyAsync(c->rs_tab, img.data(), ybytes + xbytes, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    c->rs_ytab = reinterpret_cast<const int4 *>(c->rs_tab);
-    c->rs_xtab = reinterpret_cast<const int2 *>(reinterpret_cast<const char *>(c->rs_tab) + ybytes);
-    c->rs_key[0] = sh; c->rs_key[1] = sw; c->rs_key[2] = dh; c->rs_key[3] = dw;
-    return 0;
-}
-
 int yolo_b200_resize_taps(int src, int dst, int horizontal, int32_t *taps)
 {
     if (src < 1 || dst < 1 || !taps) return fail(E_ARG, "bad resize axis %d -> %d", src, dst);
@@ -638,64 +628,6 @@ int yolo_b200_resize_taps(int src, int dst, int horizontal, int32_t *taps)
     resize_axis_table(src, dst, horizontal != 0, 1, t.data());
     for (int d = 0; d < dst; ++d) { taps[4 * d] = t[d].x; taps[4 * d + 1] = t[d].y; taps[4 * d + 2] = t[d].z; taps[4 * d + 3] = t[d].w; }
     return 0;
-}
-
-int yolo_b200_resize_u8bgr(yolo_b200_ctx *c, const uint8_t *d_src, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
-{
-    if (!c) return fail(E_ARG, "null ctx");
-    if (n < 0 || sh < 1 || sw < 1 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d %dx%d -> %dx%d", n, sh, sw, dh, dw);
-    if ((size_t)sh * sw * 3 > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "source image larger than 2 GiB");
-    CU(cudaSetDevice(c->device));
-    if (n == 0) return 0;
-    if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
-    int rc = ensure_resize_tables(c, sh, sw, dh, dw); if (rc) return rc;
-    CU(resize_u8bgr(d_src, n, sh, sw, d_dst, dh, dw, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream));
-    c->launches++;
-    return 0;
-}
-
-// A batch of images of different sizes, packed back to back without padding.  (sh, sw) of image i = src_hw[2 * i * stride]
-// and the entry after it: stride 1 reads one size per image, stride 0 gives every image the size src_hw[0..1] (a uniform batch).
-struct RaggedPlan {
-    std::vector<size_t> off;                        // [n + 1]: byte offset of image i in the packed buffer; off[n] = total
-    std::vector<ResizeFrame> frames;                // [n]: what the kernel reads per frame
-    std::vector<std::pair<int, int>> geoms;         // distinct source sizes in order of first appearance
-    std::vector<int4> img;                          // descriptors, then int4 [G][dh] row tables, then int2 [G][dw] column tables
-    size_t ytab_off = 0, xtab_off = 0, img_bytes = 0;
-};
-
-static int ragged_plan(int n, const int32_t *src_hw, int stride, RaggedPlan &p)
-{
-    p.off.assign((size_t)n + 1, 0);
-    p.frames.resize((size_t)n);
-    p.geoms.clear();
-    std::map<std::pair<int, int>, int> index;
-    for (int i = 0; i < n; ++i) {
-        const int sh = src_hw[2 * (size_t)i * stride], sw = src_hw[2 * (size_t)i * stride + 1];
-        if (sh < 1 || sw < 1) return fail(E_ARG, "image %d: bad source shape %dx%d", i, sh, sw);
-        const size_t bytes = (size_t)sh * sw * 3;
-        if (bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "image %d: source image larger than 2 GiB", i);
-        auto it = index.emplace(std::make_pair(sh, sw), (int)p.geoms.size()).first;
-        if (it->second == (int)p.geoms.size()) p.geoms.push_back(it->first);
-        p.frames[i].off = p.off[i]; p.frames[i].pitch = sw * 3; p.frames[i].geom = it->second;
-        p.off[i + 1] = p.off[i] + bytes;
-    }
-    return 0;
-}
-
-// the plan's table image: per distinct size exactly the tables ensure_resize_tables builds
-static void ragged_tables(RaggedPlan &p, int dh, int dw)
-{
-    const size_t G = p.geoms.size();
-    p.ytab_off = p.frames.size() * sizeof(ResizeFrame);
-    p.xtab_off = p.ytab_off + G * dh * sizeof(int4);
-    p.img_bytes = p.xtab_off + G * dw * sizeof(int2);
-    p.img.resize((p.img_bytes + sizeof(int4) - 1) / sizeof(int4));
-    char *b = reinterpret_cast<char *>(p.img.data());
-    memcpy(b, p.frames.data(), p.ytab_off);
-    for (size_t g = 0; g < G; ++g)
-        resize_geometry_tables(p.geoms[g].first, p.geoms[g].second, dh, dw, reinterpret_cast<int4 *>(b + p.ytab_off) + g * dh,
-                               reinterpret_cast<int2 *>(b + p.xtab_off) + g * dw);
 }
 
 static int ensure_pinned(char **p, size_t *cap, size_t need)
@@ -707,40 +639,6 @@ static int ensure_pinned(char **p, size_t *cap, size_t need)
     if (e != cudaSuccess) return fail(E_NOMEM, "cudaHostAlloc(%zu): %s", need, cudaGetErrorString(e));
     *cap = need;
     return 0;
-}
-
-// Ragged resize of the device entry points on the context stream: the plan's tables go to the context-owned buffer in
-// stream order (after every resize queued earlier on the stream has read the previous ones), then one launch.
-static int resize_ragged_dev(yolo_b200_ctx *c, const uint8_t *d_src, int n, RaggedPlan &p, uint8_t *d_dst, int dh, int dw)
-{
-    ragged_tables(p, dh, dw);
-    const int k = c->rg_next;
-    if (!c->rg_ev[k]) CU(cudaEventCreateWithFlags(&c->rg_ev[k], cudaEventDisableTiming));
-    CU(cudaEventSynchronize(c->rg_ev[k]));                    // the copy out of this staging buffer two calls ago has run
-    int rc = ensure_pinned(&c->rg_host[k], &c->rg_host_cap[k], p.img_bytes); if (rc) return rc;
-    rc = ensure(&c->rg_tab, &c->rg_tab_cap, p.img_bytes); if (rc) return rc;      // (a cudaFree waits for queued work)
-    memcpy(c->rg_host[k], p.img.data(), p.img_bytes);
-    CU(cudaMemcpyAsync(c->rg_tab, c->rg_host[k], p.img_bytes, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaEventRecord(c->rg_ev[k], c->stream));
-    c->rg_next ^= 1;
-    const char *t = (const char *)c->rg_tab;
-    CU(resize_u8bgr_ragged(d_src, p.off[n], (const ResizeFrame *)t, n, d_dst, dh, dw, (const int2 *)(t + p.xtab_off),
-                           (const int4 *)(t + p.ytab_off), c->sm_count, c->stream));
-    c->launches++;
-    return 0;
-}
-
-int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *d_src, int n, const int32_t *src_hw, uint8_t *d_dst, int dh, int dw)
-{
-    if (!c) return fail(E_ARG, "null ctx");
-    if (n < 0 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d -> %dx%d", n, dh, dw);
-    CU(cudaSetDevice(c->device));
-    if (n == 0) return 0;
-    if (!src_hw) return fail(E_ARG, "null src_hw");
-    RaggedPlan p;
-    int rc = ragged_plan(n, src_hw, 1, p); if (rc) return rc;
-    if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
-    return resize_ragged_dev(c, d_src, n, p, d_dst, dh, dw);
 }
 
 // One YUV frame of (format, sh, sw): its byte count, or E_ARG / E_UNSUPPORTED (include/yolo_b200.h)
@@ -763,20 +661,158 @@ int yolo_b200_yuv_frame_bytes(int format, int sh, int sw)
     return (int)b;
 }
 
-// YUV -> BGR + resize on the context stream with the context's cached tables (ensure_resize_tables uploads in stream order)
-int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int format, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+// A YUV entry point's format as a source format: RS_BGR is not a YUV format a caller may name, so it goes on as an
+// unknown one, which yuv_check refuses
+static int yuv_format(int format) { return format == RS_BGR ? -1 : format; }
+
+// Where the n frames of one call are and how they become dh x dw frames of the network input (plan_sources, net_plan).
+enum { RESIZE_NONE, RESIZE_UNIFORM, RESIZE_RAGGED };
+struct SourcePlan {
+    InKind kind = IN_BGR;                            // what the frames are once resized
+    int fmt = RS_BGR, n = 0, dh = 0, dw = 0, mode = RESIZE_NONE;
+    size_t frame_bytes = 0;                          // one source size: bytes per frame
+    std::vector<size_t> off;                         // RESIZE_RAGGED: [n + 1] byte offset of frame f; off[n] = total
+    std::vector<ResizeFrame> frames;                 // RESIZE_RAGGED: what the kernel reads per frame
+    std::vector<std::pair<int, int>> geoms;          // distinct source sizes in order of first appearance
+    size_t at(int f) const { return off.empty() ? (size_t)f * frame_bytes : off[f]; }     // byte offset of frame f
+};
+
+// The plan of n frames of format fmt (RS_BGR or a YUV layout) for the network size dh x dw.  Frame i has the source size
+// src_hw[2 * i * stride] x src_hw[2 * i * stride + 1] (stride 0: one size for all, checked also when n == 0).  One rule
+// picks the resize: none for a forward call whose only source size is dh x dw in BGR (the frames are the network input
+// as they are), uniform for one source size or any YUV call, ragged for several source sizes.
+static int plan_sources(int fmt, int n, const int32_t *src_hw, int stride, int dh, int dw, bool forward, SourcePlan &p)
+{
+    p = SourcePlan();
+    p.fmt = fmt; p.n = n; p.dh = dh; p.dw = dw;
+    const int m = stride ? n : 1;                                // sizes to read
+    if (m > 0 && !src_hw) return fail(E_ARG, "null src_hw");
+    if (fmt != RS_BGR) {
+        int rc = yuv_check(fmt, src_hw[0], src_hw[1], &p.frame_bytes); if (rc) return rc;
+        p.geoms.push_back({src_hw[0], src_hw[1]});
+        p.mode = RESIZE_UNIFORM;
+        return 0;
+    }
+    p.off.assign((size_t)(m > 0 ? m : 0) + 1, 0);
+    std::map<std::pair<int, int>, int> index;
+    for (int i = 0; i < m; ++i) {
+        const int sh = src_hw[2 * (size_t)i], sw = src_hw[2 * (size_t)i + 1];
+        if (sh < 1 || sw < 1) return fail(E_ARG, "image %d: bad source shape %dx%d", i, sh, sw);
+        const size_t bytes = (size_t)sh * sw * 3;
+        if (bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "image %d: source image larger than 2 GiB", i);
+        auto it = index.emplace(std::make_pair(sh, sw), (int)p.geoms.size()).first;
+        if (it->second == (int)p.geoms.size()) p.geoms.push_back(it->first);
+        p.frames.push_back({p.off[i], sw * 3, it->second});
+        p.off[i + 1] = p.off[i] + bytes;
+    }
+    if (p.geoms.size() > 1) { p.mode = RESIZE_RAGGED; return 0; }
+    p.off.clear(); p.frames.clear();
+    if (p.geoms.empty()) return 0;                               // no frames
+    p.frame_bytes = (size_t)p.geoms[0].first * p.geoms[0].second * 3;
+    p.mode = forward && p.geoms[0] == std::make_pair(dh, dw) ? RESIZE_NONE : RESIZE_UNIFORM;
+    return 0;
+}
+
+// n frames of kind k at the network size h x w: no resize, frame f at f * h * w * (bytes per pixel)
+static SourcePlan net_plan(InKind k, int n, int h, int w)
+{
+    static const size_t px_bytes[4] = { 4, 2, 3, 12 };           // IN_INT8, IN_RGB444, IN_BGR, IN_F32
+    SourcePlan p;
+    p.kind = k; p.n = n; p.dh = h; p.dw = w; p.frame_bytes = (size_t)h * w * px_bytes[k];
+    return p;
+}
+
+// Copies the table image img to t.dev in stream order on st: after everything queued there before it, and out of a staging
+// buffer that is refilled only once the copy out of it two uploads ago has run.
+static int upload_tables(ResizeTables &t, const void *img, size_t bytes, cudaStream_t st)
+{
+    const int k = t.next;
+    if (!t.ev[k]) CU(cudaEventCreateWithFlags(&t.ev[k], cudaEventDisableTiming));
+    CU(cudaEventSynchronize(t.ev[k]));
+    int rc = ensure_pinned(&t.host[k], &t.host_cap[k], bytes); if (rc) return rc;
+    rc = ensure(&t.dev, &t.dev_cap, bytes); if (rc) return rc;      // (a cudaFree waits for queued work)
+    memcpy(t.host[k], img, bytes);
+    CU(cudaMemcpyAsync(t.dev, t.host[k], bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(t.ev[k], st));
+    t.next ^= 1;
+    return 0;
+}
+
+// The tables the resize of plan p reads (*out; nothing for mode none).  One source size: the context's cache, uploaded on
+// the context stream when the geometry changes.  Several: the descriptors, then per distinct size exactly the uniform
+// tables, uploaded into `call` on stream st.
+static int resize_tables(yolo_b200_ctx *c, const SourcePlan &p, ResizeTables &call, cudaStream_t st, const ResizeTables **out)
+{
+    if (p.mode == RESIZE_NONE) return 0;
+    const bool ragged = p.mode == RESIZE_RAGGED;
+    ResizeTables &t = ragged ? call : c->rs_cache;
+    *out = &t;
+    const int key[4] = { p.geoms[0].first, p.geoms[0].second, p.dh, p.dw };
+    if (!ragged && !memcmp(t.key, key, sizeof key)) return 0;
+    const size_t G = p.geoms.size(), ytab_off = p.frames.size() * sizeof(ResizeFrame), xtab_off = ytab_off + G * p.dh * sizeof(int4);
+    const size_t bytes = xtab_off + G * p.dw * sizeof(int2);
+    std::vector<int4> img((bytes + sizeof(int4) - 1) / sizeof(int4));
+    char *b = reinterpret_cast<char *>(img.data());
+    memcpy(b, p.frames.data(), ytab_off);
+    for (size_t g = 0; g < G; ++g)
+        resize_geometry_tables(p.geoms[g].first, p.geoms[g].second, p.dh, p.dw, reinterpret_cast<int4 *>(b + ytab_off) + g * p.dh,
+                               reinterpret_cast<int2 *>(b + xtab_off) + g * p.dw);
+    t.key[0] = 0;
+    int rc = upload_tables(t, img.data(), bytes, ragged ? st : c->stream); if (rc) return rc;
+    if (!ragged) memcpy(t.key, key, sizeof key);
+    const char *d = (const char *)t.dev;
+    t.frames = (const ResizeFrame *)d; t.ytab = (const int4 *)(d + ytab_off); t.xtab = (const int2 *)(d + xtab_off);
+    return 0;
+}
+
+// One resize launch on the context stream: frames [f0, f0 + nf) of plan p (src = where frame 0 starts) into dst.  A ragged
+// launch may read up to the end of frame f0 + nf - 1 (in the host path the end of the chunk's landed bytes, never into a
+// later chunk); a uniform one reads only its own frames.
+static cudaError_t enqueue_resize(yolo_b200_ctx *c, const SourcePlan &p, const ResizeTables &t, const uint8_t *src, int f0, int nf, uint8_t *dst)
+{
+    const bool ragged = p.mode == RESIZE_RAGGED;
+    const size_t first = ragged ? 0 : p.at(f0);
+    cudaError_t e = resize_u8c3(src + first, p.at(f0 + nf) - first, p.fmt, ragged ? t.frames + f0 : nullptr, nf, p.geoms[0].first,
+                                p.geoms[0].second, dst, p.dh, p.dw, t.xtab, t.ytab, c->sm_count, c->stream);
+    if (e == cudaSuccess) c->launches++;
+    return e;
+}
+
+// The resize of the device entry points: tables, then one launch, both on the context stream
+static int resize_dev(yolo_b200_ctx *c, const SourcePlan &p, const uint8_t *d_src, uint8_t *d_dst)
+{
+    const ResizeTables *t = nullptr;
+    int rc = resize_tables(c, p, c->rs_call, c->stream, &t); if (rc) return rc;
+    CU(enqueue_resize(c, p, *t, d_src, 0, p.n, d_dst));
+    return 0;
+}
+
+// The resize stages: n frames (sizes as plan_sources reads them) -> uint8 BGR [n][dh][dw][3], one launch when n >= 1
+static int resize_stage(yolo_b200_ctx *c, int fmt, const uint8_t *d_src, int n, const int32_t *src_hw, int stride, uint8_t *d_dst, int dh, int dw)
 {
     if (!c) return fail(E_ARG, "null ctx");
     if (n < 0 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d -> %dx%d", n, dh, dw);
-    size_t fb;
-    int rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
+    SourcePlan p;
+    int rc = plan_sources(fmt, n, src_hw, stride, dh, dw, false, p); if (rc) return rc;
     CU(cudaSetDevice(c->device));
     if (n == 0) return 0;
     if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
-    rc = ensure_resize_tables(c, sh, sw, dh, dw); if (rc) return rc;
-    CU(resize_yuv_u8bgr(d_src, format, n, sh, sw, d_dst, dh, dw, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream));
-    c->launches++;
-    return 0;
+    return resize_dev(c, p, d_src, d_dst);
+}
+
+int yolo_b200_resize_u8bgr(yolo_b200_ctx *c, const uint8_t *d_src, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+{
+    const int32_t hw[2] = { sh, sw };
+    return resize_stage(c, RS_BGR, d_src, n, hw, 0, d_dst, dh, dw);
+}
+
+int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *d_src, int n, const int32_t *src_hw, uint8_t *d_dst, int dh, int dw)
+{ return resize_stage(c, RS_BGR, d_src, n, src_hw, 1, d_dst, dh, dw); }
+
+int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int format, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+{
+    const int32_t hw[2] = { sh, sw };
+    return resize_stage(c, yuv_format(format), d_src, n, hw, 0, d_dst, dh, dw);
 }
 
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
@@ -874,11 +910,11 @@ static int run_layer(yolo_b200_ctx *c, int l, const int8_t *d_in, int n, int h, 
     const bool ws_ok = aligned && conv3x3_ws_supported(a);
     if ((be == 2 || be == 3) && !umma_ok) return fail(E_UNSUPPORTED, "layer %d has no tensor-core shape (cs_in %d, cs_out %d)", l, L.cs_in, L.cs_out);
     if ((be == 4 || be == 5) && !ws_ok) return fail(E_UNSUPPORTED, "layer %d does not fit the weight-stationary kernel (cs_in %d, cs_out %d)", l, L.cs_in, L.cs_out);
-    const bool first_ok = ((uintptr_t)d_out & 3) == 0 && conv3x3_first_src_ok(0, d_in) && conv3x3_first_supported(a);
+    const bool first_ok = ((uintptr_t)d_out & 3) == 0 && conv3x3_first_src_ok(IN_INT8, d_in) && conv3x3_first_supported(a);
     const bool use_umma = be == 2 || be == 3 || (be == 0 && !first_ok && !ws_ok && umma_ok);
     if (use_umma) { int rc = ensure_swz(c, L); if (rc) return rc; a.wgt_swz = L.w_swz; }
     if (be == 1) CU(conv3x3_direct(a, c->stream));
-    else if (be == 0 && first_ok) { CU(conv3x3_first(a, c->stream)); c->launches += conv3x3_fs_supported(a, 0, a.in) ? 0 : L.cs_out / 16 - 1; }   // conv_first.cu: one pass per 16 output channels
+    else if (be == 0 && first_ok) { CU(conv3x3_first(a, c->stream)); c->launches += conv3x3_fs_supported(a, IN_INT8, a.in) ? 0 : L.cs_out / 16 - 1; }   // conv_first.cu: one pass per 16 output channels
     else if (use_umma) CU(conv3x3_umma(a, c->stream, c->sm_count));
     else if (be == 0 && conv3x3_rp_supported(a)) CU(conv3x3_rp(a, c->stream, c->sm_count));
     else if (be == 0 && aligned && conv3x3_ws2_supported(a, c->sm_count)) CU(conv3x3_ws2(a, c->stream, c->sm_count));
@@ -972,7 +1008,7 @@ static int backbone_from(yolo_b200_ctx *c, size_t first, const int8_t *net_in, i
         const bool in_split = l > 0 && !c->graph && c->layers[l - 1].xsplit;
         ConvArgs a0chk;
         fill_args(c, (int)l, cur, n, ih, iw, dst, a0chk);
-        L.xsplit = l == 0 && dst == L.out && ((uintptr_t)dst & 3) == 0 && conv3x3_first_src_ok(0, cur) && conv3x3_first_supported(a0chk) &&
+        L.xsplit = l == 0 && dst == L.out && ((uintptr_t)dst & 3) == 0 && conv3x3_first_src_ok(IN_INT8, cur) && conv3x3_first_supported(a0chk) &&
                    want_xsplit(c, l, cur, n, oh, ow);
         if (L.q.pool && L.unfused_pool) {
             rc = ensure((void **)&L.raw, &L.raw_cap, (size_t)(n > 0 ? n : 1) * ih * iw * L.cs_out); if (rc) return rc;
@@ -1233,8 +1269,8 @@ int yolo_b200_forward_int8_dev(yolo_b200_ctx *c, const int8_t *d_nhwc4, int n, i
 }
 
 // Camera / image front ends fused into the first layer (auto back end): the quantised frame never exists in HBM.
-// kind 1 = RGB444 (camera_to_inpBuf + pixel_norm_quantize, yolo_forward.c:57-123), 2 = uint8 BGR (BaseTransform + tracker).
-static int fused_front_features(yolo_b200_ctx *c, int kind, const void *d_src, int n, int h, int w, int8_t *last_out,
+// IN_RGB444 (camera_to_inpBuf + pixel_norm_quantize, yolo_forward.c:57-123), IN_BGR (BaseTransform + tracker).
+static int fused_front_features(yolo_b200_ctx *c, InKind kind, const void *d_src, int n, int h, int w, int8_t *last_out,
                                 const int8_t **pred, int *gh, int *gw, bool *done)
 {
     *done = false;
@@ -1242,8 +1278,8 @@ static int fused_front_features(yolo_b200_ctx *c, int kind, const void *d_src, i
     ConvArgs a0;
     fill_args(c, 0, nullptr, n, h, w, nullptr, a0);
     if (!(n > 0 && c->conv_backend == 0 && c->layers.size() > 1 && conv3x3_first_supported(a0) && conv3x3_first_src_ok(kind, d_src) && !(L0.q.pool && (h < 2 || w < 2)))) return 0;
-    if (kind == 1 && (((uintptr_t)d_src) & 1)) return 0;
-    if (kind == 2 && c->lut8_saturates) return 0;              // saturated inputs must be counted: the stand-alone quantiser does
+    if (kind == IN_RGB444 && (((uintptr_t)d_src) & 1)) return 0;
+    if (kind == IN_BGR && c->lut8_saturates) return 0;              // saturated inputs must be counted: the stand-alone quantiser does
     const int oh = L0.q.pool ? h / 2 : h, ow = L0.q.pool ? w / 2 : w;
     int rc = ensure((void **)&L0.out, &L0.out_cap, (size_t)n * oh * ow * L0.cs_out); if (rc) return rc;
     L0.oh = oh; L0.ow = ow; L0.rh = h; L0.rw = w; L0.view = L0.out;
@@ -1252,7 +1288,7 @@ static int fused_front_features(yolo_b200_ctx *c, int kind, const void *d_src, i
     a0.out_xsplit = L0.xsplit;
     c->ev_used = 0;
     tick(c);
-    CU(conv3x3_first(a0, c->stream, kind, d_src, kind == 1 ? (const void *)c->lut_dev : (const void *)c->lut8_dev));
+    CU(conv3x3_first(a0, c->stream, kind, d_src, kind == IN_RGB444 ? (const void *)c->lut_dev : (const void *)c->lut8_dev));
     c->launches += conv3x3_fs_supported(a0, kind, d_src) ? 1 : L0.cs_out / 16;
     tick(c);
     rc = backbone_from(c, 1, L0.out, n, oh, ow, pred, gh, gw, last_out); if (rc) return rc;
@@ -1260,22 +1296,22 @@ static int fused_front_features(yolo_b200_ctx *c, int kind, const void *d_src, i
     return 0;
 }
 
-// Front end + all convolution layers for one of the four input kinds (0 RGB444, 1 int8 NHWC4, 2 float NCHW, 3 uint8 BGR).
-static int features_dev(yolo_b200_ctx *c, int kind, const void *d_src, int n, int h, int w, int8_t *last_out,
+// Front end + all convolution layers for one of the four input kinds.
+static int features_dev(yolo_b200_ctx *c, InKind kind, const void *d_src, int n, int h, int w, int8_t *last_out,
                         const int8_t **pred, int *gh, int *gw)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     if (!d_src && n > 0) return fail(E_ARG, "null input");
-    if (kind == 0 || kind == 3) {
+    if (kind == IN_RGB444 || kind == IN_BGR) {
         bool done;
-        rc = fused_front_features(c, kind == 0 ? 1 : 2, d_src, n, h, w, last_out, pred, gh, gw, &done);
+        rc = fused_front_features(c, kind, d_src, n, h, w, last_out, pred, gh, gw, &done);
         if (rc || done) return rc;
     }
     const int8_t *x8 = (const int8_t *)d_src;
-    if (kind != 1) {
+    if (kind != IN_INT8) {
         rc = ensure((void **)&c->in_q, &c->in_q_cap, (size_t)(n > 0 ? n : 1) * h * w * 4); if (rc) return rc;
-        if (kind == 0) rc = yolo_b200_quantize_rgb444(c, (const uint16_t *)d_src, n, h, w, c->in_q);
-        else if (kind == 3) rc = yolo_b200_quantize_u8bgr(c, (const uint8_t *)d_src, n, h, w, c->in_q);
+        if (kind == IN_RGB444) rc = yolo_b200_quantize_rgb444(c, (const uint16_t *)d_src, n, h, w, c->in_q);
+        else if (kind == IN_BGR) rc = yolo_b200_quantize_u8bgr(c, (const uint8_t *)d_src, n, h, w, c->in_q);
         else rc = yolo_b200_quantize_f32(c, (const float *)d_src, n, h, w, c->in_q);
         if (rc) return rc;
         x8 = c->in_q;
@@ -1285,58 +1321,56 @@ static int features_dev(yolo_b200_ctx *c, int kind, const void *d_src, int n, in
     return backbone_from(c, 0, x8, n, h, w, pred, gh, gw, last_out);
 }
 
-static int forward_dev(yolo_b200_ctx *c, int kind, const void *d_src, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
+static int forward_dev(yolo_b200_ctx *c, InKind kind, const void *d_src, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 {
     const int8_t *pred; int gh, gw;
     int rc = features_dev(c, kind, d_src, n, h, w, nullptr, &pred, &gh, &gw); if (rc) return rc;
     return yolo_b200_detect(c, pred, n, gh, gw, h, w, d_dets, d_counts);
 }
 
+// The device forward of the resize front ends: plan, resize into the context's buffer, forward_dev
+static int forward_resize_dev(yolo_b200_ctx *c, int fmt, const uint8_t *d_src, int n, const int32_t *src_hw, int stride, int h, int w,
+                              yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    int rc = check_ready(c, n, h, w); if (rc) return rc;
+    SourcePlan p;
+    rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p); if (rc) return rc;
+    if (n == 0) return 0;
+    if (!d_src || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
+    if (p.mode != RESIZE_NONE) {
+        rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)n * h * w * 3); if (rc) return rc;
+        rc = resize_dev(c, p, d_src, c->rs_out); if (rc) return rc;
+        d_src = c->rs_out;
+    }
+    return forward_dev(c, IN_BGR, d_src, n, h, w, d_dets, d_counts);
+}
+
 int yolo_b200_forward_rgb444_dev(yolo_b200_ctx *c, const uint16_t *d_frames, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
-{ return forward_dev(c, 0, d_frames, n, h, w, d_dets, d_counts); }
+{ return forward_dev(c, IN_RGB444, d_frames, n, h, w, d_dets, d_counts); }
 
 int yolo_b200_forward_u8bgr_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
-{ return forward_dev(c, 3, d_bgr, n, h, w, d_dets, d_counts); }
+{ return forward_dev(c, IN_BGR, d_bgr, n, h, w, d_dets, d_counts); }
 
 int yolo_b200_forward_u8bgr_resize_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, int n, int sh, int sw, int h, int w,
                                        yolo_b200_det *d_dets, int32_t *d_counts)
 {
-    int rc = check_ready(c, n, h, w); if (rc) return rc;
-    if (sh == h && sw == w) return forward_dev(c, 3, d_bgr, n, h, w, d_dets, d_counts);     // identity resize copies the bytes
-    rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)(n > 0 ? n : 1) * h * w * 3); if (rc) return rc;
-    rc = yolo_b200_resize_u8bgr(c, d_bgr, n, sh, sw, c->rs_out, h, w); if (rc) return rc;
-    return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
+    const int32_t hw[2] = { sh, sw };
+    return forward_resize_dev(c, RS_BGR, d_bgr, n, hw, 0, h, w, d_dets, d_counts);
 }
 
 int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *c, const uint8_t *d_bgr, int n, const int32_t *src_hw, int h, int w,
                                        yolo_b200_det *d_dets, int32_t *d_counts)
-{
-    int rc = check_ready(c, n, h, w); if (rc) return rc;
-    if (n == 0) return 0;
-    if (!src_hw) return fail(E_ARG, "null src_hw");
-    RaggedPlan p;
-    rc = ragged_plan(n, src_hw, 1, p); if (rc) return rc;
-    if (!d_bgr || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
-    rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)n * h * w * 3); if (rc) return rc;
-    rc = resize_ragged_dev(c, d_bgr, n, p, c->rs_out, h, w); if (rc) return rc;
-    return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
-}
+{ return forward_resize_dev(c, RS_BGR, d_bgr, n, src_hw, 1, h, w, d_dets, d_counts); }
 
 int yolo_b200_forward_yuv_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
                               yolo_b200_det *d_dets, int32_t *d_counts)
 {
-    int rc = check_ready(c, n, h, w); if (rc) return rc;
-    size_t fb;
-    rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
-    if (n == 0) return 0;
-    if (!d_frames || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
-    rc = ensure((void **)&c->rs_out, &c->rs_out_cap, (size_t)n * h * w * 3); if (rc) return rc;
-    rc = yolo_b200_yuv_to_bgr_resize(c, d_frames, format, n, sh, sw, c->rs_out, h, w); if (rc) return rc;
-    return forward_dev(c, 3, c->rs_out, n, h, w, d_dets, d_counts);
+    const int32_t hw[2] = { sh, sw };
+    return forward_resize_dev(c, yuv_format(format), d_frames, n, hw, 0, h, w, d_dets, d_counts);
 }
 
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
-{ return forward_dev(c, 2, d_nchw, n, h, w, d_dets, d_counts); }
+{ return forward_dev(c, IN_F32, d_nchw, n, h, w, d_dets, d_counts); }
 
 int yolo_b200_sync(yolo_b200_ctx *c)
 {
@@ -1351,44 +1385,21 @@ int yolo_b200_sync(yolo_b200_ctx *c)
 // chunking changes no result); every chunk's prediction map lands in one batch-wide buffer and decode + NMS then run once
 // over the whole batch (a per-chunk NMS launch cannot fill the GPU: it is one CTA per frame).  Only the filled part of the
 // detection lists is copied back.
-// src_hw != nullptr (kind 3 only): the host images have the source sizes src_hw (ragged_plan: stride 0 = one size for all),
-// are packed back to back and are resized to h x w on the GPU chunk by chunk, between the copy and the first layer; chunk
-// k's copy is the byte range [off[f0], off[f0 + nk]) of the packed images.  One source size takes the uniform kernel and the
-// context's cached tables (no resize at all when it is h x w); several take the ragged kernel with the descriptors and
-// tables of this call in the slot's own buffers, uploaded on the copy stream (the slot's previous call has completed, so
-// nothing queued still reads them).
-// yuv >= 0 (kind 3 only, with src_hw = the one source size, stride 0): the host frames are YUV of that format, packed at
-// in_bytes / n bytes; each chunk's landed frames take one fused YUV -> BGR + resize launch with the context's cached
-// tables (also when the size is h x w: the conversion is needed anyway).
+// The plan p says where the host frames are and how they are resized to the network size on the GPU, chunk by chunk,
+// between the copy and the first layer: chunk k's copy is the byte range [at(f0), at(f0 + nk)) of the host buffer, and
+// enqueue_resize makes its landed frames network input.  A ragged plan's descriptors and tables go into the slot's own
+// buffers, uploaded on the copy stream (the slot's previous call has completed, so nothing queued still reads them).
 // host_enqueue queues the whole call (copies in, layers, decode + NMS, copy of the counts) on the context's streams and
 // returns; host_complete waits for the counts, copies the filled part of the lists back and waits for that copy.
-static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
+static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, const SourcePlan &p, yolo_b200_det *dets, int32_t *counts)
 {
     HostSlot &S = c->slots[si];
     S.ngroups = 0; S.dets = dets; S.counts = counts;
-    RaggedPlan rp;
-    int rc;
-    const bool packed = src_hw && yuv < 0;                       // BGR images at ragged_plan's offsets
-    if (packed) { rc = ragged_plan(n, src_hw, hw_stride, rp); if (rc) return rc; }
-    const bool resize = yuv >= 0 || (packed && !(rp.geoms.size() == 1 && rp.geoms[0] == std::make_pair(h, w)));
-    const bool ragged = packed && resize && rp.geoms.size() > 1;
-    const int sh = yuv >= 0 ? src_hw[0] : packed ? rp.geoms[0].first : 0, sw = yuv >= 0 ? src_hw[1] : packed ? rp.geoms[0].second : 0;
-    const size_t frame_bytes = packed ? 0 : in_bytes / (size_t)n;
-    auto src_off = [&](int f) { return packed ? rp.off[f] : (size_t)f * frame_bytes; };      // byte offset of frame f in host_in
-    const size_t net_frame_bytes = src_hw ? (size_t)h * w * 3 : frame_bytes;
-    rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
-    if (resize) {
-        rc = ensure(&S.rs_src, &S.rs_src_cap, src_off(n)); if (rc) return rc;
-        if (ragged) {
-            ragged_tables(rp, h, w);
-            rc = ensure(&S.rg_tab, &S.rg_tab_cap, rp.img_bytes); if (rc) return rc;
-            rc = ensure_pinned(&S.rg_host, &S.rg_host_cap, rp.img_bytes); if (rc) return rc;
-            memcpy(S.rg_host, rp.img.data(), rp.img_bytes);
-        } else {
-            rc = ensure_resize_tables(c, sh, sw, h, w); if (rc) return rc;
-        }
-    }
+    const int n = p.n, h = p.dh, w = p.dw;
+    const bool resize = p.mode != RESIZE_NONE;
+    const size_t net_frame_bytes = resize ? (size_t)h * w * 3 : p.frame_bytes;
+    int rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
+    if (resize) { rc = ensure(&S.rs_src, &S.rs_src_cap, p.at(n)); if (rc) return rc; }
     const size_t md = (size_t)c->prm.max_det;
     rc = ensure((void **)&S.d_dets, &S.dets_cap, (size_t)n * md * sizeof(yolo_b200_det)); if (rc) return rc;
     rc = ensure((void **)&S.d_counts, &S.counts_cap, (size_t)n * sizeof(int32_t)); if (rc) return rc;
@@ -1444,8 +1455,8 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
     tr.ev.clear();
     tr.on = getenv("YOLO_B200_TRACE_HOST") != nullptr;
     if (tr.on) { cudaEventCreate(&tr.t0); cudaEventRecord(tr.t0, c->s_in); }
-    if (ragged) CU(cudaMemcpyAsync(S.rg_tab, S.rg_host, rp.img_bytes, cudaMemcpyHostToDevice, c->s_in));
-    const char *rg = (const char *)S.rg_tab;
+    const ResizeTables *tabs = nullptr;
+    rc = resize_tables(c, p, S.tabs, c->s_in, &tabs); if (rc) return rc;
     // The slot's buffers are its own: nothing queued earlier reads or writes them once the slot's previous call has been
     // completed, so the copies of this call do NOT wait for the context stream (the layers of the previous call may still
     // be running there: that overlap is the point of the second slot).
@@ -1458,23 +1469,17 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, size_t in
     for (int k = 0; k < nchunks; ++k) {
         const int f0 = cf0[k], nk = cnk[k];
         char *stage = (char *)S.stage_in + (size_t)f0 * net_frame_bytes;
-        char *land = resize ? (char *)S.rs_src + src_off(f0) : stage;
-        CU(cudaMemcpyAsync(land, (const char *)host_in + src_off(f0), src_off(f0 + nk) - src_off(f0), cudaMemcpyHostToDevice, c->s_in));
+        char *land = resize ? (char *)S.rs_src + p.at(f0) : stage;
+        CU(cudaMemcpyAsync(land, (const char *)host_in + p.at(f0), p.at(f0 + nk) - p.at(f0), cudaMemcpyHostToDevice, c->s_in));
         CU(cudaEventRecord(S.ev_in[k], c->s_in));
         tr.mark("h2d done", k, c->s_in);
         CU(cudaStreamWaitEvent(c->stream, S.ev_in[k], 0));
         if (resize) {
-            // the ragged kernel reads the call's buffer up to the end of this chunk's landed bytes, never into a later chunk;
-            // the uniform and YUV kernels read only the nk frames at `land`
-            cudaError_t e = ragged ? resize_u8bgr_ragged((const uint8_t *)S.rs_src, rp.off[f0 + nk], (const ResizeFrame *)rg + f0, nk, (uint8_t *)stage, h, w,
-                                                         (const int2 *)(rg + rp.xtab_off), (const int4 *)(rg + rp.ytab_off), c->sm_count, c->stream)
-                          : yuv >= 0 ? resize_yuv_u8bgr((const uint8_t *)land, yuv, nk, sh, sw, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream)
-                                   : resize_u8bgr((const uint8_t *)land, nk, sh, sw, (uint8_t *)stage, h, w, c->rs_xtab, c->rs_ytab, c->sm_count, c->stream);
+            cudaError_t e = enqueue_resize(c, p, *tabs, (const uint8_t *)S.rs_src, f0, nk, (uint8_t *)stage);
             if (e != cudaSuccess) { drain(); return fail(E_CUDA, "resize: %s", cudaGetErrorString(e)); }
-            c->launches++;
         }
         const int8_t *pred; int g1, g2;
-        rc = features_dev(c, kind, stage, nk, h, w, S.pred_all + (size_t)f0 * pred_frame, &pred, &g1, &g2);
+        rc = features_dev(c, p.kind, stage, nk, h, w, S.pred_all + (size_t)f0 * pred_frame, &pred, &g1, &g2);
         if (rc) { drain(); return rc; }
         tr.mark("layers done", k, c->stream);
         if (k == nchunks - 2 || k == nchunks - 1) {
@@ -1528,43 +1533,37 @@ static int host_free_slot(yolo_b200_ctx *c)
     return -1;
 }
 
-// blocking call = submit + wait on any free slot
-static int forward_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                        yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
+// The host-buffer calls, frames at host_in as plan p says.  Blocking (submit == false): submit + wait on any free slot,
+// n == 0 is a no-op.  Asynchronous (submit == true, n >= 1): returns a ticket (>= 0) once the call is queued; the caller's
+// buffers belong to the library until yolo_b200_wait(ticket) returns.
+static int host_call(yolo_b200_ctx *c, bool submit, const void *host_in, const SourcePlan &p, yolo_b200_det *dets, int32_t *counts)
 {
-    int rc = check_ready(c, n, h, w); if (rc) return rc;
-    if (n == 0) return 0;
+    int rc = check_ready(c, p.n, p.dh, p.dw); if (rc) return rc;
+    if (submit && p.n < 1) return fail(E_ARG, "submit needs n >= 1");
+    if (p.n == 0) return 0;
     if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
     const int si = host_free_slot(c);
     if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride, yuv); if (rc) return rc;
-    return host_complete(c, si);
+    rc = host_enqueue(c, si, host_in, p, dets, counts); if (rc) return rc;
+    return submit ? si : host_complete(c, si);
 }
 
-// asynchronous pair: returns a ticket (>= 0) once the call is queued; the caller's buffers belong to the library until
-// yolo_b200_wait(ticket) returns
-static int submit_host(yolo_b200_ctx *c, const void *host_in, size_t in_bytes, int kind, int n, int h, int w,
-                       yolo_b200_det *dets, int32_t *counts, const int32_t *src_hw = nullptr, int hw_stride = 1, int yuv = -1)
+// host calls of the resize front ends (sizes as plan_sources reads them)
+static int host_resize(yolo_b200_ctx *c, bool submit, int fmt, const void *host_in, int n, const int32_t *src_hw, int stride, int h, int w,
+                       yolo_b200_det *dets, int32_t *counts)
 {
-    int rc = check_ready(c, n, h, w); if (rc) return rc;
-    if (n < 1) return fail(E_ARG, "submit needs n >= 1");
-    if (!host_in || !dets || !counts) return fail(E_ARG, "null buffer");
-    const int si = host_free_slot(c);
-    if (si < 0) return fail(E_STATE, "%d submissions in flight: call yolo_b200_wait first", YB_HOST_SLOTS);
-    rc = host_enqueue(c, si, host_in, in_bytes, kind, n, h, w, dets, counts, src_hw, hw_stride, yuv); if (rc) return rc;
-    return si;
+    SourcePlan p;
+    int rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p); if (rc) return rc;
+    return host_call(c, submit, host_in, p, dets, counts);
 }
 
 int yolo_b200_submit_rgb444(yolo_b200_ctx *c, const uint16_t *frames, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return submit_host(c, frames, (size_t)n * h * w * 2, 0, n, h, w, dets, counts); }
+{ return host_call(c, true, frames, net_plan(IN_RGB444, n, h, w), dets, counts); }
 int yolo_b200_submit_u8bgr(yolo_b200_ctx *c, const uint8_t *bgr, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return submit_host(c, bgr, (size_t)n * h * w * 3, 3, n, h, w, dets, counts); }
+{ return host_call(c, true, bgr, net_plan(IN_BGR, n, h, w), dets, counts); }
 int yolo_b200_submit_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
                                   yolo_b200_det *dets, int32_t *counts)
-{
-    if (!src_hw && n > 0) return fail(E_ARG, "null src_hw");
-    return submit_host(c, bgr, 0, 3, n, h, w, dets, counts, src_hw);
-}
+{ return host_resize(c, true, RS_BGR, bgr, n, src_hw, 1, h, w, dets, counts); }
 int yolo_b200_wait(yolo_b200_ctx *c, int ticket)
 {
     if (!c) return fail(E_ARG, "null ctx");
@@ -1574,42 +1573,33 @@ int yolo_b200_wait(yolo_b200_ctx *c, int ticket)
 }
 
 int yolo_b200_forward_rgb444(yolo_b200_ctx *c, const uint16_t *frames, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return forward_host(c, frames, (size_t)n * h * w * 2, 0, n, h, w, dets, counts); }
+{ return host_call(c, false, frames, net_plan(IN_RGB444, n, h, w), dets, counts); }
 int yolo_b200_forward_int8(yolo_b200_ctx *c, const int8_t *nhwc4, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return forward_host(c, nhwc4, (size_t)n * h * w * 4, 1, n, h, w, dets, counts); }
+{ return host_call(c, false, nhwc4, net_plan(IN_INT8, n, h, w), dets, counts); }
 int yolo_b200_forward_u8bgr(yolo_b200_ctx *c, const uint8_t *bgr, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return forward_host(c, bgr, (size_t)n * h * w * 3, 3, n, h, w, dets, counts); }
+{ return host_call(c, false, bgr, net_plan(IN_BGR, n, h, w), dets, counts); }
 int yolo_b200_forward_f32(yolo_b200_ctx *c, const float *nchw, int n, int h, int w, yolo_b200_det *dets, int32_t *counts)
-{ return forward_host(c, nchw, (size_t)n * h * w * 12, 2, n, h, w, dets, counts); }
+{ return host_call(c, false, nchw, net_plan(IN_F32, n, h, w), dets, counts); }
 int yolo_b200_forward_u8bgr_resize(yolo_b200_ctx *c, const uint8_t *bgr, int n, int sh, int sw, int h, int w, yolo_b200_det *dets, int32_t *counts)
 {
-    if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
     const int32_t hw[2] = { sh, sw };
-    return forward_host(c, bgr, (size_t)n * sh * sw * 3, 3, n, h, w, dets, counts, hw, 0);
+    return host_resize(c, false, RS_BGR, bgr, n, hw, 0, h, w, dets, counts);
 }
 int yolo_b200_forward_u8bgr_ragged(yolo_b200_ctx *c, const uint8_t *bgr, int n, const int32_t *src_hw, int h, int w,
                                    yolo_b200_det *dets, int32_t *counts)
-{
-    if (!src_hw && n > 0) return fail(E_ARG, "null src_hw");
-    return forward_host(c, bgr, 0, 3, n, h, w, dets, counts, src_hw);
-}
-// YUV host frames: the uniform resize pipeline with the fused conversion (host_enqueue, yuv >= 0)
-static int yuv_host(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
-                    yolo_b200_det *dets, int32_t *counts, bool submit)
-{
-    size_t fb;
-    int rc = yuv_check(format, sh, sw, &fb); if (rc) return rc;
-    const int32_t hw[2] = { sh, sw };
-    const size_t bytes = n > 0 ? (size_t)n * fb : 0;
-    return submit ? submit_host(c, frames, bytes, 3, n, h, w, dets, counts, hw, 0, format)
-                  : forward_host(c, frames, bytes, 3, n, h, w, dets, counts, hw, 0, format);
-}
+{ return host_resize(c, false, RS_BGR, bgr, n, src_hw, 1, h, w, dets, counts); }
 int yolo_b200_forward_yuv(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
                           yolo_b200_det *dets, int32_t *counts)
-{ return yuv_host(c, frames, format, n, sh, sw, h, w, dets, counts, false); }
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, false, yuv_format(format), frames, n, hw, 0, h, w, dets, counts);
+}
 int yolo_b200_submit_yuv(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
                          yolo_b200_det *dets, int32_t *counts)
-{ return yuv_host(c, frames, format, n, sh, sw, h, w, dets, counts, true); }
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, true, yuv_format(format), frames, n, hw, 0, h, w, dets, counts);
+}
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------
 int yolo_b200_pack_detections(yolo_b200_ctx *c, const yolo_b200_det *d_dets, const int32_t *d_counts, int n,

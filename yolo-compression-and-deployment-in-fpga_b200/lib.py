@@ -284,27 +284,31 @@ class Context:
         self._check(self.L.yolo_b200_set_default_context(self._h))
 
     # -- host-buffer forward (copies inside the call)
-    def _forward_host(self, fn, x: np.ndarray, n, h, w):
-        md = self.params.max_det
-        dets = np.zeros((n, md), dtype=DET_DTYPE)
+    def _forward_host(self, fn, n, *args):
+        """A blocking host-buffer call fn(ctx, *args, dets, counts) over n frames -> (dets [n][max_det], counts [n])."""
+        dets = np.zeros((n, self.params.max_det), dtype=DET_DTYPE)
         counts = np.zeros(n, dtype=np.int32)
-        self._check(fn(self._h, x.ctypes.data, n, h, w, dets.ctypes.data, counts.ctypes.data))
+        self._check(fn(self._h, *args, dets.ctypes.data, counts.ctypes.data))
         return dets, counts
+
+    def _submit(self, fn, *args) -> int:
+        """An asynchronous host-buffer call fn(ctx, *args) -> its ticket."""
+        t = fn(self._h, *args)
+        if t < 0:
+            self._check(t)
+        return t
 
     def forward_rgb444(self, frames: np.ndarray):
         f = np.ascontiguousarray(frames, dtype=np.uint16)
         n, h, w = f.shape
-        return self._forward_host(self.L.yolo_b200_forward_rgb444, f, n, h, w)
+        return self._forward_host(self.L.yolo_b200_forward_rgb444, n, f.ctypes.data, n, h, w)
 
     def submit_rgb444(self, frames: np.ndarray, dets: np.ndarray, counts: np.ndarray) -> int:
         """Queue one batch (uint16 [n][h][w], C-contiguous; dets [n][max_det] DET_DTYPE, counts int32 [n]: the arrays must
         stay alive and untouched until wait(ticket)).  Returns the ticket."""
         assert frames.dtype == np.uint16 and frames.flags.c_contiguous and dets.flags.c_contiguous and counts.flags.c_contiguous
         n, h, w = frames.shape
-        t = self.L.yolo_b200_submit_rgb444(self._h, frames.ctypes.data, n, h, w, dets.ctypes.data, counts.ctypes.data)
-        if t < 0:
-            self._check(t)
-        return t
+        return self._submit(self.L.yolo_b200_submit_rgb444, frames.ctypes.data, n, h, w, dets.ctypes.data, counts.ctypes.data)
 
     def wait(self, ticket: int):
         self._check(self.L.yolo_b200_wait(self._h, ticket))
@@ -315,7 +319,7 @@ class Context:
         f = np.ascontiguousarray(images, dtype=np.uint8)
         n, h, w, c = f.shape
         assert c == 3
-        return self._forward_host(self.L.yolo_b200_forward_u8bgr, f, n, h, w)
+        return self._forward_host(self.L.yolo_b200_forward_u8bgr, n, f.ctypes.data, n, h, w)
 
     def forward_u8bgr_resize(self, images: np.ndarray, size):
         """uint8 BGR images [n][sh][sw][3] of any one size: the reference's whole BaseTransform (cv2.resize bilinear to
@@ -323,35 +327,23 @@ class Context:
         f = np.ascontiguousarray(images, dtype=np.uint8)
         n, sh, sw, c = f.shape
         assert c == 3
-        h, w = int(size[0]), int(size[1])
-        md = self.params.max_det
-        dets = np.zeros((n, md), dtype=DET_DTYPE)
-        counts = np.zeros(n, dtype=np.int32)
-        self._check(self.L.yolo_b200_forward_u8bgr_resize(self._h, f.ctypes.data, n, sh, sw, h, w, dets.ctypes.data, counts.ctypes.data))
-        return dets, counts
+        return self._forward_host(self.L.yolo_b200_forward_u8bgr_resize, n, f.ctypes.data, n, sh, sw, int(size[0]), int(size[1]))
 
     def forward_u8bgr_images(self, images, size):
         """A list of uint8 BGR images of any sizes (cv2.imread arrays) -> (dets [n][max_det], counts [n]) in one call: the
         whole BaseTransform (resize to size = (h, w) included) + forward pass on the GPU.  Boxes are normalised: image i
         scales them by its own [w, h, w, h]."""
         flat, shapes = pack_images(images)
-        n, md = len(shapes), self.params.max_det
-        dets = np.zeros((n, md), dtype=DET_DTYPE)
-        counts = np.zeros(n, dtype=np.int32)
-        self._check(self.L.yolo_b200_forward_u8bgr_ragged(self._h, flat.ctypes.data, n, shapes.ctypes.data, int(size[0]), int(size[1]),
-                                                          dets.ctypes.data, counts.ctypes.data))
-        return dets, counts
+        n = len(shapes)
+        return self._forward_host(self.L.yolo_b200_forward_u8bgr_ragged, n, flat.ctypes.data, n, shapes.ctypes.data, int(size[0]), int(size[1]))
 
     def submit_u8bgr_images(self, packed, shapes: np.ndarray, size, dets: np.ndarray, counts: np.ndarray) -> int:
         """Queue one batch of packed images (pack_images; `packed` a numpy array or a pinned torch tensor) for size = (h, w);
         packed, dets [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until wait(ticket)."""
         shapes = np.ascontiguousarray(shapes, dtype=np.int32)
         assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= len(shapes) and len(counts) >= len(shapes)
-        t = self.L.yolo_b200_submit_u8bgr_ragged(self._h, _ptr(packed), len(shapes), shapes.ctypes.data, int(size[0]), int(size[1]),
-                                                 dets.ctypes.data, counts.ctypes.data)
-        if t < 0:
-            self._check(t)
-        return t
+        return self._submit(self.L.yolo_b200_submit_u8bgr_ragged, _ptr(packed), len(shapes), shapes.ctypes.data, int(size[0]), int(size[1]),
+                            dets.ctypes.data, counts.ctypes.data)
 
     def forward_yuv(self, frames: np.ndarray, fmt: int, size):
         """uint8 YUV frames [n, *yuv_frame_shape(fmt, sh, sw)] (cv2 Mat layout: decoder NV12 / I420, webcam YUYV) ->
@@ -359,12 +351,8 @@ class Context:
         forward_u8bgr_resize, all on the GPU; the frames cross the link as they are (1.5 or 2 bytes per pixel)."""
         f = np.ascontiguousarray(frames, dtype=np.uint8)
         sh, sw = yuv_source_size(fmt, f.shape[1:])
-        n, md = f.shape[0], self.params.max_det
-        dets = np.zeros((n, md), dtype=DET_DTYPE)
-        counts = np.zeros(n, dtype=np.int32)
-        self._check(self.L.yolo_b200_forward_yuv(self._h, f.ctypes.data, fmt, n, sh, sw, int(size[0]), int(size[1]),
-                                                 dets.ctypes.data, counts.ctypes.data))
-        return dets, counts
+        n = f.shape[0]
+        return self._forward_host(self.L.yolo_b200_forward_yuv, n, f.ctypes.data, fmt, n, sh, sw, int(size[0]), int(size[1]))
 
     def submit_yuv(self, frames, fmt: int, size, dets: np.ndarray, counts: np.ndarray) -> int:
         """Queue one batch of YUV frames [n, *yuv_frame_shape] (a C-contiguous numpy array or a pinned torch tensor) for
@@ -378,23 +366,20 @@ class Context:
         else:
             assert str(frames.dtype) == "torch.uint8" and frames.is_contiguous()
         assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= n and len(counts) >= n
-        t = self.L.yolo_b200_submit_yuv(self._h, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
-                                        dets.ctypes.data, counts.ctypes.data)
-        if t < 0:
-            self._check(t)
-        return t
+        return self._submit(self.L.yolo_b200_submit_yuv, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
+                            dets.ctypes.data, counts.ctypes.data)
 
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
         assert c == 4
-        return self._forward_host(self.L.yolo_b200_forward_int8, x, n, h, w)
+        return self._forward_host(self.L.yolo_b200_forward_int8, n, x.ctypes.data, n, h, w)
 
     def forward_f32(self, nchw: np.ndarray):
         x = np.ascontiguousarray(nchw, dtype=np.float32)
         n, c, h, w = x.shape
         assert c == 3
-        return self._forward_host(self.L.yolo_b200_forward_f32, x, n, h, w)
+        return self._forward_host(self.L.yolo_b200_forward_f32, n, x.ctypes.data, n, h, w)
 
     # -- device-buffer entry points (torch tensors or raw pointers), asynchronous
     def forward_int8_dev(self, d_in, n, h, w, d_dets, d_counts):
