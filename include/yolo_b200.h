@@ -229,6 +229,29 @@ int yolo_b200_forward_yuv(yolo_b200_ctx *ctx, const uint8_t *frames, int format,
 int yolo_b200_submit_yuv(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
                          yolo_b200_det *dets, int32_t *counts);
 
+/* Raw sensor frames in a Bayer mosaic, 8 bits per pixel, as machine-vision and embedded camera modules deliver them: each
+ * frame is demosaiced to BGR exactly as cv2.cvtColor(frame, code) does with OpenCV's default bilinear demosaic, and
+ * resized exactly as yolo_b200_forward_u8bgr_resize does, on the GPU, in one pass, chunk by chunk between the copy and the
+ * first layer; the rest is yolo_b200_forward_u8bgr_resize, so the results equal it run on the cvtColor'd frames.  A frame
+ * crosses the host-to-device link at 1 byte per pixel, against 3 for BGR.  Frames are uint8 [n][sh][sw], frame i at byte
+ * i * sh * sw, no padding, no alignment requirement.  The pattern is named by the sensor's top-left 2x2 (GenICam and
+ * ffmpeg name it so; OpenCV's legacy names count from the second row and column):
+ *   RGGB: cv2 COLOR_BayerRGGB2BGR = COLOR_BayerBG2BGR, ffmpeg bayer_rggb8, GenICam BayerRG8
+ *   BGGR: cv2 COLOR_BayerBGGR2BGR = COLOR_BayerRG2BGR, ffmpeg bayer_bggr8, GenICam BayerBG8
+ *   GRBG: cv2 COLOR_BayerGRBG2BGR = COLOR_BayerGB2BGR, ffmpeg bayer_grbg8, GenICam BayerGR8
+ *   GBRG: cv2 COLOR_BayerGBRG2BGR = COLOR_BayerGR2BGR, ffmpeg bayer_gbrg8, GenICam BayerGB8
+ * sh == h && sw == w demosaics without resizing.  Errors: unknown pattern, n < 0, sh or sw < 3, h or w < 1, null buffers:
+ * E_ARG (-1); a frame over 2 GiB: E_UNSUPPORTED (-3).  n == 0 writes nothing.  The submit form is the asynchronous pair of
+ * yolo_b200_submit_u8bgr (needs n >= 1; + yolo_b200_wait). */
+#define YOLO_B200_BAYER_RGGB  0
+#define YOLO_B200_BAYER_BGGR  1
+#define YOLO_B200_BAYER_GRBG  2
+#define YOLO_B200_BAYER_GBRG  3
+int yolo_b200_forward_bayer(yolo_b200_ctx *ctx, const uint8_t *frames, int pattern, int n, int sh, int sw, int h, int w,
+                            yolo_b200_det *dets, int32_t *counts);
+int yolo_b200_submit_bayer(yolo_b200_ctx *ctx, const uint8_t *frames, int pattern, int n, int sh, int sw, int h, int w,
+                           yolo_b200_det *dets, int32_t *counts);
+
 /* Replaces SlimYOLOv2_quantize_bnfuse.forward(x, quantization=True) inference branch,
  * slim_yolo_v2.py:212-358, for a float NCHW batch (input quantised by a_tracker_in, :218). */
 int yolo_b200_forward_f32(yolo_b200_ctx *ctx, const float *nchw, int n, int h, int w,
@@ -254,6 +277,9 @@ int yolo_b200_forward_u8bgr_ragged_dev(yolo_b200_ctx *ctx, const uint8_t *d_bgr,
 /* YUV frames in device memory (layout and errors as yolo_b200_forward_yuv). */
 int yolo_b200_forward_yuv_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
                               yolo_b200_det *d_dets, int32_t *d_counts);
+/* Bayer frames in device memory (layout and errors as yolo_b200_forward_bayer). */
+int yolo_b200_forward_bayer_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int pattern, int n, int sh, int sw, int h, int w,
+                                yolo_b200_det *d_dets, int32_t *d_counts);
 
 /* Block until everything queued on the context stream is done. */
 int yolo_b200_sync(yolo_b200_ctx *ctx);
@@ -287,6 +313,11 @@ int yolo_b200_resize_u8bgr_ragged(yolo_b200_ctx *ctx, const uint8_t *d_src, int 
  * loaded network; no alignment requirement (d_dst 4-byte aligned and dw a multiple of 4 take word stores). */
 int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int format, int n, int sh, int sw,
                                 uint8_t *d_dst, int dh, int dw);
+/* The front end of yolo_b200_forward_bayer as a stage: n Bayer frames (layout as there) -> uint8 BGR [n][dh][dw][3], equal
+ * to cv2.resize(cv2.cvtColor(frame, code), (dw, dh)); one kernel launch, nothing written at source resolution.  Needs no
+ * loaded network; no alignment requirement (d_dst 4-byte aligned and dw a multiple of 4 take word stores). */
+int yolo_b200_bayer_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int pattern, int n, int sh, int sw,
+                                  uint8_t *d_dst, int dh, int dw);
 /* Host only (no GPU needed), for tests: the per-index programme of that resize along one axis, taps[4*d + {0,1,2,3}] =
  * (source index 0, source index 1, weight 0, weight 1), weights in units of 1/2048; horizontal != 0 re-anchors the tap
  * at the image border as OpenCV's horizontal pass does. */

@@ -8,6 +8,7 @@ BaseTransform does, data/__init__.py:36) is normalised, quantised, convolved, de
     python tools/detect.py --trained_model random --images synthetic:4          (no checkpoint / no images at hand)
     python tools/detect.py --trained_model ckpt.pth --video clip.avi --batch 32  (demo.py's video / camera modes, batched)
     python tools/detect.py --yuv clip.nv12 --yuv_format nv12 --yuv_size 1920x1080   (raw decoder / webcam frames)
+    python tools/detect.py --bayer clip.raw --bayer_pattern rggb --bayer_size 640x480  (raw sensor frames)
 """
 import argparse
 import glob
@@ -79,23 +80,19 @@ def run_video(ctx, args, size):
 
 YUV_FORMATS = {"nv12": lib.YUV_NV12, "i420": lib.YUV_I420, "yuyv": lib.YUV_YUYV}
 YUV_CV2 = {"nv12": cv2.COLOR_YUV2BGR_NV12, "i420": cv2.COLOR_YUV2BGR_I420, "yuyv": cv2.COLOR_YUV2BGR_YUYV}
+BAYER_PATTERNS = {"rggb": lib.BAYER_RGGB, "bggr": lib.BAYER_BGGR, "grbg": lib.BAYER_GRBG, "gbrg": lib.BAYER_GBRG}
+BAYER_CV2 = {"rggb": cv2.COLOR_BayerRGGB2BGR, "bggr": cv2.COLOR_BayerBGGR2BGR, "grbg": cv2.COLOR_BayerGRBG2BGR, "gbrg": cv2.COLOR_BayerGBRG2BGR}
 
 
-def run_yuv(ctx, args, size):
-    """Raw video as `ffmpeg -f rawvideo -pix_fmt {nv12,yuv420p,yuyv422}` writes it (frames back to back, no header): each
-    batch of --batch frames goes to the GPU as it is (1.5 or 2 bytes per pixel, pinned), is converted to BGR, resized,
-    normalised, quantised, convolved, decoded and NMS-ed there (yolo_b200_submit_yuv), with two batches in flight.  The
-    host converts with cvtColor only to draw <out>/detections.avi (MJPG, the source size, --yuv_fps)."""
-    fmt = YUV_FORMATS[args.yuv_format]
-    try:
-        sw, sh = (int(v) for v in args.yuv_size.lower().split("x"))
-        shape = lib.yuv_frame_shape(fmt, sh, sw)
-    except ValueError as e:
-        raise SystemExit("--yuv_size %s: %s" % (args.yuv_size, e))
+def run_raw(ctx, args, size, path, shape, sh, sw, submit, cv2_code, fps, api):
+    """Raw video as `ffmpeg -f rawvideo` writes it (frames of `shape` back to back, no header): each batch of --batch frames
+    goes to the GPU as it is (pinned) through submit(frames, size, dets, counts), which converts, resizes, normalises,
+    quantises, convolves, decodes and NMS-es there, with two batches in flight.  The host converts with cvtColor (cv2_code)
+    only to draw <out>/detections.avi (MJPG, the source size sh x sw, fps)."""
     fbytes = int(np.prod(shape))
     md = 1024
     os.makedirs(args.out, exist_ok=True)
-    writer = cv2.VideoWriter(os.path.join(args.out, "detections.avi"), cv2.VideoWriter_fourcc(*"MJPG"), args.yuv_fps, (sw, sh))
+    writer = cv2.VideoWriter(os.path.join(args.out, "detections.avi"), cv2.VideoWriter_fourcc(*"MJPG"), fps, (sw, sh))
     state = {"frames": 0}
 
     def finish(job):
@@ -103,13 +100,13 @@ def run_yuv(ctx, args, size):
         ctx.wait(ticket)
         for k in range(len(frames)):
             boxes, scores, cls, _ = lib.dets_to_arrays(dets[k], int(min(counts[k], md)))
-            bgr = cv2.cvtColor(frames[k].numpy(), YUV_CV2[args.yuv_format])                 # for drawing only
+            bgr = cv2.cvtColor(frames[k].numpy(), cv2_code)                                  # for drawing only
             writer.write(vis(bgr, boxes * np.array([[sw, sh, sw, sh]], dtype=np.float32), scores, cls, args.visual_threshold))
             print("frame %d: %d detections" % (state["frames"], len(scores)))
             state["frames"] += 1
 
     t0, inflight = time.time(), []
-    with open(args.yuv, "rb") as f:
+    with open(path, "rb") as f:
         while True:
             want = args.batch if not args.max_frames else min(args.batch, args.max_frames - state["frames"] - sum(len(j[1]) for j in inflight))
             if want <= 0:
@@ -123,13 +120,48 @@ def run_yuv(ctx, args, size):
             counts = np.zeros(n, dtype=np.int32)
             if len(inflight) == 2:
                 finish(inflight.pop(0))
-            inflight.append((ctx.submit_yuv(frames, fmt, size, dets, counts), frames, dets, counts))
+            inflight.append((submit(frames, size, dets, counts), frames, dets, counts))
             if n < want:
                 break
     while inflight:
         finish(inflight.pop(0))
     writer.release()
-    print("%d frames, %.1f ms reading, detecting and writing (yolo_b200_submit_yuv / yolo_b200_wait)" % (state["frames"], 1e3 * (time.time() - t0)))
+    print("%d frames, %.1f ms reading, detecting and writing (%s / yolo_b200_wait)" % (state["frames"], 1e3 * (time.time() - t0), api))
+
+
+def frame_size(flag, value):
+    """(sh, sw) of a WxH flag value."""
+    try:
+        sw, sh = (int(v) for v in value.lower().split("x"))
+    except ValueError as e:
+        raise SystemExit("%s %s: %s" % (flag, value, e))
+    return sh, sw
+
+
+def run_yuv(ctx, args, size):
+    """Raw video as `ffmpeg -f rawvideo -pix_fmt {nv12,yuv420p,yuyv422}` writes it: 1.5 or 2 bytes per pixel cross the
+    link and are converted to BGR on the GPU (yolo_b200_submit_yuv)."""
+    fmt = YUV_FORMATS[args.yuv_format]
+    sh, sw = frame_size("--yuv_size", args.yuv_size)
+    try:
+        shape = lib.yuv_frame_shape(fmt, sh, sw)
+    except ValueError as e:
+        raise SystemExit("--yuv_size %s: %s" % (args.yuv_size, e))
+    run_raw(ctx, args, size, args.yuv, shape, sh, sw, lambda fr, sz, d, c: ctx.submit_yuv(fr, fmt, sz, d, c), YUV_CV2[args.yuv_format],
+            args.yuv_fps, "yolo_b200_submit_yuv")
+
+
+def run_bayer(ctx, args, size):
+    """Raw sensor video as `ffmpeg -f rawvideo -pix_fmt bayer_{rggb,bggr,grbg,gbrg}8` writes it: 1 byte per pixel crosses
+    the link and is demosaiced on the GPU (yolo_b200_submit_bayer)."""
+    pattern = BAYER_PATTERNS[args.bayer_pattern]
+    sh, sw = frame_size("--bayer_size", args.bayer_size)
+    try:
+        shape = lib.bayer_source_size(pattern, (sh, sw))
+    except ValueError as e:
+        raise SystemExit("--bayer_size %s: %s" % (args.bayer_size, e))
+    run_raw(ctx, args, size, args.bayer, shape, sh, sw, lambda fr, sz, d, c: ctx.submit_bayer(fr, pattern, sz, d, c),
+            BAYER_CV2[args.bayer_pattern], args.bayer_fps, "yolo_b200_submit_bayer")
 
 
 def main():
@@ -147,7 +179,11 @@ def main():
     ap.add_argument("--yuv_format", default="nv12", choices=sorted(YUV_FORMATS), help="pixel format of --yuv: nv12, i420 (ffmpeg yuv420p) or yuyv (yuyv422)")
     ap.add_argument("--yuv_size", default=None, help="frame size of --yuv as WxH, e.g. 640x480")
     ap.add_argument("--yuv_fps", default=25.0, type=float, help="frame rate written to detections.avi in --yuv mode")
-    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video / --yuv run after this many frames (0 = to the end)")
+    ap.add_argument("--bayer", default=None, help="raw Bayer sensor video file (ffmpeg -f rawvideo, 8 bits per pixel): frames are demosaiced and detected on the GPU and written, annotated, to <out>/detections.avi")
+    ap.add_argument("--bayer_pattern", default="rggb", choices=sorted(BAYER_PATTERNS), help="mosaic of --bayer, named by the sensor's top-left 2x2 (ffmpeg bayer_rggb8 ..., GenICam BayerRG8 ...)")
+    ap.add_argument("--bayer_size", default=None, help="frame size of --bayer as WxH, e.g. 640x480")
+    ap.add_argument("--bayer_fps", default=25.0, type=float, help="frame rate written to detections.avi in --bayer mode")
+    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video / --yuv / --bayer run after this many frames (0 = to the end)")
     ap.add_argument("--out", default="output")
     ap.add_argument("--batch", default=64, type=int)
     args = ap.parse_args()
@@ -166,6 +202,12 @@ def main():
         if not args.yuv_size:
             raise SystemExit("--yuv needs --yuv_size WxH")
         run_yuv(ctx, args, size)
+        ctx.close()
+        return
+    if args.bayer is not None:
+        if not args.bayer_size:
+            raise SystemExit("--bayer needs --bayer_size WxH")
+        run_bayer(ctx, args, size)
         ctx.close()
         return
     if args.video is not None:

@@ -94,13 +94,16 @@ void resize_axis_table(int src, int dst, bool clamp_weights, int index_scale, in
 // xtab: per column (byte offset of tap 0 in its row, weight0 | weight1 << 16), tap 1 = the next pixel; ytab: per row (row 0, row 1, weight0 << 16, weight1 << 16)
 // taps and weights of one geometry (sh, sw) -> (dh, dw) in that layout: ytab [dh], xtab [dw] (host)
 void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab);
-// Source formats: the YUV layouts (NV12, I420, YUYV in cv2's Mat layout, frames packed at yuv_frame_bytes) and uint8 BGR
-enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YUV_YUYV = YOLO_B200_YUV_YUYV, RS_BGR = 3 };
-size_t yuv_frame_bytes(int format, int sh, int sw);        // 0 for an unknown format
+// Source formats: the YUV layouts (NV12, I420, YUYV in cv2's Mat layout), uint8 BGR, and the Bayer mosaics (uint8 [sh][sw],
+// RS_BAYER_* - RS_BAYER_RGGB = column flip | row flip << 1 relative to RGGB).  Camera frames (YUV, Bayer) are packed at
+// camera_frame_bytes.
+enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YUV_YUYV = YOLO_B200_YUV_YUYV, RS_BGR = 3,
+       RS_BAYER_RGGB = 4, RS_BAYER_GRBG = 5, RS_BAYER_GBRG = 6, RS_BAYER_BGGR = 7 };
+size_t camera_frame_bytes(int format, int sh, int sw);     // 0 for BGR or an unknown format
 // Images of different sizes packed back to back in one buffer: frame f starts at byte off of src, its rows are
 // pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
 struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
-// One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for YUV).
+// One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for YUV and Bayer).
 // frames_dev == nullptr: the frames are sh x sw at a uniform stride from src, with the tables ytab [dh], xtab [dw].
 // Otherwise (RS_BGR only) frames_dev[f] describes frame f as above.  A BGR launch reads no byte at or past src + src_bytes.
 cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,

@@ -213,10 +213,98 @@ __device__ __forceinline__ void resize_yuv_rows(const uint8_t *__restrict__ src,
     }
 }
 
+// ---- Bayer sources: cv2.cvtColor(COLOR_Bayer**2BGR) fused in front of the resize ---------------------------------------
+// OpenCV's default bilinear demosaic.  A pattern is named by the sensor's top-left 2x2 (RGGB: row 0 = R G R G .., row 1 =
+// G B G B ..); GRBG flips RGGB's column parity, GBRG its row parity and BGGR both.  At an interior site (1 <= y <= sh - 2,
+// 1 <= x <= sw - 2) with N, S, W, E its 4-neighbours and NW, NE, SW, SE its diagonals, the site's own colour is its byte;
+// at an R or B site G = (N + S + W + E + 2) >> 2 and the opposite colour is (NW + NE + SW + SE + 2) >> 2; at a G site the
+// colour of its horizontal neighbours is (W + E + 1) >> 1 and that of its vertical neighbours (N + S + 1) >> 1.  cv2
+// copies column 1 into column 0 and column sw - 2 into sw - 1, then row 1 into row 0 and row sh - 2 into row sh - 1, so
+// BGR(y, x) = interior(clamp(y, 1, sh - 2), clamp(x, 1, sw - 2)).
+
+// B | G << 8 | R << 16 of the interior site v[1][1] of a 3x3 window (rows i, columns j of a 4x4 grid from (i0, j0));
+// xo, yo: the site's column and row parity counted from an R site
+__device__ __forceinline__ unsigned bayer_site(const unsigned (&v)[4][4], int i0, int j0, unsigned xo, unsigned yo)
+{
+    const int i = i0 + 1, j = j0 + 1;
+    const unsigned hs = v[i][j - 1] + v[i][j + 1], vs = v[i - 1][j] + v[i + 1][j];
+    const unsigned diag = (v[i - 1][j - 1] + v[i - 1][j + 1] + v[i + 1][j - 1] + v[i + 1][j + 1] + 2u) >> 2;
+    const unsigned cross = (hs + vs + 2u) >> 2, hh = (hs + 1u) >> 1, vv = (vs + 1u) >> 1, c = v[i][j];
+    const bool gsite = xo != yo;
+    const unsigned g = gsite ? c : cross;
+    const unsigned r = gsite ? (yo ? vv : hh) : (yo ? diag : c);
+    const unsigned b = gsite ? (yo ? hh : vv) : (yo ? c : diag);
+    return b | (g << 8) | (r << 16);
+}
+
+// The Bayer form of resize_u8c3_kernel's row loop: frames of sh * sw bytes at a uniform stride, the uniform row / column
+// tables (xtab's byte offsets are 3 * source column), resize_combine and the same stores.  A row's taps y0 and
+// y1 (= y0 or y0 + 1) are clamped to [1, sh - 2], a lane's x0 and x1 = min(x0 + 1, sw - 1) to [1, sw - 2]; the four
+// sites (y0 | y1) x (x0 | x1) then lie in one 4x4 grid of raw bytes (rows y0 - 1 .. y0 + 1 and y1 + 1, columns x0 - 1 ..
+// x0 + 1 and x1 + 1), loaded once and demosaiced into the 6-byte tap windows of the BGR kernel.
+// Bounds: with sh, sw >= 3 the clamps keep every row in [0, sh - 1] and every column in [0, sw - 1], so every byte read
+// lies inside its own frame, and frames are those of this launch: nothing is read before src or at or past
+// src + n * sh * sw.  In the chunked host path that is the end of the chunk's landed bytes.  Loads are bytes, so there is
+// no aligned word that could straddle the end and no clamped-row variant.
+// The pattern is compile-time (FMT - RS_BAYER_RGGB = column flip | row flip << 1): the site parities fold into constants.
+template <bool WORD_STORE, int FMT>
+__device__ __forceinline__ void resize_bayer_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
+                                                  const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+{
+    constexpr unsigned PX = (FMT - RS_BAYER_RGGB) & 1, PY = (FMT - RS_BAYER_RGGB) >> 1;
+    const int p = (4 * lane) / 3;
+    const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
+    const size_t frame_bytes = (size_t)sh * sw;
+    const unsigned ymax = (unsigned)sh - 2u, xmax = (unsigned)sw - 2u;
+    unsigned dy = row % (unsigned)dh;
+    const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
+    uint8_t *drow = dst + (size_t)row * dw * 3;
+    for (; row < row_end; ++row) {
+        const int4 yt = __ldg(ytab + dy);
+        const unsigned y0 = min(max((unsigned)yt.x, 1u), ymax), y1 = min(max((unsigned)yt.y, 1u), ymax);
+        const uint8_t *rows[4];                                      // warp-uniform
+        rows[0] = frame + (size_t)(y0 - 1u) * sw; rows[1] = rows[0] + sw; rows[2] = rows[1] + sw;
+        rows[3] = frame + (size_t)(y1 + 1u) * sw;
+        const bool ystep = y1 != y0;
+        const unsigned yo = (y0 ^ PY) & 1u;
+        for (int dx0 = 0; dx0 < dw; dx0 += 32) {
+            const int dx = dx0 + lane;
+            const bool live = dx < dw;
+            unsigned v = 0;
+            if (live) {
+                const int2 xt = __ldg(xtab + dx);
+                const unsigned xa = (unsigned)xt.x / 3u;
+                const unsigned x0 = min(max(xa, 1u), xmax), x1 = min(max(min(xa + 1u, (unsigned)sw - 1u), 1u), xmax);
+                const bool xstep = x1 != x0;
+                unsigned g[4][4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) g[i][j] = __ldg(rows[i] + x0 - 1u + j);
+                    g[i][3] = __ldg(rows[i] + x1 + 1u);
+                }
+                const unsigned xo = (x0 ^ PX) & 1u;
+                const unsigned s00 = bayer_site(g, 0, 0, xo, yo), s01 = bayer_site(g, 0, 1, xo ^ 1u, yo);
+                const unsigned s10 = bayer_site(g, 1, 0, xo, yo ^ 1u), s11 = bayer_site(g, 1, 1, xo ^ 1u, yo ^ 1u);
+                const unsigned t00 = s00, t01 = xstep ? s01 : s00;
+                const unsigned t10 = ystep ? s10 : t00, t11 = ystep ? (xstep ? s11 : s10) : t01;
+                v = resize_combine(t00 | (t01 << 24), t01 >> 8, t10 | (t11 << 24), t11 >> 8, (unsigned)xt.y, (unsigned)yt.z, (unsigned)yt.w);
+            }
+            resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
+        }
+        drow += (size_t)dw * 3;
+        if (++dy == (unsigned)dh) { dy = 0; frame += frame_bytes; }
+    }
+}
+
 // resident CTAs of 256 threads per SM the launch plans for (= the kernel's __launch_bounds__): 6 at 40 registers; the
 // ragged descriptor bookkeeping needs 48 (5 CTAs) and the 4:2:0 instantiations, which keep luma and chroma row pointers of
-// both source rows, up to 64 (4 CTAs) to run without spills; YUYV fits 40
-constexpr int resize_ctas_per_sm(bool ragged, int fmt) { return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 ? 4 : 6; }
+// both source rows, up to 64 (4 CTAs) to run without spills; YUYV fits 40; the Bayer instantiations, which keep a lane's
+// 4x4 grid of raw bytes and four row pointers, need up to 64 (4 CTAs)
+constexpr int resize_ctas_per_sm(bool ragged, int fmt)
+{
+    return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || fmt >= RS_BAYER_RGGB ? 4 : 6;
+}
 
 // One WARP = a contiguous run of output rows of the batch (so the row bookkeeping is incremental: no divisions), one
 // whole row at a time, chunk after chunk: the ~70 instructions of row bookkeeping are paid once per row, not once per
@@ -227,7 +315,8 @@ constexpr int resize_ctas_per_sm(bool ragged, int fmt) { return ragged ? 5 : fmt
 // frames[f] = {byte offset in src, row pitch, geometry g}; its row / column tables are ytab + g * dh / xtab + g * dw.  The
 // descriptor is loaded when dy wraps, so its cost is warp-uniform and paid once per frame.  Otherwise frames are
 // sh x sw and packed at a uniform stride.
-// FMT: the source format, RS_BGR (uint8 [sh][sw][3]) or one of the YUV layouts (uniform stride only; resize_yuv_rows).
+// FMT: the source format, RS_BGR (uint8 [sh][sw][3]), one of the YUV layouts (uniform stride only; resize_yuv_rows) or
+// one of the Bayer patterns (uniform stride only; resize_bayer_rows).
 template <bool WORD_STORE, bool RAGGED, int FMT = RS_BGR>
 __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                           const int2 *__restrict__ xtab, const int4 *__restrict__ ytab,
@@ -238,7 +327,11 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
     unsigned row = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * rows_per_warp;
     if (row >= rows) return;
     const unsigned row_end = min(rows, row + rows_per_warp);
-    if constexpr (FMT != RS_BGR) {
+    if constexpr (FMT >= RS_BAYER_RGGB) {
+        static_assert(!RAGGED, "Bayer sources are one size per launch");
+        resize_bayer_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        return;
+    } else if constexpr (FMT != RS_BGR) {
         static_assert(!RAGGED, "YUV sources are one size per launch");
         resize_yuv_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
         return;
@@ -307,10 +400,15 @@ static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const Res
     return cudaGetLastError();
 }
 
-size_t yuv_frame_bytes(int format, int sh, int sw)
+size_t camera_frame_bytes(int format, int sh, int sw)
 {
     const size_t px = (size_t)sh * sw;
-    return format == RS_YUV_NV12 || format == RS_YUV_I420 ? px + px / 2 : format == RS_YUV_YUYV ? 2 * px : 0;
+    switch (format) {
+    case RS_YUV_NV12: case RS_YUV_I420: return px + px / 2;
+    case RS_YUV_YUYV: return 2 * px;
+    case RS_BAYER_RGGB: case RS_BAYER_GRBG: case RS_BAYER_GBRG: case RS_BAYER_BGGR: return px;
+    default: return 0;
+    }
 }
 
 cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
@@ -323,6 +421,10 @@ cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const Res
     case RS_YUV_NV12: return resize_launch<false, RS_YUV_NV12>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     case RS_YUV_I420: return resize_launch<false, RS_YUV_I420>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     case RS_YUV_YUYV: return resize_launch<false, RS_YUV_YUYV>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_BAYER_RGGB: return resize_launch<false, RS_BAYER_RGGB>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_BAYER_GRBG: return resize_launch<false, RS_BAYER_GRBG>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_BAYER_GBRG: return resize_launch<false, RS_BAYER_GBRG>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_BAYER_BGGR: return resize_launch<false, RS_BAYER_BGGR>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     default:          return cudaErrorInvalidValue;
     }
 }

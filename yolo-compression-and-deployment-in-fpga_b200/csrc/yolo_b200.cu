@@ -641,29 +641,38 @@ static int ensure_pinned(char **p, size_t *cap, size_t need)
     return 0;
 }
 
-// One YUV frame of (format, sh, sw): its byte count, or E_ARG / E_UNSUPPORTED (include/yolo_b200.h)
-static int yuv_check(int format, int sh, int sw, size_t *bytes)
+// One camera frame (a YUV layout or a Bayer pattern) of (format, sh, sw): its byte count, or E_ARG / E_UNSUPPORTED
+// (include/yolo_b200.h).  The formats, the sizes each accepts and their frame bytes (camera_frame_bytes) live here.
+static int source_check(int format, int sh, int sw, size_t *bytes)
 {
-    if (format != YOLO_B200_YUV_NV12 && format != YOLO_B200_YUV_I420 && format != YOLO_B200_YUV_YUYV)
-        return fail(E_ARG, "unknown YUV format %d", format);
+    const bool yuv = format == RS_YUV_NV12 || format == RS_YUV_I420 || format == RS_YUV_YUYV;
+    const bool bayer = format >= RS_BAYER_RGGB && format <= RS_BAYER_BGGR;
+    if (!yuv && !bayer) return fail(E_ARG, "unknown camera format %d", format);
     if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
-    if (sw % 2 || (format != YOLO_B200_YUV_YUYV && sh % 2))
-        return fail(E_ARG, "YUV format %d needs an even %s (%dx%d)", format, format == YOLO_B200_YUV_YUYV ? "width" : "height and width", sh, sw);
-    *bytes = yuv_frame_bytes(format, sh, sw);
-    if (*bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "YUV frame larger than 2 GiB");
+    if (yuv && (sw % 2 || (format != RS_YUV_YUYV && sh % 2)))
+        return fail(E_ARG, "YUV format %d needs an even %s (%dx%d)", format, format == RS_YUV_YUYV ? "width" : "height and width", sh, sw);
+    if (bayer && (sh < 3 || sw < 3)) return fail(E_ARG, "a Bayer frame needs at least 3x3 pixels (%dx%d)", sh, sw);
+    *bytes = camera_frame_bytes(format, sh, sw);
+    if (*bytes > (size_t)INT32_MAX) return fail(E_UNSUPPORTED, "camera frame larger than 2 GiB");
     return 0;
+}
+
+// The source format of a YUV entry point's format (the public codes are the internal ones) and of a Bayer entry point's
+// pattern; anything else goes on as an unknown format, which source_check refuses
+static int yuv_format(int format) { return format >= YOLO_B200_YUV_NV12 && format <= YOLO_B200_YUV_YUYV ? format : -1; }
+static int bayer_format(int pattern)
+{
+    static const int fmt[4] = { RS_BAYER_RGGB, RS_BAYER_BGGR, RS_BAYER_GRBG, RS_BAYER_GBRG };     // YOLO_B200_BAYER_* order
+    static_assert(YOLO_B200_BAYER_RGGB == 0 && YOLO_B200_BAYER_BGGR == 1 && YOLO_B200_BAYER_GRBG == 2 && YOLO_B200_BAYER_GBRG == 3, "pattern codes");
+    return pattern >= 0 && pattern < 4 ? fmt[pattern] : -1;
 }
 
 int yolo_b200_yuv_frame_bytes(int format, int sh, int sw)
 {
     size_t b = 0;
-    int rc = yuv_check(format, sh, sw, &b); if (rc) return rc;
+    int rc = source_check(yuv_format(format), sh, sw, &b); if (rc) return rc;
     return (int)b;
 }
-
-// A YUV entry point's format as a source format: RS_BGR is not a YUV format a caller may name, so it goes on as an
-// unknown one, which yuv_check refuses
-static int yuv_format(int format) { return format == RS_BGR ? -1 : format; }
 
 // Where the n frames of one call are and how they become dh x dw frames of the network input (plan_sources, net_plan).
 enum { RESIZE_NONE, RESIZE_UNIFORM, RESIZE_RAGGED };
@@ -677,10 +686,10 @@ struct SourcePlan {
     size_t at(int f) const { return off.empty() ? (size_t)f * frame_bytes : off[f]; }     // byte offset of frame f
 };
 
-// The plan of n frames of format fmt (RS_BGR or a YUV layout) for the network size dh x dw.  Frame i has the source size
+// The plan of n frames of format fmt (RS_BGR or a camera format) for the network size dh x dw.  Frame i has the source size
 // src_hw[2 * i * stride] x src_hw[2 * i * stride + 1] (stride 0: one size for all, checked also when n == 0).  One rule
 // picks the resize: none for a forward call whose only source size is dh x dw in BGR (the frames are the network input
-// as they are), uniform for one source size or any YUV call, ragged for several source sizes.
+// as they are), uniform for one source size or any camera-format call, ragged for several source sizes.
 static int plan_sources(int fmt, int n, const int32_t *src_hw, int stride, int dh, int dw, bool forward, SourcePlan &p)
 {
     p = SourcePlan();
@@ -688,7 +697,7 @@ static int plan_sources(int fmt, int n, const int32_t *src_hw, int stride, int d
     const int m = stride ? n : 1;                                // sizes to read
     if (m > 0 && !src_hw) return fail(E_ARG, "null src_hw");
     if (fmt != RS_BGR) {
-        int rc = yuv_check(fmt, src_hw[0], src_hw[1], &p.frame_bytes); if (rc) return rc;
+        int rc = source_check(fmt, src_hw[0], src_hw[1], &p.frame_bytes); if (rc) return rc;
         p.geoms.push_back({src_hw[0], src_hw[1]});
         p.mode = RESIZE_UNIFORM;
         return 0;
@@ -813,6 +822,12 @@ int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int form
 {
     const int32_t hw[2] = { sh, sw };
     return resize_stage(c, yuv_format(format), d_src, n, hw, 0, d_dst, dh, dw);
+}
+
+int yolo_b200_bayer_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int pattern, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+{
+    const int32_t hw[2] = { sh, sw };
+    return resize_stage(c, bayer_format(pattern), d_src, n, hw, 0, d_dst, dh, dw);
 }
 
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
@@ -1369,6 +1384,13 @@ int yolo_b200_forward_yuv_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int for
     return forward_resize_dev(c, yuv_format(format), d_frames, n, hw, 0, h, w, d_dets, d_counts);
 }
 
+int yolo_b200_forward_bayer_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int pattern, int n, int sh, int sw, int h, int w,
+                                yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return forward_resize_dev(c, bayer_format(pattern), d_frames, n, hw, 0, h, w, d_dets, d_counts);
+}
+
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 { return forward_dev(c, IN_F32, d_nchw, n, h, w, d_dets, d_counts); }
 
@@ -1599,6 +1621,18 @@ int yolo_b200_submit_yuv(yolo_b200_ctx *c, const uint8_t *frames, int format, in
 {
     const int32_t hw[2] = { sh, sw };
     return host_resize(c, true, yuv_format(format), frames, n, hw, 0, h, w, dets, counts);
+}
+int yolo_b200_forward_bayer(yolo_b200_ctx *c, const uint8_t *frames, int pattern, int n, int sh, int sw, int h, int w,
+                            yolo_b200_det *dets, int32_t *counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, false, bayer_format(pattern), frames, n, hw, 0, h, w, dets, counts);
+}
+int yolo_b200_submit_bayer(yolo_b200_ctx *c, const uint8_t *frames, int pattern, int n, int sh, int sw, int h, int w,
+                           yolo_b200_det *dets, int32_t *counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, true, bayer_format(pattern), frames, n, hw, 0, h, w, dets, counts);
 }
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------

@@ -21,6 +21,8 @@ ROUND_RNE, ROUND_FLOOR, ROUND_HALF_UP = 0, 1, 2
 WLAYOUT_OIHW, WLAYOUT_OHWI, WLAYOUT_WEIGHT_H = 0, 1, 2
 HEAD_PYTHON, HEAD_C = 0, 1
 YUV_NV12, YUV_I420, YUV_YUYV = 0, 1, 2      # cv2.COLOR_YUV2BGR_NV12 / _I420 / _YUYV frames (yolo_b200_forward_yuv)
+# Bayer mosaics named by the sensor's top-left 2x2 (yolo_b200_forward_bayer): cv2.COLOR_BayerRGGB2BGR / _BGGR / _GRBG / _GBRG
+BAYER_RGGB, BAYER_BGGR, BAYER_GRBG, BAYER_GBRG = 0, 1, 2, 3
 
 EXPORTS = [
     "yolo_b200_abi_version", "yolo_b200_last_error", "yolo_b200_cstride", "yolo_b200_default_params",
@@ -40,6 +42,7 @@ EXPORTS = [
     "yolo_b200_forward_u8bgr_ragged_dev",
     "yolo_b200_yuv_frame_bytes", "yolo_b200_yuv_to_bgr_resize", "yolo_b200_forward_yuv", "yolo_b200_submit_yuv",
     "yolo_b200_forward_yuv_dev",
+    "yolo_b200_bayer_to_bgr_resize", "yolo_b200_forward_bayer", "yolo_b200_submit_bayer", "yolo_b200_forward_bayer_dev",
 ]
 
 
@@ -114,6 +117,9 @@ def load_library(path: Optional[str] = None):
     L.yolo_b200_yuv_frame_bytes.argtypes = [i32, i32, i32]
     L.yolo_b200_yuv_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
     for name in ("yolo_b200_forward_yuv", "yolo_b200_submit_yuv", "yolo_b200_forward_yuv_dev"):
+        getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
+    L.yolo_b200_bayer_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
+    for name in ("yolo_b200_forward_bayer", "yolo_b200_submit_bayer", "yolo_b200_forward_bayer_dev"):
         getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.yolo_b200_quantize_rgb444.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_quantize_f32.argtypes = [vp, vp, i32, i32, i32, vp]
@@ -213,6 +219,17 @@ def yuv_source_size(fmt: int, frame_shape) -> "tuple[int, int]":
     if size is None or yuv_frame_shape(fmt, *size) != fs:
         raise ValueError("%s is not the shape of a YUV format %r frame" % (fs, fmt))
     return size
+
+
+def bayer_source_size(pattern: int, frame_shape) -> "tuple[int, int]":
+    """(sh, sw) of Bayer frames [n][sh][sw] (frame_shape without n).  Raises ValueError for an unknown pattern or a frame
+    smaller than 3x3 (cv2 itself returns zeros there; the library refuses such frames)."""
+    if pattern not in (BAYER_RGGB, BAYER_BGGR, BAYER_GRBG, BAYER_GBRG):
+        raise ValueError("unknown Bayer pattern %r" % (pattern,))
+    fs = tuple(int(x) for x in frame_shape)
+    if len(fs) != 2 or fs[0] < 3 or fs[1] < 3:
+        raise ValueError("%s is not the shape of a Bayer frame [sh][sw] of at least 3x3" % (fs,))
+    return fs
 
 
 class Context:
@@ -369,6 +386,34 @@ class Context:
         return self._submit(self.L.yolo_b200_submit_yuv, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
                             dets.ctypes.data, counts.ctypes.data)
 
+    def forward_bayer(self, frames: np.ndarray, pattern: int, size):
+        """uint8 Bayer frames [n][sh][sw] (raw sensor mosaic, pattern BAYER_*) -> (dets [n][max_det], counts [n]):
+        cv2.cvtColor to BGR, cv2.resize to size = (h, w) and the rest of forward_u8bgr_resize, all on the GPU; the frames
+        cross the link as they are (1 byte per pixel)."""
+        f = np.ascontiguousarray(frames, dtype=np.uint8)
+        if f.ndim != 3:
+            raise ValueError("Bayer frames are [n][sh][sw], got shape %s" % (f.shape,))
+        sh, sw = bayer_source_size(pattern, f.shape[1:])
+        n = f.shape[0]
+        return self._forward_host(self.L.yolo_b200_forward_bayer, n, f.ctypes.data, pattern, n, sh, sw, int(size[0]), int(size[1]))
+
+    def submit_bayer(self, frames, pattern: int, size, dets: np.ndarray, counts: np.ndarray) -> int:
+        """Queue one batch of Bayer frames [n][sh][sw] (a C-contiguous numpy array or a pinned torch tensor) for
+        size = (h, w); frames, dets [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until
+        wait(ticket).  Returns the ticket."""
+        shape = tuple(frames.shape)
+        if len(shape) != 3:
+            raise ValueError("Bayer frames are [n][sh][sw], got shape %s" % (shape,))
+        sh, sw = bayer_source_size(pattern, shape[1:])
+        n = shape[0]
+        if isinstance(frames, np.ndarray):
+            assert frames.dtype == np.uint8 and frames.flags.c_contiguous
+        else:
+            assert str(frames.dtype) == "torch.uint8" and frames.is_contiguous()
+        assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= n and len(counts) >= n
+        return self._submit(self.L.yolo_b200_submit_bayer, _ptr(frames), pattern, n, sh, sw, int(size[0]), int(size[1]),
+                            dets.ctypes.data, counts.ctypes.data)
+
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
@@ -415,6 +460,14 @@ class Context:
     def yuv_to_bgr_resize(self, d_src, fmt, n, sh, sw, d_dst, dh, dw):
         """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device YUV frames into d_dst uint8 [n][dh][dw][3]."""
         self._check(self.L.yolo_b200_yuv_to_bgr_resize(self._h, _ptr(d_src), fmt, n, sh, sw, _ptr(d_dst), dh, dw))
+
+    def forward_bayer_dev(self, d_in, pattern, n, sh, sw, h, w, d_dets, d_counts):
+        """n Bayer frames of source size sh x sw packed in device memory (layout of forward_bayer)."""
+        self._check(self.L.yolo_b200_forward_bayer_dev(self._h, _ptr(d_in), pattern, n, sh, sw, h, w, _ptr(d_dets), _ptr(d_counts)))
+
+    def bayer_to_bgr_resize(self, d_src, pattern, n, sh, sw, d_dst, dh, dw):
+        """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device Bayer frames into d_dst uint8 [n][dh][dw][3]."""
+        self._check(self.L.yolo_b200_bayer_to_bgr_resize(self._h, _ptr(d_src), pattern, n, sh, sw, _ptr(d_dst), dh, dw))
 
     def resize_u8bgr(self, d_src, n, sh, sw, d_dst, dh, dw):
         """cv2.resize (bilinear) of n uint8 [sh][sw][3] device images into d_dst [n][dh][dw][3]."""
