@@ -252,6 +252,35 @@ int yolo_b200_forward_bayer(yolo_b200_ctx *ctx, const uint8_t *frames, int patte
 int yolo_b200_submit_bayer(yolo_b200_ctx *ctx, const uint8_t *frames, int pattern, int n, int sh, int sw, int h, int w,
                            yolo_b200_det *dets, int32_t *counts);
 
+/* Frames in the pixel formats most other code holds: packed RGB (PIL, PyAV rgb24, dataset loaders), RGBA / BGRA (screen
+ * capture, GUI toolkits, browsers, WebRTC, Android), 8-bit gray (monochrome machine-vision cameras, GenICam Mono8, thermal
+ * cameras) and planar RGB (torch CHW uint8, torchvision.io.decode_image / decode_jpeg).  Each frame is converted to BGR
+ * exactly as cv2.cvtColor does and resized exactly as yolo_b200_forward_u8bgr_resize does, on the GPU, in one pass, chunk
+ * by chunk between the copy and the first layer; the rest is yolo_b200_forward_u8bgr_resize, so the results equal it run on
+ * the cvtColor'd frames.  A gray frame crosses the host-to-device link at 1 byte per pixel and RGBA / BGRA at 4, against 3
+ * for BGR.  Frames are packed at yolo_b200_pix_frame_bytes() with no padding (frame i at byte i * frame_bytes), no
+ * alignment requirement (4-byte-aligned RGBA / BGRA sources take word loads, same results):
+ *   RGB:        uint8 [sh][sw][3] R,G,B        cv2 COLOR_RGB2BGR,  ffmpeg rgb24
+ *   RGBA:       uint8 [sh][sw][4] R,G,B,A      cv2 COLOR_RGBA2BGR, ffmpeg rgba    (alpha ignored)
+ *   BGRA:       uint8 [sh][sw][4] B,G,R,A      cv2 COLOR_BGRA2BGR, ffmpeg bgra    (alpha ignored)
+ *   GRAY:       uint8 [sh][sw]                 cv2 COLOR_GRAY2BGR, ffmpeg gray
+ *   RGB_PLANAR: uint8 [3][sh][sw], planes R,G,B (torch CHW): cv2 COLOR_RGB2BGR of the HWC transpose; no ffmpeg name
+ *               (ffmpeg's gbrp orders the planes G,B,R)
+ * sh == h && sw == w converts without resizing.  Errors: unknown format, n < 0, sh / sw / h / w < 1, null buffers: E_ARG (-1);
+ * a frame over 2 GiB: E_UNSUPPORTED (-3).  n == 0 writes nothing.  The submit form is the asynchronous pair of
+ * yolo_b200_submit_u8bgr (needs n >= 1; + yolo_b200_wait). */
+#define YOLO_B200_PIX_RGB        0
+#define YOLO_B200_PIX_RGBA       1
+#define YOLO_B200_PIX_BGRA       2
+#define YOLO_B200_PIX_GRAY       3
+#define YOLO_B200_PIX_RGB_PLANAR 4
+/* Bytes of one frame of this format and size (host only, no GPU needed), or a negative error as above. */
+int yolo_b200_pix_frame_bytes(int format, int sh, int sw);
+int yolo_b200_forward_pix(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                          yolo_b200_det *dets, int32_t *counts);
+int yolo_b200_submit_pix(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                         yolo_b200_det *dets, int32_t *counts);
+
 /* Replaces SlimYOLOv2_quantize_bnfuse.forward(x, quantization=True) inference branch,
  * slim_yolo_v2.py:212-358, for a float NCHW batch (input quantised by a_tracker_in, :218). */
 int yolo_b200_forward_f32(yolo_b200_ctx *ctx, const float *nchw, int n, int h, int w,
@@ -280,6 +309,11 @@ int yolo_b200_forward_yuv_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int f
 /* Bayer frames in device memory (layout and errors as yolo_b200_forward_bayer). */
 int yolo_b200_forward_bayer_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int pattern, int n, int sh, int sw, int h, int w,
                                 yolo_b200_det *d_dets, int32_t *d_counts);
+
+/* Frames of a pixel format in device memory (layout and errors as yolo_b200_forward_pix), e.g. torchvision's decoded
+ * uint8 [3][sh][sw] tensors as YOLO_B200_PIX_RGB_PLANAR. */
+int yolo_b200_forward_pix_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
+                              yolo_b200_det *d_dets, int32_t *d_counts);
 
 /* Block until everything queued on the context stream is done. */
 int yolo_b200_sync(yolo_b200_ctx *ctx);
@@ -318,6 +352,12 @@ int yolo_b200_yuv_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int fo
  * loaded network; no alignment requirement (d_dst 4-byte aligned and dw a multiple of 4 take word stores). */
 int yolo_b200_bayer_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int pattern, int n, int sh, int sw,
                                   uint8_t *d_dst, int dh, int dw);
+/* The front end of yolo_b200_forward_pix as a stage: n frames of a pixel format (layout as there) -> uint8 BGR
+ * [n][dh][dw][3], equal to cv2.resize(cv2.cvtColor(frame, code), (dw, dh)); one kernel launch, nothing written at source
+ * resolution.  Needs no loaded network; no alignment requirement (d_dst 4-byte aligned and dw a multiple of 4 take word
+ * stores). */
+int yolo_b200_pix_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int format, int n, int sh, int sw,
+                                uint8_t *d_dst, int dh, int dw);
 /* Host only (no GPU needed), for tests: the per-index programme of that resize along one axis, taps[4*d + {0,1,2,3}] =
  * (source index 0, source index 1, weight 0, weight 1), weights in units of 1/2048; horizontal != 0 re-anchors the tap
  * at the image border as OpenCV's horizontal pass does. */

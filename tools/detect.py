@@ -9,6 +9,7 @@ BaseTransform does, data/__init__.py:36) is normalised, quantised, convolved, de
     python tools/detect.py --trained_model ckpt.pth --video clip.avi --batch 32  (demo.py's video / camera modes, batched)
     python tools/detect.py --yuv clip.nv12 --yuv_format nv12 --yuv_size 1920x1080   (raw decoder / webcam frames)
     python tools/detect.py --bayer clip.raw --bayer_pattern rggb --bayer_size 640x480  (raw sensor frames)
+    python tools/detect.py --pix clip.rgb --pix_format rgb24 --pix_size 640x480     (raw RGB / RGBA / BGRA / gray frames)
 """
 import argparse
 import glob
@@ -82,6 +83,9 @@ YUV_FORMATS = {"nv12": lib.YUV_NV12, "i420": lib.YUV_I420, "yuyv": lib.YUV_YUYV}
 YUV_CV2 = {"nv12": cv2.COLOR_YUV2BGR_NV12, "i420": cv2.COLOR_YUV2BGR_I420, "yuyv": cv2.COLOR_YUV2BGR_YUYV}
 BAYER_PATTERNS = {"rggb": lib.BAYER_RGGB, "bggr": lib.BAYER_BGGR, "grbg": lib.BAYER_GRBG, "gbrg": lib.BAYER_GBRG}
 BAYER_CV2 = {"rggb": cv2.COLOR_BayerRGGB2BGR, "bggr": cv2.COLOR_BayerBGGR2BGR, "grbg": cv2.COLOR_BayerGRBG2BGR, "gbrg": cv2.COLOR_BayerGBRG2BGR}
+
+PIX_FORMATS = {"rgb24": lib.PIX_RGB, "rgba": lib.PIX_RGBA, "bgra": lib.PIX_BGRA, "gray": lib.PIX_GRAY}
+PIX_CV2 = {"rgb24": cv2.COLOR_RGB2BGR, "rgba": cv2.COLOR_RGBA2BGR, "bgra": cv2.COLOR_BGRA2BGR, "gray": cv2.COLOR_GRAY2BGR}
 
 
 def run_raw(ctx, args, size, path, shape, sh, sw, submit, cv2_code, fps, api):
@@ -164,6 +168,19 @@ def run_bayer(ctx, args, size):
             BAYER_CV2[args.bayer_pattern], args.bayer_fps, "yolo_b200_submit_bayer")
 
 
+def run_pix(ctx, args, size):
+    """Raw video as `ffmpeg -f rawvideo -pix_fmt {rgb24,rgba,bgra,gray}` writes it: the frames cross the link as they are (3,
+    4, 4 or 1 bytes per pixel) and are converted to BGR on the GPU (yolo_b200_submit_pix)."""
+    fmt = PIX_FORMATS[args.pix_format]
+    sh, sw = frame_size("--pix_size", args.pix_size)
+    try:
+        shape = lib.pix_frame_shape(fmt, sh, sw)
+    except ValueError as e:
+        raise SystemExit("--pix_size %s: %s" % (args.pix_size, e))
+    run_raw(ctx, args, size, args.pix, shape, sh, sw, lambda fr, sz, d, c: ctx.submit_pix(fr, fmt, sz, d, c), PIX_CV2[args.pix_format],
+            args.pix_fps, "yolo_b200_submit_pix")
+
+
 def main():
     ap = argparse.ArgumentParser(description="slim_yolo_v2 fixed-point detection on B200")
     ap.add_argument("-v", "--version", default="slim_yolo_v2_q_bf", help="only slim_yolo_v2_q_bf runs on this path")
@@ -183,7 +200,11 @@ def main():
     ap.add_argument("--bayer_pattern", default="rggb", choices=sorted(BAYER_PATTERNS), help="mosaic of --bayer, named by the sensor's top-left 2x2 (ffmpeg bayer_rggb8 ..., GenICam BayerRG8 ...)")
     ap.add_argument("--bayer_size", default=None, help="frame size of --bayer as WxH, e.g. 640x480")
     ap.add_argument("--bayer_fps", default=25.0, type=float, help="frame rate written to detections.avi in --bayer mode")
-    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video / --yuv / --bayer run after this many frames (0 = to the end)")
+    ap.add_argument("--pix", default=None, help="raw RGB, RGBA, BGRA or gray video file (ffmpeg -f rawvideo): frames are converted and detected on the GPU and written, annotated, to <out>/detections.avi")
+    ap.add_argument("--pix_format", default="rgb24", choices=sorted(PIX_FORMATS), help="pixel format of --pix, named as ffmpeg's -pix_fmt")
+    ap.add_argument("--pix_size", default=None, help="frame size of --pix as WxH, e.g. 640x480")
+    ap.add_argument("--pix_fps", default=25.0, type=float, help="frame rate written to detections.avi in --pix mode")
+    ap.add_argument("--max_frames", default=0, type=int, help="stop a --video / --yuv / --bayer / --pix run after this many frames (0 = to the end)")
     ap.add_argument("--out", default="output")
     ap.add_argument("--batch", default=64, type=int)
     args = ap.parse_args()
@@ -208,6 +229,12 @@ def main():
         if not args.bayer_size:
             raise SystemExit("--bayer needs --bayer_size WxH")
         run_bayer(ctx, args, size)
+        ctx.close()
+        return
+    if args.pix is not None:
+        if not args.pix_size:
+            raise SystemExit("--pix needs --pix_size WxH")
+        run_pix(ctx, args, size)
         ctx.close()
         return
     if args.video is not None:

@@ -94,18 +94,24 @@ void resize_axis_table(int src, int dst, bool clamp_weights, int index_scale, in
 // xtab: per column (byte offset of tap 0 in its row, weight0 | weight1 << 16), tap 1 = the next pixel; ytab: per row (row 0, row 1, weight0 << 16, weight1 << 16)
 // taps and weights of one geometry (sh, sw) -> (dh, dw) in that layout: ytab [dh], xtab [dw] (host)
 void resize_geometry_tables(int sh, int sw, int dh, int dw, int4 *ytab, int2 *xtab);
-// Source formats: the YUV layouts (NV12, I420, YUYV in cv2's Mat layout), uint8 BGR, and the Bayer mosaics (uint8 [sh][sw],
-// RS_BAYER_* - RS_BAYER_RGGB = column flip | row flip << 1 relative to RGGB).  Camera frames (YUV, Bayer) are packed at
+// Source formats: the YUV layouts (NV12, I420, YUYV in cv2's Mat layout), uint8 BGR, the Bayer mosaics (uint8 [sh][sw],
+// RS_BAYER_* - RS_BAYER_RGGB = column flip | row flip << 1 relative to RGGB), and the pixel formats of
+// yolo_b200_forward_pix (RS_RGB + YOLO_B200_PIX_*).  Camera frames (YUV, Bayer, pixel formats) are packed at
 // camera_frame_bytes.
 enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YUV_YUYV = YOLO_B200_YUV_YUYV, RS_BGR = 3,
-       RS_BAYER_RGGB = 4, RS_BAYER_GRBG = 5, RS_BAYER_GBRG = 6, RS_BAYER_BGGR = 7 };
+       RS_BAYER_RGGB = 4, RS_BAYER_GRBG = 5, RS_BAYER_GBRG = 6, RS_BAYER_BGGR = 7,
+       RS_RGB = 8, RS_RGBA = 9, RS_BGRA = 10, RS_GRAY = 11, RS_RGB_PLANAR = 12 };
+static_assert(RS_RGBA - RS_RGB == YOLO_B200_PIX_RGBA && RS_BGRA - RS_RGB == YOLO_B200_PIX_BGRA && RS_GRAY - RS_RGB == YOLO_B200_PIX_GRAY &&
+              RS_RGB_PLANAR - RS_RGB == YOLO_B200_PIX_RGB_PLANAR && YOLO_B200_PIX_RGB == 0, "pixel format codes");
 size_t camera_frame_bytes(int format, int sh, int sw);     // 0 for BGR or an unknown format
 // Images of different sizes packed back to back in one buffer: frame f starts at byte off of src, its rows are
 // pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
 struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
-// One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for YUV and Bayer).
+// One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for the
+// formats other than BGR).
 // frames_dev == nullptr: the frames are sh x sw at a uniform stride from src, with the tables ytab [dh], xtab [dw].
-// Otherwise (RS_BGR only) frames_dev[f] describes frame f as above.  A BGR launch reads no byte at or past src + src_bytes.
+// Otherwise (RS_BGR only) frames_dev[f] describes frame f as above.  A BGR or RGB launch reads no byte at or past
+// src + src_bytes; the other formats read only the bytes of their own frames.
 cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
                         uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
 

@@ -72,12 +72,16 @@ __device__ __forceinline__ void resize_row_taps(const unsigned char *__restrict_
 
 // a01 = weight0 | weight1 << 16 (units of 1/2048), B0/B1 = row weights << 16.  Per channel: the horizontal pass of one
 // row is one PRMT (tap 0 and tap 1 bytes side by side) + one unsigned DP2A; `(b * (h >> 4)) >> 16` is a high multiply.
+// The window of a row is lo | hi << 32: tap 0 from byte 0, tap 1 from byte TAP1 (3 for packed 3-byte pixels, 4 for one
+// 32-bit word per pixel).  RGB: the pixels are R, G, B, so output channel ch (B, G, R) comes from byte 2 - ch of a tap.
+template <bool RGB = false, unsigned TAP1 = 3>
 __device__ __forceinline__ unsigned resize_combine(unsigned lo0, unsigned hi0, unsigned lo1, unsigned hi1, unsigned a01, unsigned B0, unsigned B1)
 {
     unsigned o[3];
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) {
-        const unsigned sel = (unsigned)ch | ((unsigned)(3 + ch) << 4);          // bytes ch and 3 + ch of the 8-byte window
+        const unsigned c = RGB ? 2u - (unsigned)ch : (unsigned)ch;
+        const unsigned sel = c | ((TAP1 + c) << 4);                              // bytes c and TAP1 + c of the 8-byte window
         const unsigned h0 = __dp2a_lo(a01, __byte_perm(lo0, hi0, sel), 0u);    // horizontal pass, scale 2^11
         const unsigned h1 = __dp2a_lo(a01, __byte_perm(lo1, hi1, sel), 0u);
         o[ch] = (__umulhi(B0, h0 >> 4) + __umulhi(B1, h1 >> 4) + 2u) >> 2;      // <= 255 by construction
@@ -102,7 +106,8 @@ __device__ __forceinline__ void resize_store(unsigned v, bool live, int dx0, int
 }
 
 // One output row of the batch: one thread = one output pixel, a warp = 32 consecutive pixels = 96 contiguous output bytes.
-template <bool WORD_STORE, bool CLAMP>
+// RGB: the source pixels are R, G, B (resize_combine).
+template <bool WORD_STORE, bool CLAMP, bool RGB>
 __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__ r0, const unsigned char *__restrict__ r1,
                                                unsigned d0, unsigned d1, unsigned lim0, unsigned lim1, unsigned B0, unsigned B1,
                                                const int2 *__restrict__ xtab, uint8_t *__restrict__ drow, int dw,
@@ -117,7 +122,7 @@ __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__
             unsigned lo0, hi0, lo1, hi1;
             resize_row_taps<CLAMP>(r0, (unsigned)xt.x + d0, lim0, lo0, hi0);
             resize_row_taps<CLAMP>(r1, (unsigned)xt.x + d1, lim1, lo1, hi1);
-            v = resize_combine(lo0, hi0, lo1, hi1, (unsigned)xt.y, B0, B1);
+            v = resize_combine<RGB>(lo0, hi0, lo1, hi1, (unsigned)xt.y, B0, B1);
         }
         resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
     }
@@ -297,13 +302,102 @@ __device__ __forceinline__ void resize_bayer_rows(const uint8_t *__restrict__ sr
     }
 }
 
+// ---- RGB, RGBA, BGRA, gray and planar RGB sources: cv2.cvtColor(COLOR_RGB2BGR / _RGBA2BGR / _BGRA2BGR / _GRAY2BGR) ------
+// Each conversion selects (or, for gray, replicates) channels per pixel, and the resize treats the channels alike, so
+// resize(convert(f)) = convert(resize(f)): the kernel resizes the source's own channels and writes them in B, G, R order.
+// Packed RGB is the BGR row loop with the channel order swapped in resize_combine.  The others use resize_pix_rows.
+// The RGBA / BGRA loops read one aligned 32-bit word per tap pixel when src is 4-byte aligned (frames are 4 * sh * sw
+// bytes, so every frame and row then is); resize_u8c3 sends other sources to these byte-load variants of the two formats:
+enum { RS_RGBA_BYTES = 13, RS_BGRA_BYTES = 14 };
+
+// The horizontal and vertical pass of one channel: p0 / p1 = tap 0 | tap 1 << 8 of the two source rows (resize_combine).
+__device__ __forceinline__ unsigned resize_channel(unsigned p0, unsigned p1, unsigned a01, unsigned B0, unsigned B1)
+{
+    return (__umulhi(B0, __dp2a_lo(a01, p0, 0u) >> 4) + __umulhi(B1, __dp2a_lo(a01, p1, 0u) >> 4) + 2u) >> 2;
+}
+
+// bytes 0..2 (the colour channels) of pixel x of a 4-byte-per-pixel row, as one word
+__device__ __forceinline__ unsigned rgba_bytes(const uint8_t *row, unsigned x)
+{
+    const uint8_t *q = row + 4u * x;
+    return (unsigned)__ldg(q) | ((unsigned)__ldg(q + 1) << 8) | ((unsigned)__ldg(q + 2) << 16);
+}
+
+// The gray / RGBA / BGRA / planar RGB form of resize_u8c3_kernel's row loop: frames of BPP * sh * sw bytes at a uniform
+// stride, the uniform row / column tables (xtab's byte offsets are 3 * source column), the same stores.  Per source row
+// and lane, the two tap pixels x0 and x1 = min(x0 + 1, sw - 1) (tap 1 has weight 0 where x0 = sw - 1):
+//   GRAY:          two bytes, one channel resized and replicated into B, G and R (a third of the arithmetic);
+//   RGBA / BGRA:   two aligned words (or, in the byte variants, the three colour bytes of each), resize_combine;
+//   RGB_PLANAR:    two bytes from each of the three planes, whose row pointers are warp-uniform.
+// Bounds: a source row index comes from ytab (clamped to [0, sh - 1]) and a column from xtab (in [0, sw - 1]) or its
+// clamped successor, so every byte read (a word: the pixel's own four bytes) lies inside its own frame, and frames are
+// those of this launch: nothing is read before src or at or past src + n * frame_bytes.  In the chunked host path that is
+// the end of the chunk's landed bytes.  So there is no clamped-row variant.
+template <bool WORD_STORE, int FMT>
+__device__ __forceinline__ void resize_pix_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
+                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+{
+    constexpr bool GRAY = FMT == RS_GRAY, PLANAR = FMT == RS_RGB_PLANAR;
+    constexpr bool WORDS = FMT == RS_RGBA || FMT == RS_BGRA, RGB = FMT == RS_RGBA || FMT == RS_RGBA_BYTES;
+    constexpr unsigned BPP = GRAY ? 1 : PLANAR ? 3 : 4;           // frame bytes per pixel
+    constexpr unsigned ROW = PLANAR ? 1 : BPP;                    // row bytes per pixel (of one plane)
+    const int p = (4 * lane) / 3;
+    const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
+    const size_t plane = (size_t)sh * sw, frame_bytes = BPP * plane;
+    unsigned dy = row % (unsigned)dh;
+    const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
+    uint8_t *drow = dst + (size_t)row * dw * 3;
+    for (; row < row_end; ++row) {
+        const int4 yt = __ldg(ytab + dy);
+        const uint8_t *r0 = frame + (size_t)yt.x * sw * ROW, *r1 = frame + (size_t)yt.y * sw * ROW;   // warp-uniform
+        for (int dx0 = 0; dx0 < dw; dx0 += 32) {
+            const int dx = dx0 + lane;
+            const bool live = dx < dw;
+            unsigned v = 0;
+            if (live) {
+                const int2 xt = __ldg(xtab + dx);
+                const unsigned x0 = (unsigned)xt.x / 3u, x1 = min(x0 + 1u, (unsigned)sw - 1u);
+                const unsigned a01 = (unsigned)xt.y, B0 = (unsigned)yt.z, B1 = (unsigned)yt.w;
+                if constexpr (GRAY) {
+                    v = 0x010101u * resize_channel(__ldg(r0 + x0) | ((unsigned)__ldg(r0 + x1) << 8),
+                                                   __ldg(r1 + x0) | ((unsigned)__ldg(r1 + x1) << 8), a01, B0, B1);
+                } else if constexpr (PLANAR) {
+#pragma unroll
+                    for (int ch = 0; ch < 3; ++ch) {                  // output B, G, R = planes 2, 1, 0
+                        const uint8_t *q0 = r0 + (2 - ch) * plane, *q1 = r1 + (2 - ch) * plane;
+                        v |= resize_channel(__ldg(q0 + x0) | ((unsigned)__ldg(q0 + x1) << 8),
+                                            __ldg(q1 + x0) | ((unsigned)__ldg(q1 + x1) << 8), a01, B0, B1) << (8 * ch);
+                    }
+                } else if constexpr (WORDS) {
+                    const unsigned *w0 = reinterpret_cast<const unsigned *>(r0), *w1 = reinterpret_cast<const unsigned *>(r1);
+                    v = resize_combine<RGB, 4>(__ldg(w0 + x0), __ldg(w0 + x1), __ldg(w1 + x0), __ldg(w1 + x1), a01, B0, B1);
+                } else {
+                    v = resize_combine<RGB, 4>(rgba_bytes(r0, x0), rgba_bytes(r0, x1), rgba_bytes(r1, x0), rgba_bytes(r1, x1), a01, B0, B1);
+                }
+            }
+            resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
+        }
+        drow += (size_t)dw * 3;
+        if (++dy == (unsigned)dh) { dy = 0; frame += frame_bytes; }
+    }
+}
+
+constexpr bool rs_is_yuv(int fmt) { return fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || fmt == RS_YUV_YUYV; }
+constexpr bool rs_is_bayer(int fmt) { return fmt >= RS_BAYER_RGGB && fmt <= RS_BAYER_BGGR; }
+constexpr bool rs_is_pix_rows(int fmt)          // the formats of resize_pix_rows
+{
+    return fmt == RS_GRAY || fmt == RS_RGB_PLANAR || fmt == RS_RGBA || fmt == RS_BGRA || fmt == RS_RGBA_BYTES || fmt == RS_BGRA_BYTES;
+}
+
 // resident CTAs of 256 threads per SM the launch plans for (= the kernel's __launch_bounds__): 6 at 40 registers; the
 // ragged descriptor bookkeeping needs 48 (5 CTAs) and the 4:2:0 instantiations, which keep luma and chroma row pointers of
 // both source rows, up to 64 (4 CTAs) to run without spills; YUYV fits 40; the Bayer instantiations, which keep a lane's
-// 4x4 grid of raw bytes and four row pointers, need up to 64 (4 CTAs)
+// 4x4 grid of raw bytes and four row pointers, need up to 64 (4 CTAs); gray and the RGBA / BGRA word loads fit 40; RGB
+// (the BGR loop with its word stores), the RGBA / BGRA byte loads and planar RGB need up to 48 (5 CTAs)
 constexpr int resize_ctas_per_sm(bool ragged, int fmt)
 {
-    return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || fmt >= RS_BAYER_RGGB ? 4 : 6;
+    return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || rs_is_bayer(fmt) ? 4
+         : fmt == RS_RGB || fmt == RS_RGB_PLANAR || fmt == RS_RGBA_BYTES || fmt == RS_BGRA_BYTES ? 5 : 6;
 }
 
 // One WARP = a contiguous run of output rows of the batch (so the row bookkeeping is incremental: no divisions), one
@@ -315,8 +409,9 @@ constexpr int resize_ctas_per_sm(bool ragged, int fmt)
 // frames[f] = {byte offset in src, row pitch, geometry g}; its row / column tables are ytab + g * dh / xtab + g * dw.  The
 // descriptor is loaded when dy wraps, so its cost is warp-uniform and paid once per frame.  Otherwise frames are
 // sh x sw and packed at a uniform stride.
-// FMT: the source format, RS_BGR (uint8 [sh][sw][3]), one of the YUV layouts (uniform stride only; resize_yuv_rows) or
-// one of the Bayer patterns (uniform stride only; resize_bayer_rows).
+// FMT: the source format, RS_BGR (uint8 [sh][sw][3]), RS_RGB (the same loop with R and B swapped; uniform stride only),
+// one of the YUV layouts (uniform stride only; resize_yuv_rows), one of the Bayer patterns (uniform stride only;
+// resize_bayer_rows) or gray, RGBA / BGRA (either load variant) and planar RGB (uniform stride only; resize_pix_rows).
 template <bool WORD_STORE, bool RAGGED, int FMT = RS_BGR>
 __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                           const int2 *__restrict__ xtab, const int4 *__restrict__ ytab,
@@ -327,14 +422,20 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
     unsigned row = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * rows_per_warp;
     if (row >= rows) return;
     const unsigned row_end = min(rows, row + rows_per_warp);
-    if constexpr (FMT >= RS_BAYER_RGGB) {
+    if constexpr (rs_is_bayer(FMT)) {
         static_assert(!RAGGED, "Bayer sources are one size per launch");
         resize_bayer_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
         return;
-    } else if constexpr (FMT != RS_BGR) {
+    } else if constexpr (rs_is_pix_rows(FMT)) {
+        static_assert(!RAGGED, "gray, RGBA, BGRA and planar sources are one size per launch");
+        resize_pix_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        return;
+    } else if constexpr (rs_is_yuv(FMT)) {
         static_assert(!RAGGED, "YUV sources are one size per launch");
         resize_yuv_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
         return;
+    } else {
+        static_assert(FMT == RS_BGR || (FMT == RS_RGB && !RAGGED), "the packed 3-byte row loop takes BGR, and RGB at a uniform stride");
     }
     const size_t delta = reinterpret_cast<uintptr_t>(src) & 3;                             // word-aligned view of the source
     const unsigned char *base = src - delta;
@@ -366,10 +467,10 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
         // clamp (in a ragged batch, bytes past a frame's last pixel belong to the next frame and carry zero weight)
         const size_t omax = o0 > o1 ? o0 : o1;
         if (omax + src_row + 12 <= end) {
-            resize_one_row<WORD_STORE, false>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
+            resize_one_row<WORD_STORE, false, FMT == RS_RGB>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
         } else {
             const size_t room0 = end - 1 - (o0 & ~(size_t)3), room1 = end - 1 - (o1 & ~(size_t)3);
-            resize_one_row<WORD_STORE, true>(r0, r1, d0, d1, (unsigned)room0, (unsigned)room1, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
+            resize_one_row<WORD_STORE, true, FMT == RS_RGB>(r0, r1, d0, d1, (unsigned)room0, (unsigned)room1, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
         }
         drow += (size_t)dw * 3;
         if (++dy == (unsigned)dh) {
@@ -406,7 +507,9 @@ size_t camera_frame_bytes(int format, int sh, int sw)
     switch (format) {
     case RS_YUV_NV12: case RS_YUV_I420: return px + px / 2;
     case RS_YUV_YUYV: return 2 * px;
-    case RS_BAYER_RGGB: case RS_BAYER_GRBG: case RS_BAYER_GBRG: case RS_BAYER_BGGR: return px;
+    case RS_BAYER_RGGB: case RS_BAYER_GRBG: case RS_BAYER_GBRG: case RS_BAYER_BGGR: case RS_GRAY: return px;
+    case RS_RGB: case RS_RGB_PLANAR: return 3 * px;
+    case RS_RGBA: case RS_BGRA: return 4 * px;
     default: return 0;
     }
 }
@@ -425,6 +528,17 @@ cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const Res
     case RS_BAYER_GRBG: return resize_launch<false, RS_BAYER_GRBG>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     case RS_BAYER_GBRG: return resize_launch<false, RS_BAYER_GBRG>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     case RS_BAYER_BGGR: return resize_launch<false, RS_BAYER_BGGR>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_RGB:        return resize_launch<false, RS_RGB>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_GRAY:       return resize_launch<false, RS_GRAY>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_RGB_PLANAR: return resize_launch<false, RS_RGB_PLANAR>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    case RS_RGBA: case RS_BGRA: {
+        const bool words = (reinterpret_cast<uintptr_t>(src) & 3) == 0;
+        if (fmt == RS_RGBA)
+            return words ? resize_launch<false, RS_RGBA>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st)
+                         : resize_launch<false, RS_RGBA_BYTES>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+        return words ? resize_launch<false, RS_BGRA>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st)
+                     : resize_launch<false, RS_BGRA_BYTES>(src, src_bytes, nullptr, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
+    }
     default:          return cudaErrorInvalidValue;
     }
 }

@@ -321,6 +321,15 @@ static int host_shr_round(int x, int n, int mode)
     return fl + (fl & 1);
 }
 
+// Host-to-device copy of data that work queued afterwards on the context stream reads (weights, biases, tables): queued on
+// that stream, so it lands before that work starts.  A synchronous cudaMemcpy from pageable memory may return before its
+// DMA has landed, and the context's streams are non-blocking, so they would not be ordered after it.  The source may be
+// reused when this returns (pageable memory is staged before the call returns).
+static cudaError_t upload(yolo_b200_ctx *c, void *dst, const void *src, size_t bytes)
+{
+    return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, c->stream);
+}
+
 // Epilogue programme of layer l from the context's tables (set_quantize_scale, yolo_forward.c:235-254, for contract F;
 // slim_yolo_v2.py:33-38 for contract P) and the pre-shifted biases; uploads the biases.
 static int derive_layer(yolo_b200_ctx *c, int l)
@@ -351,7 +360,7 @@ static int derive_layer(yolo_b200_ctx *c, int l)
     } else return fail(E_ARG, "contract %d", p->contract);
     d.bias_abs_max = 0;
     for (int o = 0; o < L.cout; ++o) d.bias_abs_max = abs(bsh[o]) > d.bias_abs_max ? abs(bsh[o]) : d.bias_abs_max;
-    CU(cudaMemcpy(d.bias_sh, bsh.data(), bsh.size() * sizeof(int), cudaMemcpyHostToDevice));
+    CU(upload(c, d.bias_sh, bsh.data(), bsh.size() * sizeof(int)));
     return 0;
 }
 
@@ -413,18 +422,18 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                     wp[((size_t)o * 9 + (ks == 1 ? 4 : t)) * d.cs_in + i] = w[src];
                 }
         CU(cudaMalloc(&d.w, wp.size()));
-        CU(cudaMemcpy(d.w, wp.data(), wp.size(), cudaMemcpyHostToDevice));
+        CU(upload(c, d.w, wp.data(), wp.size()));
         if (ks == 1) {
             std::vector<int8_t> w1((size_t)d.cout_pad * d.cs_in, 0);
             for (int o = 0; o < d.cout_pad; ++o) memcpy(&w1[(size_t)o * d.cs_in], &wp[((size_t)o * 9 + 4) * d.cs_in], d.cs_in);
             CU(cudaMalloc(&d.w1, w1.size()));
-            CU(cudaMemcpy(d.w1, w1.data(), w1.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.w1, w1.data(), w1.size()));
         }
         if (d.cs_in == 16 && ks == 3) {
             std::vector<int8_t> wk((size_t)d.cout_pad * 160, 0);
             for (int o = 0; o < d.cout_pad; ++o) memcpy(&wk[(size_t)o * 160], &wp[(size_t)o * 144], 144);
             CU(cudaMalloc(&d.w_k160, wk.size()));
-            CU(cudaMemcpy(d.w_k160, wk.data(), wk.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.w_k160, wk.data(), wk.size()));
         }
         if (d.cs_in >= 16 && d.cs_in <= 256 && d.cs_out <= 256 && ks == 3) {
             // conv_ws.cu: B operand as UMMA no-swizzle K-major core matrices, [n/8][kchunk][n%8][16 B].  K chunk order is
@@ -442,7 +451,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                     memcpy(&img[(((size_t)(o / 8) * kc + k) * 8 + (o % 8)) * 16], &wp[((size_t)o * 9 + tap) * d.cs_in + 16 * c], 16);
                 }
             CU(cudaMalloc(&d.wimg, img.size()));
-            CU(cudaMemcpy(d.wimg, img.data(), img.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.wimg, img.data(), img.size()));
             if (d.cs_in == 128 || d.cs_in == 256) {
                 std::vector<uint8_t> imt((size_t)d.cs_out * 9 * d.cs_in, 0);
                 // chunk = (tap, 128-channel plane): [tap][plane][cs_out/8][8 K chunks][8][16 B]
@@ -452,7 +461,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                             memcpy(&imt[(((((size_t)tap * (np / 8) + cc / 8) * (d.cs_out / 8) + o / 8) * 8 + cc % 8) * 8 + (o % 8)) * 16],
                                    &wp[((size_t)o * 9 + tap) * d.cs_in + 16 * cc], 16);
                 CU(cudaMalloc(&d.wimg_tap, imt.size()));
-                CU(cudaMemcpy(d.wimg_tap, imt.data(), imt.size(), cudaMemcpyHostToDevice));
+                CU(upload(c, d.wimg_tap, imt.data(), imt.size()));
                 if (d.cs_out == 256) {
                     // conv_wsp.cu: chunk = (half of the output channels, 128-channel plane, tap): [half][plane][tap][128/8][8 K chunks][8][16 B]
                     std::vector<uint8_t> im2(imt.size(), 0);
@@ -465,7 +474,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                                         memcpy(&im2[((((size_t)(nh * npl + pl) * 9 + tap) * 16 + o / 8) * 8 + cc) * 128 + (size_t)(o % 8) * 16],
                                                &wp[((size_t)(nh * 128 + o) * 9 + tap) * d.cs_in + pl * 128 + 16 * cc], 16);
                     CU(cudaMalloc(&d.wimg_tap2, im2.size()));
-                    CU(cudaMemcpy(d.wimg_tap2, im2.data(), im2.size(), cudaMemcpyHostToDevice));
+                    CU(upload(c, d.wimg_tap2, im2.data(), im2.size()));
                 }
             }
         }
@@ -482,7 +491,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                             memcpy(&img[(((size_t)(n / 8) * 12 + khh * 3 + kw) * 8 + (n % 8)) * 16], &wp[((size_t)o * 9 + kh * 3 + kw) * 16], 16);
                         }
             CU(cudaMalloc(&d.wimg_rp, img.size()));
-            CU(cudaMemcpy(d.wimg_rp, img.data(), img.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.wimg_rp, img.data(), img.size()));
             // x-split variant: chunks 2r, 2r+1 = (input row r, kw 0), (r, kw 2); chunks 8 + r = (r, kw 1)
             std::vector<uint8_t> ims((size_t)64 * 12 * 16, 0);
             for (int dy = 0; dy < 2; ++dy)
@@ -495,7 +504,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                             memcpy(&ims[(((size_t)(n / 8) * 12 + chunk) * 8 + (n % 8)) * 16], &wp[((size_t)o * 9 + kh * 3 + kw) * 16], 16);
                         }
             CU(cudaMalloc(&d.wimg_rps, ims.size()));
-            CU(cudaMemcpy(d.wimg_rps, ims.data(), ims.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.wimg_rps, ims.data(), ims.size()));
         }
         if (ks == 3 && d.cs_in % 128 == 0 && d.cs_out % 256 == 0 && (d.cs_in > 256 || d.cs_out > 256)) {
             // conv_ws3.cu: chunk = (slice of 256 output channels, half of the slice, 128-channel plane, tap): [128/8][8 K chunks][8][16 B]
@@ -510,7 +519,7 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
                                     memcpy(&im3[((((((size_t)(sl * 2 + hf) * npl + pl) * 9 + tap) * 16 + o / 8) * 8 + cc) * 8 + (o % 8)) * 16],
                                            &wp[((size_t)(sl * 256 + hf * 128 + o) * 9 + tap) * d.cs_in + pl * 128 + 16 * cc], 16);
             CU(cudaMalloc(&d.wimg_tap3, im3.size()));
-            CU(cudaMemcpy(d.wimg_tap3, im3.data(), im3.size(), cudaMemcpyHostToDevice));
+            CU(upload(c, d.wimg_tap3, im3.data(), im3.size()));
         }
         // (the 128B-swizzled image of conv_umma.cu is built on first use: ensure_swz)
         CU(cudaMalloc(&d.bias_sh, (size_t)d.cout_pad * sizeof(int)));
@@ -526,9 +535,10 @@ int yolo_b200_load(yolo_b200_ctx *c, const int8_t *const *weights, const int8_t 
     }
     CU(cudaMemset(c->ovf_dev, 0, sizeof(unsigned)));      // the saturation counter belongs to the loaded network
     build_rgb444_lut(p->scale_a[0], c->lut_host);
-    CU(cudaMemcpy(c->lut_dev, c->lut_host, sizeof c->lut_host, cudaMemcpyHostToDevice));
+    CU(upload(c, c->lut_dev, c->lut_host, sizeof c->lut_host));
     c->lut8_saturates = build_u8_lut(p->scale_a[0], c->lut8_host);
-    CU(cudaMemcpy(c->lut8_dev, c->lut8_host, sizeof c->lut8_host, cudaMemcpyHostToDevice));
+    CU(upload(c, c->lut8_dev, c->lut8_host, sizeof c->lut8_host));
+    CU(cudaStreamSynchronize(c->stream));                  // the network is on the device, whichever stream runs next
     c->loaded = true;
     return 0;
 }
@@ -641,13 +651,15 @@ static int ensure_pinned(char **p, size_t *cap, size_t need)
     return 0;
 }
 
-// One camera frame (a YUV layout or a Bayer pattern) of (format, sh, sw): its byte count, or E_ARG / E_UNSUPPORTED
-// (include/yolo_b200.h).  The formats, the sizes each accepts and their frame bytes (camera_frame_bytes) live here.
+// One camera frame (a YUV layout, a Bayer pattern or a pixel format) of (format, sh, sw): its byte count, or E_ARG /
+// E_UNSUPPORTED (include/yolo_b200.h).  The formats, the sizes each accepts and their frame bytes (camera_frame_bytes) live
+// here.  The pixel formats take any size of at least 1x1.
 static int source_check(int format, int sh, int sw, size_t *bytes)
 {
     const bool yuv = format == RS_YUV_NV12 || format == RS_YUV_I420 || format == RS_YUV_YUYV;
     const bool bayer = format >= RS_BAYER_RGGB && format <= RS_BAYER_BGGR;
-    if (!yuv && !bayer) return fail(E_ARG, "unknown camera format %d", format);
+    const bool pix = format >= RS_RGB && format <= RS_RGB_PLANAR;
+    if (!yuv && !bayer && !pix) return fail(E_ARG, "unknown camera format %d", format);
     if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
     if (yuv && (sw % 2 || (format != RS_YUV_YUYV && sh % 2)))
         return fail(E_ARG, "YUV format %d needs an even %s (%dx%d)", format, format == RS_YUV_YUYV ? "width" : "height and width", sh, sw);
@@ -657,9 +669,10 @@ static int source_check(int format, int sh, int sw, size_t *bytes)
     return 0;
 }
 
-// The source format of a YUV entry point's format (the public codes are the internal ones) and of a Bayer entry point's
-// pattern; anything else goes on as an unknown format, which source_check refuses
+// The source format of a YUV entry point's format (the public codes are the internal ones), of a Bayer entry point's
+// pattern and of a pixel-format entry point's format; anything else goes on as an unknown format, which source_check refuses
 static int yuv_format(int format) { return format >= YOLO_B200_YUV_NV12 && format <= YOLO_B200_YUV_YUYV ? format : -1; }
+static int pix_format(int format) { return format >= YOLO_B200_PIX_RGB && format <= YOLO_B200_PIX_RGB_PLANAR ? RS_RGB + format : -1; }
 static int bayer_format(int pattern)
 {
     static const int fmt[4] = { RS_BAYER_RGGB, RS_BAYER_BGGR, RS_BAYER_GRBG, RS_BAYER_GBRG };     // YOLO_B200_BAYER_* order
@@ -671,6 +684,13 @@ int yolo_b200_yuv_frame_bytes(int format, int sh, int sw)
 {
     size_t b = 0;
     int rc = source_check(yuv_format(format), sh, sw, &b); if (rc) return rc;
+    return (int)b;
+}
+
+int yolo_b200_pix_frame_bytes(int format, int sh, int sw)
+{
+    size_t b = 0;
+    int rc = source_check(pix_format(format), sh, sw, &b); if (rc) return rc;
     return (int)b;
 }
 
@@ -830,6 +850,12 @@ int yolo_b200_bayer_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int pa
     return resize_stage(c, bayer_format(pattern), d_src, n, hw, 0, d_dst, dh, dw);
 }
 
+int yolo_b200_pix_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int format, int n, int sh, int sw, uint8_t *d_dst, int dh, int dw)
+{
+    const int32_t hw[2] = { sh, sw };
+    return resize_stage(c, pix_format(format), d_src, n, hw, 0, d_dst, dh, dw);
+}
+
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
 {
     if (!c || !lut_host) return fail(E_ARG, "null argument");
@@ -855,7 +881,7 @@ static int ensure_swz(yolo_b200_ctx *c, LayerDev &d)
     }
     CU(cudaSetDevice(c->device));
     CU(cudaMalloc(&d.w_swz, sw.size()));
-    CU(cudaMemcpy(d.w_swz, sw.data(), sw.size(), cudaMemcpyHostToDevice));
+    CU(upload(c, d.w_swz, sw.data(), sw.size()));
     return 0;
 }
 
@@ -1069,9 +1095,9 @@ enum { TRK_FIRST = 0, TRK_EMA = 1, TRK_MEASURE = 2 };
 static int reprogram_all(yolo_b200_ctx *c)
 {
     build_rgb444_lut(c->prm.scale_a[0], c->lut_host);
-    CU(cudaMemcpy(c->lut_dev, c->lut_host, sizeof c->lut_host, cudaMemcpyHostToDevice));
+    CU(upload(c, c->lut_dev, c->lut_host, sizeof c->lut_host));
     c->lut8_saturates = build_u8_lut(c->prm.scale_a[0], c->lut8_host);
-    CU(cudaMemcpy(c->lut8_dev, c->lut8_host, sizeof c->lut8_host, cudaMemcpyHostToDevice));
+    CU(upload(c, c->lut8_dev, c->lut8_host, sizeof c->lut8_host));
     for (size_t l = 0; l < c->layers.size(); ++l) { int rc = derive_layer(c, (int)l); if (rc) return rc; }
     return 0;
 }
@@ -1101,9 +1127,9 @@ static int tracker_pass_inner(yolo_b200_ctx *c, const float *d_nchw, int n, int 
         if (scales) scales[0] = sc;
         p.scale_a[0] = (int)floorf(log2f(sc));
         build_rgb444_lut(p.scale_a[0], c->lut_host);
-        CU(cudaMemcpy(c->lut_dev, c->lut_host, sizeof c->lut_host, cudaMemcpyHostToDevice));
+        CU(upload(c, c->lut_dev, c->lut_host, sizeof c->lut_host));
         c->lut8_saturates = build_u8_lut(p.scale_a[0], c->lut8_host);
-        CU(cudaMemcpy(c->lut8_dev, c->lut8_host, sizeof c->lut8_host, cudaMemcpyHostToDevice));
+        CU(upload(c, c->lut8_dev, c->lut8_host, sizeof c->lut8_host));
     }
     rc = ensure((void **)&c->in_q, &c->in_q_cap, (size_t)n * h * w * 4); if (rc) return rc;
     rc = yolo_b200_quantize_f32(c, d_nchw, n, h, w, c->in_q); if (rc) return rc;
@@ -1119,7 +1145,7 @@ static int tracker_pass_inner(yolo_b200_ctx *c, const float *d_nchw, int n, int 
         if (la > 6 || lb > 23 || la < 0) return fail(E_UNSUPPORTED, "layer %zu: exponents out of range in the tracker pass (la %d lb %d)", l, la, lb);
         std::vector<int> bp(L.cout_pad, 0);
         for (int o = 0; o < L.cout; ++o) bp[o] = (int)L.bias_host[o] * (1 << lb);
-        CU(cudaMemcpy(L.bias_sh, bp.data(), bp.size() * sizeof(int), cudaMemcpyHostToDevice));
+        CU(upload(c, L.bias_sh, bp.data(), bp.size() * sizeof(int)));
         const int init[2] = { INT32_MIN, INT32_MAX };
         CU(cudaMemcpyAsync(c->stats_dev, init, sizeof init, cudaMemcpyHostToDevice, c->stream));
         ConvArgs a;
@@ -1391,6 +1417,13 @@ int yolo_b200_forward_bayer_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int p
     return forward_resize_dev(c, bayer_format(pattern), d_frames, n, hw, 0, h, w, d_dets, d_counts);
 }
 
+int yolo_b200_forward_pix_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
+                              yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return forward_resize_dev(c, pix_format(format), d_frames, n, hw, 0, h, w, d_dets, d_counts);
+}
+
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 { return forward_dev(c, IN_F32, d_nchw, n, h, w, d_dets, d_counts); }
 
@@ -1633,6 +1666,18 @@ int yolo_b200_submit_bayer(yolo_b200_ctx *c, const uint8_t *frames, int pattern,
 {
     const int32_t hw[2] = { sh, sw };
     return host_resize(c, true, bayer_format(pattern), frames, n, hw, 0, h, w, dets, counts);
+}
+int yolo_b200_forward_pix(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                          yolo_b200_det *dets, int32_t *counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, false, pix_format(format), frames, n, hw, 0, h, w, dets, counts);
+}
+int yolo_b200_submit_pix(yolo_b200_ctx *c, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
+                         yolo_b200_det *dets, int32_t *counts)
+{
+    const int32_t hw[2] = { sh, sw };
+    return host_resize(c, true, pix_format(format), frames, n, hw, 0, h, w, dets, counts);
 }
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------

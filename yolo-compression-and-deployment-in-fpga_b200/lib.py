@@ -23,6 +23,9 @@ HEAD_PYTHON, HEAD_C = 0, 1
 YUV_NV12, YUV_I420, YUV_YUYV = 0, 1, 2      # cv2.COLOR_YUV2BGR_NV12 / _I420 / _YUYV frames (yolo_b200_forward_yuv)
 # Bayer mosaics named by the sensor's top-left 2x2 (yolo_b200_forward_bayer): cv2.COLOR_BayerRGGB2BGR / _BGGR / _GRBG / _GBRG
 BAYER_RGGB, BAYER_BGGR, BAYER_GRBG, BAYER_GBRG = 0, 1, 2, 3
+# pixel formats (yolo_b200_forward_pix): packed R,G,B / R,G,B,A / B,G,R,A, 8-bit gray, and R,G,B planes (torch CHW) =
+# cv2.COLOR_RGB2BGR / _RGBA2BGR / _BGRA2BGR / _GRAY2BGR / RGB2BGR of the HWC transpose
+PIX_RGB, PIX_RGBA, PIX_BGRA, PIX_GRAY, PIX_RGB_PLANAR = 0, 1, 2, 3, 4
 
 EXPORTS = [
     "yolo_b200_abi_version", "yolo_b200_last_error", "yolo_b200_cstride", "yolo_b200_default_params",
@@ -43,6 +46,8 @@ EXPORTS = [
     "yolo_b200_yuv_frame_bytes", "yolo_b200_yuv_to_bgr_resize", "yolo_b200_forward_yuv", "yolo_b200_submit_yuv",
     "yolo_b200_forward_yuv_dev",
     "yolo_b200_bayer_to_bgr_resize", "yolo_b200_forward_bayer", "yolo_b200_submit_bayer", "yolo_b200_forward_bayer_dev",
+    "yolo_b200_pix_frame_bytes", "yolo_b200_pix_to_bgr_resize", "yolo_b200_forward_pix", "yolo_b200_submit_pix",
+    "yolo_b200_forward_pix_dev",
 ]
 
 
@@ -120,6 +125,10 @@ def load_library(path: Optional[str] = None):
         getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.yolo_b200_bayer_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
     for name in ("yolo_b200_forward_bayer", "yolo_b200_submit_bayer", "yolo_b200_forward_bayer_dev"):
+        getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
+    L.yolo_b200_pix_frame_bytes.argtypes = [i32, i32, i32]
+    L.yolo_b200_pix_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
+    for name in ("yolo_b200_forward_pix", "yolo_b200_submit_pix", "yolo_b200_forward_pix_dev"):
         getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.yolo_b200_quantize_rgb444.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_quantize_f32.argtypes = [vp, vp, i32, i32, i32, vp]
@@ -230,6 +239,30 @@ def bayer_source_size(pattern: int, frame_shape) -> "tuple[int, int]":
     if len(fs) != 2 or fs[0] < 3 or fs[1] < 3:
         raise ValueError("%s is not the shape of a Bayer frame [sh][sw] of at least 3x3" % (fs,))
     return fs
+
+
+def pix_frame_shape(fmt: int, sh: int, sw: int) -> "tuple[int, ...]":
+    """The array shape of one frame of pixel format fmt and source size sh x sw: (sh, sw, 3) for PIX_RGB, (sh, sw, 4) for
+    PIX_RGBA / PIX_BGRA, (sh, sw) for PIX_GRAY, (3, sh, sw) for PIX_RGB_PLANAR.  Raises ValueError for an unknown format or
+    a size below 1x1."""
+    if fmt not in (PIX_RGB, PIX_RGBA, PIX_BGRA, PIX_GRAY, PIX_RGB_PLANAR):
+        raise ValueError("unknown pixel format %r" % (fmt,))
+    sh, sw = int(sh), int(sw)
+    if sh < 1 or sw < 1:
+        raise ValueError("pixel format %d cannot hold a %dx%d frame" % (fmt, sh, sw))
+    return {PIX_RGB: (sh, sw, 3), PIX_RGBA: (sh, sw, 4), PIX_BGRA: (sh, sw, 4), PIX_GRAY: (sh, sw), PIX_RGB_PLANAR: (3, sh, sw)}[fmt]
+
+
+def pix_source_size(fmt: int, frame_shape) -> "tuple[int, int]":
+    """(sh, sw) of a frame of pixel format fmt from its array shape (the inverse of pix_frame_shape)."""
+    fs = tuple(int(x) for x in frame_shape)
+    if fmt == PIX_RGB_PLANAR:
+        size = fs[1:] if len(fs) == 3 else None
+    else:
+        size = fs[:2] if len(fs) in (2, 3) else None
+    if size is None or pix_frame_shape(fmt, *size) != fs:
+        raise ValueError("%s is not the shape of a pixel format %r frame" % (fs, fmt))
+    return size
 
 
 class Context:
@@ -414,6 +447,30 @@ class Context:
         return self._submit(self.L.yolo_b200_submit_bayer, _ptr(frames), pattern, n, sh, sw, int(size[0]), int(size[1]),
                             dets.ctypes.data, counts.ctypes.data)
 
+    def forward_pix(self, frames: np.ndarray, fmt: int, size):
+        """uint8 frames [n, *pix_frame_shape(fmt, sh, sw)] (packed RGB / RGBA / BGRA, gray, or planar RGB) ->
+        (dets [n][max_det], counts [n]): cv2.cvtColor to BGR, cv2.resize to size = (h, w) and the rest of
+        forward_u8bgr_resize, all on the GPU; the frames cross the link as they are."""
+        f = np.ascontiguousarray(frames, dtype=np.uint8)
+        sh, sw = pix_source_size(fmt, f.shape[1:])
+        n = f.shape[0]
+        return self._forward_host(self.L.yolo_b200_forward_pix, n, f.ctypes.data, fmt, n, sh, sw, int(size[0]), int(size[1]))
+
+    def submit_pix(self, frames, fmt: int, size, dets: np.ndarray, counts: np.ndarray) -> int:
+        """Queue one batch of frames [n, *pix_frame_shape] (a C-contiguous numpy array or a pinned torch tensor) for
+        size = (h, w); frames, dets [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until
+        wait(ticket).  Returns the ticket."""
+        shape = tuple(frames.shape)
+        sh, sw = pix_source_size(fmt, shape[1:])
+        n = shape[0]
+        if isinstance(frames, np.ndarray):
+            assert frames.dtype == np.uint8 and frames.flags.c_contiguous
+        else:
+            assert str(frames.dtype) == "torch.uint8" and frames.is_contiguous()
+        assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= n and len(counts) >= n
+        return self._submit(self.L.yolo_b200_submit_pix, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
+                            dets.ctypes.data, counts.ctypes.data)
+
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
@@ -468,6 +525,15 @@ class Context:
     def bayer_to_bgr_resize(self, d_src, pattern, n, sh, sw, d_dst, dh, dw):
         """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device Bayer frames into d_dst uint8 [n][dh][dw][3]."""
         self._check(self.L.yolo_b200_bayer_to_bgr_resize(self._h, _ptr(d_src), pattern, n, sh, sw, _ptr(d_dst), dh, dw))
+
+    def forward_pix_dev(self, d_in, fmt, n, sh, sw, h, w, d_dets, d_counts):
+        """n frames of pixel format fmt and source size sh x sw packed in device memory (layout of forward_pix), e.g. a
+        torchvision-decoded uint8 [3][sh][sw] tensor as PIX_RGB_PLANAR."""
+        self._check(self.L.yolo_b200_forward_pix_dev(self._h, _ptr(d_in), fmt, n, sh, sw, h, w, _ptr(d_dets), _ptr(d_counts)))
+
+    def pix_to_bgr_resize(self, d_src, fmt, n, sh, sw, d_dst, dh, dw):
+        """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device frames of pixel format fmt into d_dst uint8 [n][dh][dw][3]."""
+        self._check(self.L.yolo_b200_pix_to_bgr_resize(self._h, _ptr(d_src), fmt, n, sh, sw, _ptr(d_dst), dh, dw))
 
     def resize_u8bgr(self, d_src, n, sh, sw, d_dst, dh, dw):
         """cv2.resize (bilinear) of n uint8 [sh][sw][3] device images into d_dst [n][dh][dw][3]."""
