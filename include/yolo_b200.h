@@ -281,6 +281,48 @@ int yolo_b200_forward_pix(yolo_b200_ctx *ctx, const uint8_t *frames, int format,
 int yolo_b200_submit_pix(yolo_b200_ctx *ctx, const uint8_t *frames, int format, int n, int sh, int sw, int h, int w,
                          yolo_b200_det *dets, int32_t *counts);
 
+/* Frames as decoders, cameras and array libraries lay them out: any of the formats above, one format and one size per
+ * call, at a row pitch, plane offsets and a frame stride of the caller's choosing (NVDEC / PyNvVideoCodec / DALI surfaces,
+ * cv2.cuda.GpuMat, V4L2 and GenICam buffers, FFmpeg AVFrame, strided numpy / torch views, and regions of a larger image).
+ * Row r of plane p of frame i is at frames + i * frame_stride + plane_offset[p] + r * row_pitch[p].  The format decides the
+ * planes and the bytes each row holds:
+ *   BGR, RGB: 1 plane, sh rows of 3*sw     RGBA, BGRA: 1 plane, sh rows of 4*sw     gray, Bayer: 1 plane, sh rows of sw
+ *   YUYV: 1 plane, sh rows of 2*sw          NV12: Y sh rows of sw, interleaved UV sh/2 rows of sw
+ *   I420: Y sh rows of sw, U and V sh/2 rows of sw/2 each                        planar RGB: R, G, B, sh rows of sw each
+ * Entries for planes the format lacks are ignored.  The results equal the family's packed call on the same frames compacted
+ * (yolo_b200_forward_u8bgr_resize and the _yuv, _bayer and _pix entry points), byte for byte; packed frames are the layout
+ * yolo_b200_frames_packed fills in.  Errors (E_ARG, -1): unknown family or format, sizes the format refuses, a negative stride or offset, a pitch
+ * below the bytes of a row, n < 0, null pointers; E_UNSUPPORTED (-3): a frame spanning more than 2 GiB.  Frames may
+ * overlap (frame_stride = 0 repeats one frame): the source is only read.
+ * What a call reads: [frames + first, frames + end) of yolo_b200_frames_span, which the caller keeps addressable; nothing
+ * outside it is read.  Inside it, the 3-byte and RGBA / BGRA word loads may touch padding between rows, but never use
+ * it (weight 0).  RGBA / BGRA take word loads when every
+ * row starts 4-byte aligned (frames + plane_offset[0], the pitch and the stride multiples of 4), bytes otherwise (same
+ * results).  The host calls copy each chunk's span to the GPU as one copy, padding included: a generously padded layout
+ * costs link time. */
+#define YOLO_B200_SRC_BGR    0   /* format ignored: uint8 B,G,R pixels */
+#define YOLO_B200_SRC_YUV    1   /* format = YOLO_B200_YUV_* */
+#define YOLO_B200_SRC_BAYER  2   /* format = YOLO_B200_BAYER_* */
+#define YOLO_B200_SRC_PIX    3   /* format = YOLO_B200_PIX_* */
+typedef struct yolo_b200_frames {
+    int32_t family, format;     /* YOLO_B200_SRC_*, the family's code */
+    int32_t sh, sw;             /* source size in pixels */
+    int64_t frame_stride;       /* bytes from frame i to frame i + 1 (>= 0) */
+    int64_t plane_offset[3];    /* bytes from a frame's start to row 0 of plane p */
+    int64_t row_pitch[3];       /* bytes from row r to row r + 1 of plane p */
+} yolo_b200_frames;
+/* Host only (no GPU needed): *d = the packed layout the family's entry points assume (frame i at i * frame bytes, planes
+ * back to back, rows unpadded). */
+int yolo_b200_frames_packed(yolo_b200_frames *d, int family, int format, int sh, int sw);
+/* Host only: the bytes [frames + *first, frames + *end) a call over n frames of layout *d may read (n == 0: 0, 0). */
+int yolo_b200_frames_span(const yolo_b200_frames *d, int n, int64_t *first, int64_t *end);
+/* yolo_b200_forward_u8bgr_resize / _yuv / _bayer / _pix, and their submit form (+ yolo_b200_wait), on frames laid out as
+ * *d says. */
+int yolo_b200_forward_frames(yolo_b200_ctx *ctx, const uint8_t *frames, const yolo_b200_frames *d, int n, int h, int w,
+                             yolo_b200_det *dets, int32_t *counts);
+int yolo_b200_submit_frames(yolo_b200_ctx *ctx, const uint8_t *frames, const yolo_b200_frames *d, int n, int h, int w,
+                            yolo_b200_det *dets, int32_t *counts);
+
 /* Replaces SlimYOLOv2_quantize_bnfuse.forward(x, quantization=True) inference branch,
  * slim_yolo_v2.py:212-358, for a float NCHW batch (input quantised by a_tracker_in, :218). */
 int yolo_b200_forward_f32(yolo_b200_ctx *ctx, const float *nchw, int n, int h, int w,
@@ -314,6 +356,11 @@ int yolo_b200_forward_bayer_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int
  * uint8 [3][sh][sw] tensors as YOLO_B200_PIX_RGB_PLANAR. */
 int yolo_b200_forward_pix_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, int format, int n, int sh, int sw, int h, int w,
                               yolo_b200_det *d_dets, int32_t *d_counts);
+
+/* Frames at a pitched layout in device memory (layout and errors as yolo_b200_forward_frames): a decoder surface, a
+ * GpuMat or a strided CUDA tensor without a compacting copy. */
+int yolo_b200_forward_frames_dev(yolo_b200_ctx *ctx, const uint8_t *d_frames, const yolo_b200_frames *d, int n, int h, int w,
+                                 yolo_b200_det *d_dets, int32_t *d_counts);
 
 /* Block until everything queued on the context stream is done. */
 int yolo_b200_sync(yolo_b200_ctx *ctx);
@@ -358,6 +405,10 @@ int yolo_b200_bayer_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int 
  * stores). */
 int yolo_b200_pix_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, int format, int n, int sh, int sw,
                                 uint8_t *d_dst, int dh, int dw);
+/* The front end of yolo_b200_forward_frames as a stage: n frames laid out as *d says (device memory) -> uint8 BGR
+ * [n][dh][dw][3], equal to the family's stage on the frames compacted; one kernel launch.  Needs no loaded network. */
+int yolo_b200_frames_to_bgr_resize(yolo_b200_ctx *ctx, const uint8_t *d_src, const yolo_b200_frames *d, int n,
+                                   uint8_t *d_dst, int dh, int dw);
 /* Host only (no GPU needed), for tests: the per-index programme of that resize along one axis, taps[4*d + {0,1,2,3}] =
  * (source index 0, source index 1, weight 0, weight 1), weights in units of 1/2048; horizontal != 0 re-anchors the tap
  * at the image border as OpenCV's horizontal pass does. */

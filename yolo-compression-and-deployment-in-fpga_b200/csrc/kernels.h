@@ -103,17 +103,27 @@ enum { RS_YUV_NV12 = YOLO_B200_YUV_NV12, RS_YUV_I420 = YOLO_B200_YUV_I420, RS_YU
        RS_RGB = 8, RS_RGBA = 9, RS_BGRA = 10, RS_GRAY = 11, RS_RGB_PLANAR = 12 };
 static_assert(RS_RGBA - RS_RGB == YOLO_B200_PIX_RGBA && RS_BGRA - RS_RGB == YOLO_B200_PIX_BGRA && RS_GRAY - RS_RGB == YOLO_B200_PIX_GRAY &&
               RS_RGB_PLANAR - RS_RGB == YOLO_B200_PIX_RGB_PLANAR && YOLO_B200_PIX_RGB == 0, "pixel format codes");
-size_t camera_frame_bytes(int format, int sh, int sw);     // 0 for BGR or an unknown format
+size_t camera_frame_bytes(int format, int sh, int sw);     // packed bytes of one frame (BGR: 3 * sh * sw), 0 for an unknown format
+// The planes of one frame of a format (all formats, BGR included): how many, and per plane its rows and the bytes of
+// each row (include/yolo_b200.h, yolo_b200_frames).  0 for an unknown format.
+int source_planes(int format, int sh, int sw, int rows[3], int row_bytes[3]);
 // Images of different sizes packed back to back in one buffer: frame f starts at byte off of src, its rows are
 // pitch = 3 * sw bytes apart, and its tables are ytab + geom * dh, xtab + geom * dw.
 struct alignas(16) ResizeFrame { unsigned long long off; int pitch; int geom; };
+// Frames of one size at a pitched layout (yolo_b200_frames), relative to src = the first byte any frame's planes hold:
+// row r of plane p of frame f is at src + f * stride + off[p] + r * pitch[p].  A frame spans less than 2 GiB, so
+// off[p] + r * pitch[p] fits 32 bits.
+struct alignas(16) ResizeLayout { unsigned long long stride; unsigned off[3], pitch[3]; };
 // One launch: n frames of format fmt -> uint8 BGR [n][dh][dw][3], bit-exact with cv2.resize (of cv2.cvtColor for the
 // formats other than BGR).
-// frames_dev == nullptr: the frames are sh x sw at a uniform stride from src, with the tables ytab [dh], xtab [dw].
+// frames_dev == nullptr: the frames are sh x sw, with the tables ytab [dh], xtab [dw]; layout_dev == nullptr: packed at a
+// uniform stride from src; otherwise pitched as *layout_dev (device memory) says, and word_pitch says whether its stride
+// and row pitches are multiples of 4 (RGBA / BGRA then take word loads when src is 4-byte aligned).
 // Otherwise (RS_BGR only) frames_dev[f] describes frame f as above.  A BGR or RGB launch reads no byte at or past
-// src + src_bytes; the other formats read only the bytes of their own frames.
+// src + src_bytes; the other formats read only the bytes of their own frames' rows.
 cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
-                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st);
+                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st,
+                        const ResizeLayout *layout_dev = nullptr, bool word_pitch = false);
 
 // head.cu
 struct HeadArgs {

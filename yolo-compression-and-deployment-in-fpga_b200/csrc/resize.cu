@@ -107,7 +107,11 @@ __device__ __forceinline__ void resize_store(unsigned v, bool live, int dx0, int
 
 // One output row of the batch: one thread = one output pixel, a warp = 32 consecutive pixels = 96 contiguous output bytes.
 // RGB: the source pixels are R, G, B (resize_combine).
-template <bool WORD_STORE, bool CLAMP, bool RGB>
+// GROUP_LOADS (the pitched instantiations' unclamped rows): the six words of both source rows are loaded in one asm
+// statement before any is used.  Left to itself, ptxas schedules the pitched loop at its 48-register budget with the second
+// row's loads after the first row's funnel shifts, so every chunk waits for two load latencies in turn (0.234 against
+// 0.205 ms for the same loop in the ragged instantiation).
+template <bool WORD_STORE, bool CLAMP, bool RGB, bool GROUP_LOADS = false>
 __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__ r0, const unsigned char *__restrict__ r1,
                                                unsigned d0, unsigned d1, unsigned lim0, unsigned lim1, unsigned B0, unsigned B1,
                                                const int2 *__restrict__ xtab, uint8_t *__restrict__ drow, int dw,
@@ -120,8 +124,19 @@ __device__ __forceinline__ void resize_one_row(const unsigned char *__restrict__
         if (live) {
             const int2 xt = __ldg(xtab + dx);
             unsigned lo0, hi0, lo1, hi1;
-            resize_row_taps<CLAMP>(r0, (unsigned)xt.x + d0, lim0, lo0, hi0);
-            resize_row_taps<CLAMP>(r1, (unsigned)xt.x + d1, lim1, lo1, hi1);
+            if constexpr (GROUP_LOADS && !CLAMP) {
+                const unsigned off0 = (unsigned)xt.x + d0, off1 = (unsigned)xt.x + d1;
+                const unsigned char *a0 = r0 + (off0 & ~3u), *a1 = r1 + (off1 & ~3u);
+                unsigned w0, w1, w2, w3, w4, w5;
+                asm volatile("ld.global.nc.u32 %0, [%6];\n\tld.global.nc.u32 %1, [%6+4];\n\tld.global.nc.u32 %2, [%6+8];\n\t"
+                             "ld.global.nc.u32 %3, [%7];\n\tld.global.nc.u32 %4, [%7+4];\n\tld.global.nc.u32 %5, [%7+8];"
+                             : "=r"(w0), "=r"(w1), "=r"(w2), "=r"(w3), "=r"(w4), "=r"(w5) : "l"(a0), "l"(a1));
+                lo0 = __funnelshift_r(w0, w1, (off0 & 3u) * 8u); hi0 = __funnelshift_r(w1, w2, (off0 & 3u) * 8u);
+                lo1 = __funnelshift_r(w3, w4, (off1 & 3u) * 8u); hi1 = __funnelshift_r(w4, w5, (off1 & 3u) * 8u);
+            } else {
+                resize_row_taps<CLAMP>(r0, (unsigned)xt.x + d0, lim0, lo0, hi0);
+                resize_row_taps<CLAMP>(r1, (unsigned)xt.x + d1, lim1, lo1, hi1);
+            }
             v = resize_combine<RGB>(lo0, hi0, lo1, hi1, (unsigned)xt.y, B0, B1);
         }
         resize_store<WORD_STORE>(v, live, dx0, dx, dw, drow, lane, p, rsh);
@@ -157,6 +172,18 @@ __device__ __forceinline__ YuvRow yuv_row(const uint8_t *frame, unsigned r, int 
     return { frame + (size_t)r * 2 * sw, nullptr, nullptr };
 }
 
+// The same rows of a pitched frame (ResizeLayout): row r of plane p at frame + off[p] + r * pitch[p]; NV12's plane 1 and
+// I420's planes 1 and 2 are the chroma rows r/2
+template <int FMT>
+__device__ __forceinline__ YuvRow yuv_row_pitched(const uint8_t *frame, unsigned r, const ResizeLayout &L)
+{
+    const unsigned c = r >> 1;
+    const uint8_t *y = frame + (L.off[0] + r * L.pitch[0]);
+    if (FMT == RS_YUV_NV12) return { y, frame + (L.off[1] + c * L.pitch[1]), nullptr };
+    if (FMT == RS_YUV_I420) return { y, frame + (L.off[1] + c * L.pitch[1]), frame + (L.off[2] + c * L.pitch[2]) };
+    return { y, nullptr, nullptr };
+}
+
 // B | G << 8 | R << 16 of source pixel x of the row
 template <int FMT>
 __device__ __forceinline__ unsigned yuv_pixel(const YuvRow &row, unsigned x)
@@ -186,19 +213,26 @@ __device__ __forceinline__ void yuv_row_taps(const YuvRow &row, unsigned x0, uns
 // src + n * frame_bytes.  In the chunked host path that is the end of the chunk's landed bytes.  Loads are bytes (a warp's
 // lanes are ~1.5 luma bytes apart for 640 -> 416, so each byte load touches one or two 128-byte lines), so there is no
 // aligned word that could straddle the end and no clamped-row variant.
-template <bool WORD_STORE, int FMT>
+// LAYOUT: the frames are pitched as *lay says (rows of the same bytes, at other addresses; the bounds argument holds row by
+// row, and nothing is read outside the rows of this launch's frames).
+template <bool WORD_STORE, int FMT, bool LAYOUT>
 __device__ __forceinline__ void resize_yuv_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
-                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane,
+                                                const ResizeLayout *__restrict__ lay)
 {
     const int p = (4 * lane) / 3;
     const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
-    const size_t plane = (size_t)sh * sw, frame_bytes = FMT == RS_YUV_YUYV ? 2 * plane : plane + plane / 2;
+    const size_t plane = (size_t)sh * sw;
+    ResizeLayout L{};
+    if constexpr (LAYOUT) L = *lay;
+    const size_t frame_bytes = LAYOUT ? (size_t)L.stride : FMT == RS_YUV_YUYV ? 2 * plane : plane + plane / 2;
     unsigned dy = row % (unsigned)dh;
     const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
     uint8_t *drow = dst + (size_t)row * dw * 3;
     for (; row < row_end; ++row) {
         const int4 yt = __ldg(ytab + dy);
-        const YuvRow r0 = yuv_row<FMT>(frame, (unsigned)yt.x, sh, sw), r1 = yuv_row<FMT>(frame, (unsigned)yt.y, sh, sw);
+        const YuvRow r0 = LAYOUT ? yuv_row_pitched<FMT>(frame, (unsigned)yt.x, L) : yuv_row<FMT>(frame, (unsigned)yt.x, sh, sw);
+        const YuvRow r1 = LAYOUT ? yuv_row_pitched<FMT>(frame, (unsigned)yt.y, L) : yuv_row<FMT>(frame, (unsigned)yt.y, sh, sw);
         for (int dx0 = 0; dx0 < dw; dx0 += 32) {
             const int dx = dx0 + lane;
             const bool live = dx < dw;
@@ -252,14 +286,18 @@ __device__ __forceinline__ unsigned bayer_site(const unsigned (&v)[4][4], int i0
 // src + n * sh * sw.  In the chunked host path that is the end of the chunk's landed bytes.  Loads are bytes, so there is
 // no aligned word that could straddle the end and no clamped-row variant.
 // The pattern is compile-time (FMT - RS_BAYER_RGGB = column flip | row flip << 1): the site parities fold into constants.
-template <bool WORD_STORE, int FMT>
+// LAYOUT: the frames are pitched as *lay says (the same grid of rows at other addresses).
+template <bool WORD_STORE, int FMT, bool LAYOUT>
 __device__ __forceinline__ void resize_bayer_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
-                                                  const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+                                                  const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane,
+                                                  const ResizeLayout *__restrict__ lay)
 {
     constexpr unsigned PX = (FMT - RS_BAYER_RGGB) & 1, PY = (FMT - RS_BAYER_RGGB) >> 1;
     const int p = (4 * lane) / 3;
     const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
-    const size_t frame_bytes = (size_t)sh * sw;
+    ResizeLayout L{};
+    if constexpr (LAYOUT) L = *lay;
+    const size_t frame_bytes = LAYOUT ? (size_t)L.stride : (size_t)sh * sw;
     const unsigned ymax = (unsigned)sh - 2u, xmax = (unsigned)sw - 2u;
     unsigned dy = row % (unsigned)dh;
     const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
@@ -268,8 +306,13 @@ __device__ __forceinline__ void resize_bayer_rows(const uint8_t *__restrict__ sr
         const int4 yt = __ldg(ytab + dy);
         const unsigned y0 = min(max((unsigned)yt.x, 1u), ymax), y1 = min(max((unsigned)yt.y, 1u), ymax);
         const uint8_t *rows[4];                                      // warp-uniform
-        rows[0] = frame + (size_t)(y0 - 1u) * sw; rows[1] = rows[0] + sw; rows[2] = rows[1] + sw;
-        rows[3] = frame + (size_t)(y1 + 1u) * sw;
+        if constexpr (LAYOUT) {
+            rows[0] = frame + (L.off[0] + (y0 - 1u) * L.pitch[0]); rows[1] = rows[0] + L.pitch[0]; rows[2] = rows[1] + L.pitch[0];
+            rows[3] = frame + (L.off[0] + (y1 + 1u) * L.pitch[0]);
+        } else {
+            rows[0] = frame + (size_t)(y0 - 1u) * sw; rows[1] = rows[0] + sw; rows[2] = rows[1] + sw;
+            rows[3] = frame + (size_t)(y1 + 1u) * sw;
+        }
         const bool ystep = y1 != y0;
         const unsigned yo = (y0 ^ PY) & 1u;
         for (int dx0 = 0; dx0 < dw; dx0 += 32) {
@@ -333,9 +376,12 @@ __device__ __forceinline__ unsigned rgba_bytes(const uint8_t *row, unsigned x)
 // clamped successor, so every byte read (a word: the pixel's own four bytes) lies inside its own frame, and frames are
 // those of this launch: nothing is read before src or at or past src + n * frame_bytes.  In the chunked host path that is
 // the end of the chunk's landed bytes.  So there is no clamped-row variant.
-template <bool WORD_STORE, int FMT>
+// LAYOUT: the frames are pitched as *lay says; planar RGB then reads plane p's rows at off[p] + r * pitch[p], the others
+// plane 0's.  The RGBA / BGRA word loads need every row 4-byte aligned: src, the stride and the pitch multiples of 4.
+template <bool WORD_STORE, int FMT, bool LAYOUT>
 __device__ __forceinline__ void resize_pix_rows(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, const int2 *__restrict__ xtab,
-                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane)
+                                                const int4 *__restrict__ ytab, unsigned row, unsigned row_end, int sh, int sw, int dh, int dw, int lane,
+                                                const ResizeLayout *__restrict__ lay)
 {
     constexpr bool GRAY = FMT == RS_GRAY, PLANAR = FMT == RS_RGB_PLANAR;
     constexpr bool WORDS = FMT == RS_RGBA || FMT == RS_BGRA, RGB = FMT == RS_RGBA || FMT == RS_RGBA_BYTES;
@@ -343,13 +389,21 @@ __device__ __forceinline__ void resize_pix_rows(const uint8_t *__restrict__ src,
     constexpr unsigned ROW = PLANAR ? 1 : BPP;                    // row bytes per pixel (of one plane)
     const int p = (4 * lane) / 3;
     const unsigned rsh = 8u * (unsigned)(4 * lane - 3 * p);
-    const size_t plane = (size_t)sh * sw, frame_bytes = BPP * plane;
+    const size_t plane = (size_t)sh * sw;
+    ResizeLayout L{};
+    if constexpr (LAYOUT) L = *lay;
+    const size_t frame_bytes = LAYOUT ? (size_t)L.stride : BPP * plane;
     unsigned dy = row % (unsigned)dh;
     const uint8_t *frame = src + (size_t)(row / (unsigned)dh) * frame_bytes;
     uint8_t *drow = dst + (size_t)row * dw * 3;
     for (; row < row_end; ++row) {
         const int4 yt = __ldg(ytab + dy);
-        const uint8_t *r0 = frame + (size_t)yt.x * sw * ROW, *r1 = frame + (size_t)yt.y * sw * ROW;   // warp-uniform
+        const uint8_t *r0, *r1;                                      // warp-uniform
+        if constexpr (LAYOUT) {
+            r0 = frame + (L.off[0] + (unsigned)yt.x * L.pitch[0]); r1 = frame + (L.off[0] + (unsigned)yt.y * L.pitch[0]);
+        } else {
+            r0 = frame + (size_t)yt.x * sw * ROW; r1 = frame + (size_t)yt.y * sw * ROW;
+        }
         for (int dx0 = 0; dx0 < dw; dx0 += 32) {
             const int dx = dx0 + lane;
             const bool live = dx < dw;
@@ -365,6 +419,10 @@ __device__ __forceinline__ void resize_pix_rows(const uint8_t *__restrict__ src,
 #pragma unroll
                     for (int ch = 0; ch < 3; ++ch) {                  // output B, G, R = planes 2, 1, 0
                         const uint8_t *q0 = r0 + (2 - ch) * plane, *q1 = r1 + (2 - ch) * plane;
+                        if constexpr (LAYOUT) {
+                            q0 = frame + (L.off[2 - ch] + (unsigned)yt.x * L.pitch[2 - ch]);
+                            q1 = frame + (L.off[2 - ch] + (unsigned)yt.y * L.pitch[2 - ch]);
+                        }
                         v |= resize_channel(__ldg(q0 + x0) | ((unsigned)__ldg(q0 + x1) << 8),
                                             __ldg(q1 + x0) | ((unsigned)__ldg(q1 + x1) << 8), a01, B0, B1) << (8 * ch);
                     }
@@ -394,8 +452,12 @@ constexpr bool rs_is_pix_rows(int fmt)          // the formats of resize_pix_row
 // both source rows, up to 64 (4 CTAs) to run without spills; YUYV fits 40; the Bayer instantiations, which keep a lane's
 // 4x4 grid of raw bytes and four row pointers, need up to 64 (4 CTAs); gray and the RGBA / BGRA word loads fit 40; RGB
 // (the BGR loop with its word stores), the RGBA / BGRA byte loads and planar RGB need up to 48 (5 CTAs)
-constexpr int resize_ctas_per_sm(bool ragged, int fmt)
+// The pitched (LAYOUT) instantiations keep a frame stride and plane offsets / pitches besides: gray still fits 40, the
+// packed 3-byte loops, YUYV and RGBA / BGRA (both load variants) need up to 48 (5 CTAs), 4:2:0, Bayer and planar RGB up to
+// 64 (4 CTAs) to run without spills
+constexpr int resize_ctas_per_sm(bool ragged, int fmt, bool layout = false)
 {
+    if (layout) return fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || rs_is_bayer(fmt) || fmt == RS_RGB_PLANAR ? 4 : fmt == RS_GRAY ? 6 : 5;
     return ragged ? 5 : fmt == RS_YUV_NV12 || fmt == RS_YUV_I420 || rs_is_bayer(fmt) ? 4
          : fmt == RS_RGB || fmt == RS_RGB_PLANAR || fmt == RS_RGBA_BYTES || fmt == RS_BGRA_BYTES ? 5 : 6;
 }
@@ -412,8 +474,15 @@ constexpr int resize_ctas_per_sm(bool ragged, int fmt)
 // FMT: the source format, RS_BGR (uint8 [sh][sw][3]), RS_RGB (the same loop with R and B swapped; uniform stride only),
 // one of the YUV layouts (uniform stride only; resize_yuv_rows), one of the Bayer patterns (uniform stride only;
 // resize_bayer_rows) or gray, RGBA / BGRA (either load variant) and planar RGB (uniform stride only; resize_pix_rows).
-template <bool WORD_STORE, bool RAGGED, int FMT = RS_BGR>
-__global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+// LAYOUT (not RAGGED): the frames are sh x sw at the pitched layout `frames` points to (a ResizeLayout: no new kernel
+// argument), src = the first byte of frame 0's planes and src_bytes the bytes from there to the end of the launch's last
+// row.  The packed 3-byte loop then takes its frame stride and row pitch from the record, and the rule "rows whose
+// window could reach past the end" holds as it is: a window reaches at most 11 bytes past its pixel, so less than
+// pitch + 12 past its row's start, whatever the pitch.  Bytes between rows (padding) are read only as tap 1 of a
+// right-border pixel or the slack of a word, both with weight 0; rows that start in the first word of the buffer take the
+// clamped byte loads too, so nothing before src is read.
+template <bool WORD_STORE, bool RAGGED, int FMT = RS_BGR, bool LAYOUT = false>
+__global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT, LAYOUT)) resize_u8c3_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                           const int2 *__restrict__ xtab, const int4 *__restrict__ ytab,
                                                           const ResizeFrame *__restrict__ frames,
                                                           unsigned rows, unsigned rows_per_warp, int sh, int sw, int dh, int dw, size_t src_bytes)
@@ -422,17 +491,19 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
     unsigned row = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * rows_per_warp;
     if (row >= rows) return;
     const unsigned row_end = min(rows, row + rows_per_warp);
+    static_assert(!(RAGGED && LAYOUT), "a pitched launch is one size");
+    const ResizeLayout *lay = reinterpret_cast<const ResizeLayout *>(frames);
     if constexpr (rs_is_bayer(FMT)) {
         static_assert(!RAGGED, "Bayer sources are one size per launch");
-        resize_bayer_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        resize_bayer_rows<WORD_STORE, FMT, LAYOUT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane, lay);
         return;
     } else if constexpr (rs_is_pix_rows(FMT)) {
         static_assert(!RAGGED, "gray, RGBA, BGRA and planar sources are one size per launch");
-        resize_pix_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        resize_pix_rows<WORD_STORE, FMT, LAYOUT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane, lay);
         return;
     } else if constexpr (rs_is_yuv(FMT)) {
         static_assert(!RAGGED, "YUV sources are one size per launch");
-        resize_yuv_rows<WORD_STORE, FMT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane);
+        resize_yuv_rows<WORD_STORE, FMT, LAYOUT>(src, dst, xtab, ytab, row, row_end, sh, sw, dh, dw, lane, lay);
         return;
     } else {
         static_assert(FMT == RS_BGR || (FMT == RS_RGB && !RAGGED), "the packed 3-byte row loop takes BGR, and RGB at a uniform stride");
@@ -453,6 +524,9 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
     };
     if constexpr (RAGGED) {
         load_frame(f);
+    } else if constexpr (LAYOUT) {
+        src_frame = lay->stride; src_row = lay->pitch[0];
+        frame_off = delta + lay->off[0] + (size_t)f * src_frame;
     } else {
         src_frame = (size_t)sh * sw * 3; src_row = (size_t)sw * 3;
         frame_off = delta + (size_t)f * src_frame;
@@ -465,9 +539,11 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
         const unsigned d0 = (unsigned)o0 & 3u, d1 = (unsigned)o1 & 3u;
         // a window reaches at most 11 bytes past the start of its pixel; rows for which that stays inside the buffer need no
         // clamp (in a ragged batch, bytes past a frame's last pixel belong to the next frame and carry zero weight)
+        // LAYOUT: nor the rows that start in the buffer's first word (o0 < 4, o0 <= o1), whose first aligned word would
+        // hold bytes before src: src is the first byte of the span, and a pitched call reads nothing outside its span
         const size_t omax = o0 > o1 ? o0 : o1;
-        if (omax + src_row + 12 <= end) {
-            resize_one_row<WORD_STORE, false, FMT == RS_RGB>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
+        if (omax + src_row + 12 <= end && (!LAYOUT || o0 >= 4)) {
+            resize_one_row<WORD_STORE, false, FMT == RS_RGB, LAYOUT>(r0, r1, d0, d1, 0u, 0u, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
         } else {
             const size_t room0 = end - 1 - (o0 & ~(size_t)3), room1 = end - 1 - (o1 & ~(size_t)3);
             resize_one_row<WORD_STORE, true, FMT == RS_RGB>(r0, r1, d0, d1, (unsigned)room0, (unsigned)room1, (unsigned)yt.z, (unsigned)yt.w, RAGGED ? xtab + geom * (unsigned)dw : xtab, drow, dw, lane, 0, 1, p, rsh);
@@ -482,7 +558,7 @@ __global__ void __launch_bounds__(256, resize_ctas_per_sm(RAGGED, FMT)) resize_u
 }
 
 // one wave of resident CTAs (8 warps each), equal runs of rows per warp
-template <bool RAGGED, int FMT = RS_BGR>
+template <bool RAGGED, int FMT = RS_BGR, bool LAYOUT = false>
 static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const ResizeFrame *frames, int n, int sh, int sw, uint8_t *dst,
                                  int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
 {
@@ -490,14 +566,14 @@ static cudaError_t resize_launch(const uint8_t *src, size_t src_bytes, const Res
     const size_t rows = (size_t)n * dh;
     if (rows > 0x7fffffffull) return cudaErrorInvalidValue;
     const int threads = 256;
-    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * resize_ctas_per_sm(RAGGED, FMT) * (threads / 32);
+    const size_t max_warps = (size_t)(sm_count > 0 ? sm_count : 148) * resize_ctas_per_sm(RAGGED, FMT, LAYOUT) * (threads / 32);
     const unsigned rows_per_warp = (unsigned)((rows + max_warps - 1) / max_warps);
     const size_t warps = (rows + rows_per_warp - 1) / rows_per_warp;
     const size_t blocks = (warps + threads / 32 - 1) / (threads / 32);
     if ((reinterpret_cast<uintptr_t>(dst) & 3) == 0 && dw % 4 == 0)
-        resize_u8c3_kernel<true, RAGGED, FMT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+        resize_u8c3_kernel<true, RAGGED, FMT, LAYOUT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
     else
-        resize_u8c3_kernel<false, RAGGED, FMT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
+        resize_u8c3_kernel<false, RAGGED, FMT, LAYOUT><<<(unsigned)blocks, threads, 0, st>>>(src, dst, xtab_dev, ytab_dev, frames, (unsigned)rows, rows_per_warp, sh, sw, dh, dw, src_bytes);
     return cudaGetLastError();
 }
 
@@ -508,15 +584,62 @@ size_t camera_frame_bytes(int format, int sh, int sw)
     case RS_YUV_NV12: case RS_YUV_I420: return px + px / 2;
     case RS_YUV_YUYV: return 2 * px;
     case RS_BAYER_RGGB: case RS_BAYER_GRBG: case RS_BAYER_GBRG: case RS_BAYER_BGGR: case RS_GRAY: return px;
-    case RS_RGB: case RS_RGB_PLANAR: return 3 * px;
+    case RS_BGR: case RS_RGB: case RS_RGB_PLANAR: return 3 * px;
     case RS_RGBA: case RS_BGRA: return 4 * px;
     default: return 0;
     }
 }
 
-cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
-                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+int source_planes(int format, int sh, int sw, int rows[3], int row_bytes[3])
 {
+    auto set = [&](int p, int r, int b) { rows[p] = r; row_bytes[p] = b; };
+    switch (format) {
+    case RS_YUV_NV12: set(0, sh, sw); set(1, sh / 2, sw); return 2;
+    case RS_YUV_I420: set(0, sh, sw); set(1, sh / 2, sw / 2); set(2, sh / 2, sw / 2); return 3;
+    case RS_YUV_YUYV: set(0, sh, 2 * sw); return 1;
+    case RS_BAYER_RGGB: case RS_BAYER_GRBG: case RS_BAYER_GBRG: case RS_BAYER_BGGR: case RS_GRAY: set(0, sh, sw); return 1;
+    case RS_BGR: case RS_RGB: set(0, sh, 3 * sw); return 1;
+    case RS_RGBA: case RS_BGRA: set(0, sh, 4 * sw); return 1;
+    case RS_RGB_PLANAR: set(0, sh, sw); set(1, sh, sw); set(2, sh, sw); return 3;
+    default: return 0;
+    }
+}
+
+// The launches of the pitched layout: the uniform dispatch below with LAYOUT set and the record as `frames`
+static cudaError_t resize_u8c3_pitched(const uint8_t *src, size_t src_bytes, int fmt, const ResizeLayout *lay, bool word_pitch, int n, int sh, int sw,
+                                       uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st)
+{
+    const ResizeFrame *f = reinterpret_cast<const ResizeFrame *>(lay);
+#define RS_PITCHED(F) resize_launch<false, F, true>(src, src_bytes, f, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st)
+    switch (fmt) {
+    case RS_BGR:        return RS_PITCHED(RS_BGR);
+    case RS_YUV_NV12:   return RS_PITCHED(RS_YUV_NV12);
+    case RS_YUV_I420:   return RS_PITCHED(RS_YUV_I420);
+    case RS_YUV_YUYV:   return RS_PITCHED(RS_YUV_YUYV);
+    case RS_BAYER_RGGB: return RS_PITCHED(RS_BAYER_RGGB);
+    case RS_BAYER_GRBG: return RS_PITCHED(RS_BAYER_GRBG);
+    case RS_BAYER_GBRG: return RS_PITCHED(RS_BAYER_GBRG);
+    case RS_BAYER_BGGR: return RS_PITCHED(RS_BAYER_BGGR);
+    case RS_RGB:        return RS_PITCHED(RS_RGB);
+    case RS_GRAY:       return RS_PITCHED(RS_GRAY);
+    case RS_RGB_PLANAR: return RS_PITCHED(RS_RGB_PLANAR);
+    case RS_RGBA: case RS_BGRA: {
+        const bool words = word_pitch && (reinterpret_cast<uintptr_t>(src) & 3) == 0;     // every row 4-byte aligned
+        if (fmt == RS_RGBA) return words ? RS_PITCHED(RS_RGBA) : RS_PITCHED(RS_RGBA_BYTES);
+        return words ? RS_PITCHED(RS_BGRA) : RS_PITCHED(RS_BGRA_BYTES);
+    }
+    default:            return cudaErrorInvalidValue;
+    }
+#undef RS_PITCHED
+}
+
+cudaError_t resize_u8c3(const uint8_t *src, size_t src_bytes, int fmt, const ResizeFrame *frames_dev, int n, int sh, int sw,
+                        uint8_t *dst, int dh, int dw, const int2 *xtab_dev, const int4 *ytab_dev, int sm_count, cudaStream_t st,
+                        const ResizeLayout *layout_dev, bool word_pitch)
+{
+    if (layout_dev)
+        return frames_dev ? cudaErrorInvalidValue
+                          : resize_u8c3_pitched(src, src_bytes, fmt, layout_dev, word_pitch, n, sh, sw, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st);
     if (frames_dev)
         return fmt == RS_BGR ? resize_launch<true>(src, src_bytes, frames_dev, n, 0, 0, dst, dh, dw, xtab_dev, ytab_dev, sm_count, st) : cudaErrorInvalidValue;
     switch (fmt) {

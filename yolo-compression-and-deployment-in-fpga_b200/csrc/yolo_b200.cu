@@ -9,6 +9,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <map>
 #include <mutex>
 #include <vector>
@@ -79,7 +80,7 @@ struct ResizeTables {
     char *host[2] = {nullptr, nullptr}; size_t host_cap[2] = {0, 0};
     cudaEvent_t ev[2] = {nullptr, nullptr};                 // recorded after the copy out of host[k]
     int next = 0;
-    int key[4] = {0, 0, 0, 0};                              // the context's uniform cache: (sh, sw, dh, dw) of its tables
+    long long key[10] = {};                                 // the context's uniform cache: (sh, sw, dh, dw) and the layout of its tables
     const ResizeFrame *frames = nullptr; const int4 *ytab = nullptr; const int2 *xtab = nullptr;     // inside dev
 };
 
@@ -651,15 +652,15 @@ static int ensure_pinned(char **p, size_t *cap, size_t need)
     return 0;
 }
 
-// One camera frame (a YUV layout, a Bayer pattern or a pixel format) of (format, sh, sw): its byte count, or E_ARG /
+// One frame (BGR, a YUV layout, a Bayer pattern or a pixel format) of (format, sh, sw): its packed byte count, or E_ARG /
 // E_UNSUPPORTED (include/yolo_b200.h).  The formats, the sizes each accepts and their frame bytes (camera_frame_bytes) live
-// here.  The pixel formats take any size of at least 1x1.
+// here, and so does the check of a pitched layout (layout_check).  BGR and the pixel formats take any size of at least 1x1.
 static int source_check(int format, int sh, int sw, size_t *bytes)
 {
     const bool yuv = format == RS_YUV_NV12 || format == RS_YUV_I420 || format == RS_YUV_YUYV;
     const bool bayer = format >= RS_BAYER_RGGB && format <= RS_BAYER_BGGR;
     const bool pix = format >= RS_RGB && format <= RS_RGB_PLANAR;
-    if (!yuv && !bayer && !pix) return fail(E_ARG, "unknown camera format %d", format);
+    if (!yuv && !bayer && !pix && format != RS_BGR) return fail(E_ARG, "unknown source format %d", format);
     if (sh < 1 || sw < 1) return fail(E_ARG, "bad source shape %dx%d", sh, sw);
     if (yuv && (sw % 2 || (format != RS_YUV_YUYV && sh % 2)))
         return fail(E_ARG, "YUV format %d needs an even %s (%dx%d)", format, format == RS_YUV_YUYV ? "width" : "height and width", sh, sw);
@@ -678,6 +679,81 @@ static int bayer_format(int pattern)
     static const int fmt[4] = { RS_BAYER_RGGB, RS_BAYER_BGGR, RS_BAYER_GRBG, RS_BAYER_GBRG };     // YOLO_B200_BAYER_* order
     static_assert(YOLO_B200_BAYER_RGGB == 0 && YOLO_B200_BAYER_BGGR == 1 && YOLO_B200_BAYER_GRBG == 2 && YOLO_B200_BAYER_GBRG == 3, "pattern codes");
     return pattern >= 0 && pattern < 4 ? fmt[pattern] : -1;
+}
+// The source format of a frames descriptor's (family, format)
+static int family_format(int family, int format)
+{
+    switch (family) {
+    case YOLO_B200_SRC_BGR:   return RS_BGR;
+    case YOLO_B200_SRC_YUV:   return yuv_format(format);
+    case YOLO_B200_SRC_BAYER: return bayer_format(format);
+    case YOLO_B200_SRC_PIX:   return pix_format(format);
+    default:                  return -1;
+    }
+}
+
+// A pitched layout of frames of (format, sh, sw), already checked by source_check: where one frame's planes start
+// relative to the frame and how far they reach.  Every plane the format has needs offset >= 0 and a pitch of at least its
+// row bytes (E_ARG; planes it lacks are ignored), the stride >= 0 (E_ARG; frames may overlap, the source is read only);
+// a frame spanning more than 2 GiB is E_UNSUPPORTED.  *first / *end: the frame's span [first, end) from its start.
+static int layout_check(int format, const yolo_b200_frames &d, int64_t *first, int64_t *end, ResizeLayout *lay)
+{
+    int rows[3], row_bytes[3];
+    const int planes = source_planes(format, d.sh, d.sw, rows, row_bytes);
+    if (d.frame_stride < 0) return fail(E_ARG, "negative frame stride %lld", (long long)d.frame_stride);
+    constexpr int64_t FAR = (int64_t)1 << 62;                       // keeps the sums below exact; nothing real is so far
+    int64_t lo = INT64_MAX, hi = 0;
+    for (int p = 0; p < planes; ++p) {
+        const int64_t off = d.plane_offset[p], pitch = d.row_pitch[p];
+        if (off < 0) return fail(E_ARG, "plane %d: negative offset %lld", p, (long long)off);
+        if (pitch < row_bytes[p]) return fail(E_ARG, "plane %d: row pitch %lld below the %d bytes of a row", p, (long long)pitch, row_bytes[p]);
+        if (off > FAR || d.frame_stride > FAR || (rows[p] > 1 && pitch > INT32_MAX))
+            return fail(E_UNSUPPORTED, "plane %d: a frame larger than 2 GiB", p);
+        lo = std::min(lo, off);
+        hi = std::max(hi, off + (int64_t)(rows[p] - 1) * pitch + row_bytes[p]);
+    }
+    if (hi - lo > INT32_MAX) return fail(E_UNSUPPORTED, "a frame spans %lld bytes, more than 2 GiB", (long long)(hi - lo));
+    *first = lo; *end = hi;
+    if (lay) {
+        *lay = ResizeLayout{};
+        lay->stride = (unsigned long long)d.frame_stride;
+        for (int p = 0; p < planes; ++p) {
+            lay->off[p] = (unsigned)(d.plane_offset[p] - lo);
+            lay->pitch[p] = rows[p] > 1 ? (unsigned)d.row_pitch[p] : (unsigned)row_bytes[p];     // one row: its pitch is never used
+        }
+    }
+    return 0;
+}
+
+int yolo_b200_frames_packed(yolo_b200_frames *d, int family, int format, int sh, int sw)
+{
+    if (!d) return fail(E_ARG, "null descriptor");
+    const int fmt = family_format(family, format);
+    size_t bytes = 0;
+    int rc = source_check(fmt, sh, sw, &bytes); if (rc) return rc;
+    int rows[3], row_bytes[3];
+    const int planes = source_planes(fmt, sh, sw, rows, row_bytes);
+    yolo_b200_frames f{};
+    f.family = family; f.format = family == YOLO_B200_SRC_BGR ? 0 : format; f.sh = sh; f.sw = sw;
+    f.frame_stride = (int64_t)bytes;
+    for (int p = 0, off = 0; p < planes; off += rows[p] * row_bytes[p], ++p) { f.plane_offset[p] = off; f.row_pitch[p] = row_bytes[p]; }
+    *d = f;
+    return 0;
+}
+
+int yolo_b200_frames_span(const yolo_b200_frames *d, int n, int64_t *first, int64_t *end)
+{
+    if (!d || !first || !end) return fail(E_ARG, "null argument");
+    if (n < 0) return fail(E_ARG, "n %d", n);
+    const int fmt = family_format(d->family, d->format);
+    size_t bytes = 0;
+    int rc = source_check(fmt, d->sh, d->sw, &bytes); if (rc) return rc;
+    int64_t lo = 0, hi = 0;
+    rc = layout_check(fmt, *d, &lo, &hi, nullptr); if (rc) return rc;
+    if (n == 0) { *first = *end = 0; return 0; }
+    if (n > 1 && d->frame_stride > (INT64_MAX - hi) / (n - 1)) return fail(E_UNSUPPORTED, "the frames span more than 2^63 bytes");
+    *first = lo; *end = (int64_t)(n - 1) * d->frame_stride + hi;
+    return 0;
 }
 
 int yolo_b200_yuv_frame_bytes(int format, int sh, int sw)
@@ -699,27 +775,38 @@ enum { RESIZE_NONE, RESIZE_UNIFORM, RESIZE_RAGGED };
 struct SourcePlan {
     InKind kind = IN_BGR;                            // what the frames are once resized
     int fmt = RS_BGR, n = 0, dh = 0, dw = 0, mode = RESIZE_NONE;
-    size_t frame_bytes = 0;                          // one source size: bytes per frame
+    size_t frame_bytes = 0;                          // one source size: bytes per frame (pitched: the frame stride)
     std::vector<size_t> off;                         // RESIZE_RAGGED: [n + 1] byte offset of frame f; off[n] = total
     std::vector<ResizeFrame> frames;                 // RESIZE_RAGGED: what the kernel reads per frame
     std::vector<std::pair<int, int>> geoms;          // distinct source sizes in order of first appearance
+    bool pitched = false;                            // a yolo_b200_frames layout (uniform): lay, and a frame's span
+    ResizeLayout lay{};                              // [first, last) from its start
+    size_t first = 0, last = 0;
     size_t at(int f) const { return off.empty() ? (size_t)f * frame_bytes : off[f]; }     // byte offset of frame f
+    size_t begin(int f) const { return at(f) + first; }                                  // first byte frames f.. read
+    size_t end(int f0, int nf) const { return pitched ? at(f0 + nf - 1) + last : at(f0 + nf); }   // one past frames [f0, f0 + nf)
 };
 
 // The plan of n frames of format fmt (RS_BGR or a camera format) for the network size dh x dw.  Frame i has the source size
 // src_hw[2 * i * stride] x src_hw[2 * i * stride + 1] (stride 0: one size for all, checked also when n == 0).  One rule
 // picks the resize: none for a forward call whose only source size is dh x dw in BGR (the frames are the network input
 // as they are), uniform for one source size or any camera-format call, ragged for several source sizes.
-static int plan_sources(int fmt, int n, const int32_t *src_hw, int stride, int dh, int dw, bool forward, SourcePlan &p)
+// layout (one size, src_hw = its size): the frames are pitched as it says, and are resized even at the network size.
+static int plan_sources(int fmt, int n, const int32_t *src_hw, int stride, int dh, int dw, bool forward, SourcePlan &p,
+                        const yolo_b200_frames *layout = nullptr)
 {
     p = SourcePlan();
     p.fmt = fmt; p.n = n; p.dh = dh; p.dw = dw;
     const int m = stride ? n : 1;                                // sizes to read
     if (m > 0 && !src_hw) return fail(E_ARG, "null src_hw");
-    if (fmt != RS_BGR) {
+    if (fmt != RS_BGR || layout) {
         int rc = source_check(fmt, src_hw[0], src_hw[1], &p.frame_bytes); if (rc) return rc;
         p.geoms.push_back({src_hw[0], src_hw[1]});
         p.mode = RESIZE_UNIFORM;
+        if (!layout) return 0;
+        int64_t first = 0, last = 0;
+        rc = layout_check(fmt, *layout, &first, &last, &p.lay); if (rc) return rc;
+        p.pitched = true; p.frame_bytes = (size_t)layout->frame_stride; p.first = (size_t)first; p.last = (size_t)last;
         return 0;
     }
     p.off.assign((size_t)(m > 0 ? m : 0) + 1, 0);
@@ -776,13 +863,18 @@ static int resize_tables(yolo_b200_ctx *c, const SourcePlan &p, ResizeTables &ca
     const bool ragged = p.mode == RESIZE_RAGGED;
     ResizeTables &t = ragged ? call : c->rs_cache;
     *out = &t;
-    const int key[4] = { p.geoms[0].first, p.geoms[0].second, p.dh, p.dw };
+    // a pitched plan's layout record leads the image (the kernel reads it through `frames`) and is part of the key
+    const long long key[10] = { p.geoms[0].first, p.geoms[0].second, p.dh, p.dw, p.pitched, (long long)p.lay.stride,
+                                p.lay.off[0] | (long long)p.lay.pitch[0] << 32, p.lay.off[1] | (long long)p.lay.pitch[1] << 32,
+                                p.lay.off[2] | (long long)p.lay.pitch[2] << 32, 0 };
     if (!ragged && !memcmp(t.key, key, sizeof key)) return 0;
-    const size_t G = p.geoms.size(), ytab_off = p.frames.size() * sizeof(ResizeFrame), xtab_off = ytab_off + G * p.dh * sizeof(int4);
+    const size_t G = p.geoms.size(), head = p.pitched ? sizeof(ResizeLayout) : p.frames.size() * sizeof(ResizeFrame);
+    const size_t ytab_off = head, xtab_off = ytab_off + G * p.dh * sizeof(int4);
     const size_t bytes = xtab_off + G * p.dw * sizeof(int2);
     std::vector<int4> img((bytes + sizeof(int4) - 1) / sizeof(int4));
     char *b = reinterpret_cast<char *>(img.data());
-    memcpy(b, p.frames.data(), ytab_off);
+    if (p.pitched) memcpy(b, &p.lay, head);
+    else memcpy(b, p.frames.data(), head);
     for (size_t g = 0; g < G; ++g)
         resize_geometry_tables(p.geoms[g].first, p.geoms[g].second, p.dh, p.dw, reinterpret_cast<int4 *>(b + ytab_off) + g * p.dh,
                                reinterpret_cast<int2 *>(b + xtab_off) + g * p.dw);
@@ -794,15 +886,18 @@ static int resize_tables(yolo_b200_ctx *c, const SourcePlan &p, ResizeTables &ca
     return 0;
 }
 
-// One resize launch on the context stream: frames [f0, f0 + nf) of plan p (src = where frame 0 starts) into dst.  A ragged
-// launch may read up to the end of frame f0 + nf - 1 (in the host path the end of the chunk's landed bytes, never into a
-// later chunk); a uniform one reads only its own frames.
+// One resize launch on the context stream: frames [f0, f0 + nf) of plan p (src = where byte p.begin(0) is: frame 0's start,
+// or the first byte of its span when pitched) into dst.  A ragged launch may read up to the end of frame f0 + nf - 1 (in the
+// host path the end of the chunk's landed bytes, never into a later chunk); a uniform one reads only its own frames, a
+// pitched one only the span of its frames, p.begin(f0) .. p.end(f0, nf).
 static cudaError_t enqueue_resize(yolo_b200_ctx *c, const SourcePlan &p, const ResizeTables &t, const uint8_t *src, int f0, int nf, uint8_t *dst)
 {
     const bool ragged = p.mode == RESIZE_RAGGED;
     const size_t first = ragged ? 0 : p.at(f0);
-    cudaError_t e = resize_u8c3(src + first, p.at(f0 + nf) - first, p.fmt, ragged ? t.frames + f0 : nullptr, nf, p.geoms[0].first,
-                                p.geoms[0].second, dst, p.dh, p.dw, t.xtab, t.ytab, c->sm_count, c->stream);
+    const bool words = p.lay.stride % 4 == 0 && p.lay.pitch[0] % 4 == 0;
+    cudaError_t e = resize_u8c3(src + first, p.end(f0, nf) - p.first - first, p.fmt, ragged ? t.frames + f0 : nullptr, nf, p.geoms[0].first,
+                                p.geoms[0].second, dst, p.dh, p.dw, t.xtab, t.ytab, c->sm_count, c->stream,
+                                p.pitched ? reinterpret_cast<const ResizeLayout *>(t.frames) : nullptr, words);
     if (e == cudaSuccess) c->launches++;
     return e;
 }
@@ -812,17 +907,18 @@ static int resize_dev(yolo_b200_ctx *c, const SourcePlan &p, const uint8_t *d_sr
 {
     const ResizeTables *t = nullptr;
     int rc = resize_tables(c, p, c->rs_call, c->stream, &t); if (rc) return rc;
-    CU(enqueue_resize(c, p, *t, d_src, 0, p.n, d_dst));
+    CU(enqueue_resize(c, p, *t, d_src + p.first, 0, p.n, d_dst));
     return 0;
 }
 
 // The resize stages: n frames (sizes as plan_sources reads them) -> uint8 BGR [n][dh][dw][3], one launch when n >= 1
-static int resize_stage(yolo_b200_ctx *c, int fmt, const uint8_t *d_src, int n, const int32_t *src_hw, int stride, uint8_t *d_dst, int dh, int dw)
+static int resize_stage(yolo_b200_ctx *c, int fmt, const uint8_t *d_src, int n, const int32_t *src_hw, int stride, uint8_t *d_dst, int dh, int dw,
+                        const yolo_b200_frames *layout = nullptr)
 {
     if (!c) return fail(E_ARG, "null ctx");
     if (n < 0 || dh < 1 || dw < 1) return fail(E_ARG, "bad resize shape n=%d -> %dx%d", n, dh, dw);
     SourcePlan p;
-    int rc = plan_sources(fmt, n, src_hw, stride, dh, dw, false, p); if (rc) return rc;
+    int rc = plan_sources(fmt, n, src_hw, stride, dh, dw, false, p, layout); if (rc) return rc;
     CU(cudaSetDevice(c->device));
     if (n == 0) return 0;
     if (!d_src || !d_dst) return fail(E_ARG, "null buffer");
@@ -854,6 +950,15 @@ int yolo_b200_pix_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, int form
 {
     const int32_t hw[2] = { sh, sw };
     return resize_stage(c, pix_format(format), d_src, n, hw, 0, d_dst, dh, dw);
+}
+
+// The calls on a frames descriptor: its format and size, then the family's path with the layout
+#define YB_FRAMES(d) if (!(d)) return fail(E_ARG, "null frames descriptor"); const int32_t hw[2] = { (d)->sh, (d)->sw }; const int fmt = family_format((d)->family, (d)->format)
+
+int yolo_b200_frames_to_bgr_resize(yolo_b200_ctx *c, const uint8_t *d_src, const yolo_b200_frames *d, int n, uint8_t *d_dst, int dh, int dw)
+{
+    YB_FRAMES(d);
+    return resize_stage(c, fmt, d_src, n, hw, 0, d_dst, dh, dw, d);
 }
 
 int yolo_b200_u8bgr_lut(yolo_b200_ctx *c, int8_t *lut_host)
@@ -1371,11 +1476,11 @@ static int forward_dev(yolo_b200_ctx *c, InKind kind, const void *d_src, int n, 
 
 // The device forward of the resize front ends: plan, resize into the context's buffer, forward_dev
 static int forward_resize_dev(yolo_b200_ctx *c, int fmt, const uint8_t *d_src, int n, const int32_t *src_hw, int stride, int h, int w,
-                              yolo_b200_det *d_dets, int32_t *d_counts)
+                              yolo_b200_det *d_dets, int32_t *d_counts, const yolo_b200_frames *layout = nullptr)
 {
     int rc = check_ready(c, n, h, w); if (rc) return rc;
     SourcePlan p;
-    rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p); if (rc) return rc;
+    rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p, layout); if (rc) return rc;
     if (n == 0) return 0;
     if (!d_src || !d_dets || !d_counts) return fail(E_ARG, "null buffer");
     if (p.mode != RESIZE_NONE) {
@@ -1424,6 +1529,13 @@ int yolo_b200_forward_pix_dev(yolo_b200_ctx *c, const uint8_t *d_frames, int for
     return forward_resize_dev(c, pix_format(format), d_frames, n, hw, 0, h, w, d_dets, d_counts);
 }
 
+int yolo_b200_forward_frames_dev(yolo_b200_ctx *c, const uint8_t *d_frames, const yolo_b200_frames *d, int n, int h, int w,
+                                 yolo_b200_det *d_dets, int32_t *d_counts)
+{
+    YB_FRAMES(d);
+    return forward_resize_dev(c, fmt, d_frames, n, hw, 0, h, w, d_dets, d_counts, d);
+}
+
 int yolo_b200_forward_f32_dev(yolo_b200_ctx *c, const float *d_nchw, int n, int h, int w, yolo_b200_det *d_dets, int32_t *d_counts)
 { return forward_dev(c, IN_F32, d_nchw, n, h, w, d_dets, d_counts); }
 
@@ -1454,7 +1566,7 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, const Sou
     const bool resize = p.mode != RESIZE_NONE;
     const size_t net_frame_bytes = resize ? (size_t)h * w * 3 : p.frame_bytes;
     int rc = ensure(&S.stage_in, &S.stage_in_cap, (size_t)n * net_frame_bytes); if (rc) return rc;
-    if (resize) { rc = ensure(&S.rs_src, &S.rs_src_cap, p.at(n)); if (rc) return rc; }
+    if (resize) { rc = ensure(&S.rs_src, &S.rs_src_cap, p.end(0, n) - p.first); if (rc) return rc; }
     const size_t md = (size_t)c->prm.max_det;
     rc = ensure((void **)&S.d_dets, &S.dets_cap, (size_t)n * md * sizeof(yolo_b200_det)); if (rc) return rc;
     rc = ensure((void **)&S.d_counts, &S.counts_cap, (size_t)n * sizeof(int32_t)); if (rc) return rc;
@@ -1521,11 +1633,18 @@ static int host_enqueue(yolo_b200_ctx *c, int si, const void *host_in, const Sou
     // would otherwise wait for), and once for the last chunk.  (A head per chunk was measured slower: the NMS CTAs hold
     // shared memory the persistent convolution CTAs of the next chunk need, so the two serialise.)
     int head_f0 = 0;
+    size_t landed = 0;                                           // host bytes below this are already copied (or queued)
     for (int k = 0; k < nchunks; ++k) {
         const int f0 = cf0[k], nk = cnk[k];
         char *stage = (char *)S.stage_in + (size_t)f0 * net_frame_bytes;
+        // host byte p.begin(0) + b lands at rs_src + b: a pitched chunk is its span, padding included.  Where frames overlap
+        // (stride below a frame's span) the chunk copies only what earlier chunks have not, so no copy writes bytes an
+        // earlier chunk's resize reads; those landed before this chunk's copy (s_in is in order), which its resize waits for.
         char *land = resize ? (char *)S.rs_src + p.at(f0) : stage;
-        CU(cudaMemcpyAsync(land, (const char *)host_in + p.at(f0), p.at(f0 + nk) - p.at(f0), cudaMemcpyHostToDevice, c->s_in));
+        const size_t from = std::max(p.begin(f0), landed), to = p.end(f0, nk);
+        if (to > from)
+            CU(cudaMemcpyAsync(land + (from - p.begin(f0)), (const char *)host_in + from, to - from, cudaMemcpyHostToDevice, c->s_in));
+        landed = std::max(landed, to);
         CU(cudaEventRecord(S.ev_in[k], c->s_in));
         tr.mark("h2d done", k, c->s_in);
         CU(cudaStreamWaitEvent(c->stream, S.ev_in[k], 0));
@@ -1605,10 +1724,10 @@ static int host_call(yolo_b200_ctx *c, bool submit, const void *host_in, const S
 
 // host calls of the resize front ends (sizes as plan_sources reads them)
 static int host_resize(yolo_b200_ctx *c, bool submit, int fmt, const void *host_in, int n, const int32_t *src_hw, int stride, int h, int w,
-                       yolo_b200_det *dets, int32_t *counts)
+                       yolo_b200_det *dets, int32_t *counts, const yolo_b200_frames *layout = nullptr)
 {
     SourcePlan p;
-    int rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p); if (rc) return rc;
+    int rc = plan_sources(fmt, n, src_hw, stride, h, w, true, p, layout); if (rc) return rc;
     return host_call(c, submit, host_in, p, dets, counts);
 }
 
@@ -1679,6 +1798,19 @@ int yolo_b200_submit_pix(yolo_b200_ctx *c, const uint8_t *frames, int format, in
     const int32_t hw[2] = { sh, sw };
     return host_resize(c, true, pix_format(format), frames, n, hw, 0, h, w, dets, counts);
 }
+int yolo_b200_forward_frames(yolo_b200_ctx *c, const uint8_t *frames, const yolo_b200_frames *d, int n, int h, int w,
+                             yolo_b200_det *dets, int32_t *counts)
+{
+    YB_FRAMES(d);
+    return host_resize(c, false, fmt, frames, n, hw, 0, h, w, dets, counts, d);
+}
+int yolo_b200_submit_frames(yolo_b200_ctx *c, const uint8_t *frames, const yolo_b200_frames *d, int n, int h, int w,
+                            yolo_b200_det *dets, int32_t *counts)
+{
+    YB_FRAMES(d);
+    return host_resize(c, true, fmt, frames, n, hw, 0, h, w, dets, counts, d);
+}
+#undef YB_FRAMES
 
 // ---- multi-GPU collection of the detection lists -----------------------------------------------------------------
 int yolo_b200_pack_detections(yolo_b200_ctx *c, const yolo_b200_det *d_dets, const int32_t *d_counts, int n,

@@ -26,6 +26,8 @@ BAYER_RGGB, BAYER_BGGR, BAYER_GRBG, BAYER_GBRG = 0, 1, 2, 3
 # pixel formats (yolo_b200_forward_pix): packed R,G,B / R,G,B,A / B,G,R,A, 8-bit gray, and R,G,B planes (torch CHW) =
 # cv2.COLOR_RGB2BGR / _RGBA2BGR / _BGRA2BGR / _GRAY2BGR / RGB2BGR of the HWC transpose
 PIX_RGB, PIX_RGBA, PIX_BGRA, PIX_GRAY, PIX_RGB_PLANAR = 0, 1, 2, 3, 4
+# families of a frames descriptor (yolo_b200_frames): BGR (format ignored), YUV_*, BAYER_*, PIX_*
+SRC_BGR, SRC_YUV, SRC_BAYER, SRC_PIX = 0, 1, 2, 3
 
 EXPORTS = [
     "yolo_b200_abi_version", "yolo_b200_last_error", "yolo_b200_cstride", "yolo_b200_default_params",
@@ -48,6 +50,8 @@ EXPORTS = [
     "yolo_b200_bayer_to_bgr_resize", "yolo_b200_forward_bayer", "yolo_b200_submit_bayer", "yolo_b200_forward_bayer_dev",
     "yolo_b200_pix_frame_bytes", "yolo_b200_pix_to_bgr_resize", "yolo_b200_forward_pix", "yolo_b200_submit_pix",
     "yolo_b200_forward_pix_dev",
+    "yolo_b200_frames_packed", "yolo_b200_frames_span", "yolo_b200_forward_frames", "yolo_b200_submit_frames",
+    "yolo_b200_forward_frames_dev", "yolo_b200_frames_to_bgr_resize",
 ]
 
 
@@ -66,6 +70,16 @@ class Params(C.Structure):
         ("anchors", (C.c_float * 2) * MAX_ANCHORS),
         ("conf_thresh", C.c_float), ("nms_thresh", C.c_float), ("max_det", C.c_int32),
     ]
+
+
+class Frames(C.Structure):
+    """yolo_b200_frames: row r of plane p of frame i at frames + i * frame_stride + plane_offset[p] + r * row_pitch[p]."""
+    _fields_ = [("family", C.c_int32), ("format", C.c_int32), ("sh", C.c_int32), ("sw", C.c_int32), ("frame_stride", C.c_int64),
+                ("plane_offset", C.c_int64 * 3), ("row_pitch", C.c_int64 * 3)]
+
+    def __repr__(self):
+        return "Frames(family=%d, format=%d, %dx%d, stride=%d, offsets=%s, pitches=%s)" % (
+            self.family, self.format, self.sh, self.sw, self.frame_stride, list(self.plane_offset), list(self.row_pitch))
 
 
 class Det(C.Structure):
@@ -130,6 +144,12 @@ def load_library(path: Optional[str] = None):
     L.yolo_b200_pix_to_bgr_resize.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, i32]
     for name in ("yolo_b200_forward_pix", "yolo_b200_submit_pix", "yolo_b200_forward_pix_dev"):
         getattr(L, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
+    fp = C.POINTER(Frames)
+    L.yolo_b200_frames_packed.argtypes = [fp, i32, i32, i32, i32]
+    L.yolo_b200_frames_span.argtypes = [fp, i32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    for name in ("yolo_b200_forward_frames", "yolo_b200_submit_frames", "yolo_b200_forward_frames_dev"):
+        getattr(L, name).argtypes = [vp, vp, fp, i32, i32, i32, vp, vp]
+    L.yolo_b200_frames_to_bgr_resize.argtypes = [vp, vp, fp, i32, vp, i32, i32]
     L.yolo_b200_quantize_rgb444.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_quantize_f32.argtypes = [vp, vp, i32, i32, i32, vp]
     L.yolo_b200_rgb444_lut.argtypes = [vp, vp]
@@ -263,6 +283,89 @@ def pix_source_size(fmt: int, frame_shape) -> "tuple[int, int]":
     if size is None or pix_frame_shape(fmt, *size) != fs:
         raise ValueError("%s is not the shape of a pixel format %r frame" % (fs, fmt))
     return size
+
+
+def _lib_check(rc):
+    if rc != 0:
+        raise YoloB200Error("yolo_b200 error %d: %s" % (rc, load_library().yolo_b200_last_error().decode()))
+
+
+def frames_packed(family: int, fmt: int, sh: int, sw: int) -> Frames:
+    """The packed layout the family's own entry points assume (yolo_b200_frames_packed; host only)."""
+    d = Frames()
+    _lib_check(load_library().yolo_b200_frames_packed(C.byref(d), family, fmt, sh, sw))
+    return d
+
+
+def frames_span(d: Frames, n: int) -> "tuple[int, int]":
+    """(first, end): a call over n frames of layout d reads only [frames + first, frames + end) (yolo_b200_frames_span)."""
+    first, end = C.c_int64(), C.c_int64()
+    _lib_check(load_library().yolo_b200_frames_span(C.byref(d), n, C.byref(first), C.byref(end)))
+    return first.value, end.value
+
+
+# frame shape of the single-plane formats and planar RGB as arrays hold them: (rows, pixels, bytes per pixel or None)
+def _frame_axes(family, fmt):
+    if family == SRC_BGR or (family == SRC_PIX and fmt == PIX_RGB):
+        return 3
+    if family == SRC_PIX and fmt in (PIX_RGBA, PIX_BGRA):
+        return 4
+    if (family == SRC_PIX and fmt == PIX_GRAY) or (family == SRC_BAYER and fmt in (BAYER_RGGB, BAYER_BGGR, BAYER_GRBG, BAYER_GBRG)):
+        return 1
+    if family == SRC_YUV and fmt == YUV_YUYV:
+        return 2
+    if family == SRC_PIX and fmt == PIX_RGB_PLANAR:
+        return 0
+    if family == SRC_YUV and fmt in (YUV_NV12, YUV_I420):
+        raise ValueError("NV12 / I420 frames have several planes: give their offsets and pitches in a Frames explicitly")
+    raise ValueError("unknown family / format %r / %r" % (family, fmt))
+
+
+def frames_layout(x, family: int, fmt: int) -> Frames:
+    """The descriptor of a batch of frames held by a uint8 numpy array or torch tensor (CPU or CUDA) of any strides, to be
+    passed with the array's own data pointer: [n][sh][sw][c] for the packed formats (BGR, RGB, RGBA, BGRA, YUYV with
+    c = 2), [n][sh][sw] for gray and Bayer, [n][3][sh][sw] for planar RGB.  Crops, CHW crops and x[::k] need no copy.
+    Raises ValueError for what a descriptor cannot express: negative strides, a channel stride other than 1 in a packed
+    format, pixels that are not contiguous in a row, and NV12 / I420 (several planes: describe them explicitly)."""
+    bpp = _frame_axes(family, fmt)
+    shape = tuple(int(v) for v in x.shape)
+    if isinstance(x, np.ndarray):
+        ok, strides = x.dtype == np.uint8, tuple(int(v) for v in x.strides)
+    else:
+        ok, strides = str(x.dtype) == "torch.uint8", tuple(int(v) for v in x.stride())     # uint8: elements = bytes
+    if not ok:
+        raise ValueError("frames must be uint8, got %s" % (x.dtype,))
+    want = 4 if bpp in (0, 2, 3, 4) else 3
+    if len(shape) != want:
+        raise ValueError("frames of this format are %d-D arrays (batch first), got shape %s" % (want, shape))
+    # a dimension of size 1 has no meaningful stride
+    st = [0 if n == 1 else s for n, s in zip(shape, strides)]
+    if any(s < 0 for s in st):
+        raise ValueError("negative strides (flipped views) cannot be described: %s" % (strides,))
+    d = Frames()
+    d.family, d.format = family, fmt if family != SRC_BGR else 0
+    if bpp == 0:
+        n, planes, sh, sw = shape
+        if planes != 3:
+            raise ValueError("planar RGB frames are [n][3][sh][sw], got shape %s" % (shape,))
+        if sw > 1 and st[3] != 1:
+            raise ValueError("the pixels of a row are not contiguous (stride %d)" % st[3])
+        pitch = st[2] if sh > 1 else sw
+        d.plane_offset[:] = [0, st[1], 2 * st[1]]
+        d.row_pitch[:] = [pitch] * 3
+    else:
+        n, sh, sw = shape[:3]
+        if bpp > 1:
+            if shape[3] != bpp:
+                raise ValueError("a pixel of this format is %d bytes, got shape %s" % (bpp, shape))
+            if st[3] != 1:
+                raise ValueError("the channels of a pixel are not contiguous (channel stride %d)" % strides[3])
+        if sw > 1 and st[2] != bpp:
+            raise ValueError("the pixels of a row are not contiguous (pixel stride %d, %d bytes per pixel)" % (st[2], bpp))
+        d.row_pitch[0] = st[1] if sh > 1 else sw * bpp
+    d.sh, d.sw = sh, sw
+    d.frame_stride = st[0]
+    return d
 
 
 class Context:
@@ -471,6 +574,19 @@ class Context:
         return self._submit(self.L.yolo_b200_submit_pix, _ptr(frames), fmt, n, sh, sw, int(size[0]), int(size[1]),
                             dets.ctypes.data, counts.ctypes.data)
 
+    def forward_frames(self, frames, d: Frames, n: int, size):
+        """n host frames laid out as d says (frames: a numpy array, a torch tensor or an address; frames_layout derives d
+        from an array's strides) -> (dets [n][max_det], counts [n]): the family's forward_* on the frames, without
+        compacting them first."""
+        return self._forward_host(self.L.yolo_b200_forward_frames, n, _ptr(frames), C.byref(d), n, int(size[0]), int(size[1]))
+
+    def submit_frames(self, frames, d: Frames, n: int, size, dets: np.ndarray, counts: np.ndarray) -> int:
+        """Queue n host frames laid out as d says (pinned memory for an asynchronous copy) for size = (h, w); frames, dets
+        [n][max_det] DET_DTYPE and counts int32 [n] must stay alive and untouched until wait(ticket).  Returns the ticket."""
+        assert dets.flags.c_contiguous and counts.flags.c_contiguous and len(dets) >= n and len(counts) >= n
+        return self._submit(self.L.yolo_b200_submit_frames, _ptr(frames), C.byref(d), n, int(size[0]), int(size[1]),
+                            dets.ctypes.data, counts.ctypes.data)
+
     def forward_int8(self, nhwc4: np.ndarray):
         x = np.ascontiguousarray(nhwc4, dtype=np.int8)
         n, h, w, c = x.shape
@@ -534,6 +650,14 @@ class Context:
     def pix_to_bgr_resize(self, d_src, fmt, n, sh, sw, d_dst, dh, dw):
         """cv2.resize(cv2.cvtColor(frame, code), (dw, dh)) of n device frames of pixel format fmt into d_dst uint8 [n][dh][dw][3]."""
         self._check(self.L.yolo_b200_pix_to_bgr_resize(self._h, _ptr(d_src), fmt, n, sh, sw, _ptr(d_dst), dh, dw))
+
+    def forward_frames_dev(self, d_in, d: Frames, n, h, w, d_dets, d_counts):
+        """n frames in device memory laid out as d says (a decoder surface, a strided CUDA tensor: frames_layout)."""
+        self._check(self.L.yolo_b200_forward_frames_dev(self._h, _ptr(d_in), C.byref(d), n, h, w, _ptr(d_dets), _ptr(d_counts)))
+
+    def frames_to_bgr_resize(self, d_src, d: Frames, n, d_dst, dh, dw):
+        """The front-end stage of forward_frames_dev: n device frames laid out as d says -> d_dst uint8 [n][dh][dw][3]."""
+        self._check(self.L.yolo_b200_frames_to_bgr_resize(self._h, _ptr(d_src), C.byref(d), n, _ptr(d_dst), dh, dw))
 
     def resize_u8bgr(self, d_src, n, sh, sw, d_dst, dh, dw):
         """cv2.resize (bilinear) of n uint8 [sh][sw][3] device images into d_dst [n][dh][dw][3]."""
